@@ -12,6 +12,7 @@ pair, 20k matched points (~40k triangles), 6-level pyramid; 600 phases per step 
     python bench.py --workload 1080p|4k|8k                     # the other points of the metric (default 4k = configs[3])
     python bench.py --workload 8k --total-frames 2400 --gpus N   # configs[4]: 2,400 8K phases sharded over N ranks (strong scaling)
     python bench.py --mode chain                                # configs[0]: the reference demo pair, 60 chained frames, 64 levels
+    python bench.py --dump-outputs DIR                          # + a fixed sample of the last timed step's outputs, DIR/*.npy
 
 JSON line (rank 0):
   value       whole-job frames/s with inputs resident in HBM, device time (CUDA events on the context's stream),
@@ -248,6 +249,25 @@ class Job:
                 "timing": "CUDA events on the renderer's stream, max over ranks"}
 
 
+DUMP_FRAMES, DUMP_PIXELS = 8, 1 << 19     # 8 frames x 2^19 pixels x 3 channels x 4 bytes = 48 MiB
+
+
+def dump_outputs(out_dir, r, job):
+    """What the last timed step handed back, as float32 .npy files in out_dir: the frames still resident in the ring (the
+    step's last ring slice) and their morphed points. A 4K frame alone is 100 MB in float32, so the files hold a fixed
+    sample: up to DUMP_FRAMES frames spread evenly over the slice, and in each the same seeded set of at most DUMP_PIXELS
+    pixel positions. Inputs and sample depend on the arguments only, so two builds can be compared file for file."""
+    a, b = job.slices[-1]
+    ks = np.unique(np.linspace(0, b - a - 1, min(b - a, DUMP_FRAMES)).round().astype(int))
+    px = job.W * job.H
+    sel = np.sort(np.random.default_rng(0).choice(px, DUMP_PIXELS, replace=False)) if px > DUMP_PIXELS else slice(None)
+    frames = np.stack([r.download(int(k), 1)[0].reshape(px, 3)[sel] for k in ks]).astype(np.float32)
+    points = np.stack([r.morphed_points(int(k)) for k in ks]).astype(np.float32)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "frames.npy"), frames)                  # (frames, pixels, BGR) values 0..255
+    np.save(os.path.join(out_dir, "morphed_points.npy"), points)          # (frames, points, xy)
+
+
 def _kproc_worker(q, path, w, h, levels, phases):
     """One process of the K-process CPU baseline: the reference library on one OpenCV thread."""
     try:
@@ -358,7 +378,13 @@ def main():
     ap.add_argument("--e2e-slice", type=int, default=64, help="frames per planned/rendered/downloaded slice of the e2e pipeline")
     ap.add_argument("--no-stage-pass", action="store_true",
                     help="profiling runs (under ncu): skip the per-kernel-class timing pass and the e2e leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write a fixed sample of the frames and morphed points of the last timed step (rank 0) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "cuda":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; the reference arm does not dump")
     if args.kprocs < 0:
         args.kprocs = min(os.cpu_count() or 1, 16) if args.cpu_frames > 0 and args.mode == "direct" and args.workload != "8k" else 0
 
@@ -443,6 +469,8 @@ def main():
     dev_ms = e0.elapsed_time(e1)
     launches = r.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, r, job)
     exact_chunks, all_chunks = r.unsharp_stats()
     sums = []
     if len(job.slices) > 1:

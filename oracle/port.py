@@ -140,3 +140,31 @@ def morph_frame(bgr1, bgr2, gabor2, pts1, pts2, tri_idx, shape, mask_ratio, leve
     lib().poppy_oracle_morph_frame(w, h, _p(bgr1), _p(bgr2), _p(gabor2), _p(pts1), _p(pts2), n, _p(tri_idx), t,
                                    C.c_double(shape), C.c_double(mask_ratio), int(levels), C.byref(d))
     return Stages(**out)
+
+
+# The entry points of oracle/ref.py with the same signatures: the frame path above around the host topology stage
+# (poppy_b200.host, pinned to cv::Subdiv2D by tests/golden/topology.npz). Tests compare against these where the
+# reference library is not built.
+def stages(bgr1, bgr2, gabor2, pts1, pts2, shape, mask, levels) -> Stages:
+    from poppy_b200 import host
+    h, w = np.shape(bgr1)[:2]
+    tri = host.triangulate(host.morph_points(pts1, pts2, shape, w, h), w, h)
+    return morph_frame(bgr1, bgr2, gabor2, pts1, pts2, tri, shape, mask, levels)
+
+
+def morph_images(bgr1, bgr2, gabor2, pts1, pts2, shape, mask, levels):
+    st = stages(bgr1, bgr2, gabor2, pts1, pts2, shape, mask, levels)
+    return st.dst, st.morphed_points
+
+
+def chain(bgr1, bgr2, gabor2, pts1, pts2, n_frames, levels):
+    """The frame-loop recurrence of reference src/poppy.hpp:177-243: frame j morphs frame j-1 and its points."""
+    from poppy_b200 import host
+    frames, points = [], []
+    cur_img, cur_pts = bgr1, pts1
+    for j in range(n_frames):
+        s = host.chain_ratio(j, n_frames)
+        cur_img, cur_pts = morph_images(cur_img, bgr2, gabor2, cur_pts, pts2, s, s, levels)
+        frames.append(cur_img)
+        points.append(cur_pts)
+    return np.stack(frames), np.stack(points)

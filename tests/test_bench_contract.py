@@ -48,6 +48,37 @@ def test_job_configs_are_identical_for_both_arms():
     assert j0.phases[0] == 0 and abs(j0.masks[-1] - 1.0) < 1e-12
 
 
+def test_dump_outputs_writes_a_fixed_float32_sample_under_64_mb(tmp_path):
+    """--dump-outputs at the 4K workload: frames sampled from the ring slots of the last slice, the same sample every
+    run, float32 files of at most 64 MB in all."""
+    import argparse
+    import numpy as np
+    b = _bench()
+
+    class Ring:                                  # stands in for MorphRenderer: slot k holds frame k of the slice
+        def download(self, first, count):
+            return np.full((count, 2160, 3840, 3), first % 256, np.uint8) + np.arange(3, dtype=np.uint8)
+
+        def morphed_points(self, k):
+            return np.full((20004, 2), k, np.float32)
+
+    a = argparse.Namespace(mode="direct", workload="4k", content="synthetic", total_frames=0, frames=600, ring=0)
+    job = b.Job(a, 0, 1)
+    sizes = []
+    for run in ("a", "b"):
+        b.dump_outputs(str(tmp_path / run), Ring(), job)
+        files = sorted(p.name for p in (tmp_path / run).iterdir())
+        assert files == ["frames.npy", "morphed_points.npy"]
+        sizes.append(sum((tmp_path / run / f).stat().st_size for f in files))
+    assert sizes[0] <= 64 * 2 ** 20
+    for f in files:
+        x, y = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert x.dtype == np.float32 and (x == y).all()
+    frames = np.load(tmp_path / "a" / "frames.npy")
+    assert frames.shape == (b.DUMP_FRAMES, b.DUMP_PIXELS, 3)
+    assert frames[0, 0, 0] == 0 and frames[-1, 0, 2] == 599 % 256 + 2   # first and last frame of the 600-frame slice
+
+
 def test_committed_traffic_file_is_well_formed():
     t = json.load(open(os.path.join(ROOT, "profiles", "ncu_traffic.json")))
     assert set(t["bytes_per_frame"]) >= {"raster_warp", "pyr_down", "blend_collapse", "unsharp_store"}

@@ -33,19 +33,25 @@ def test_port_reproduces_golden_stages(path):
 
 def test_port_reproduces_golden_chain():
     """Frame-loop recurrence (reference src/poppy.hpp:177-243) restated around the port + the host topology."""
-    from poppy_b200 import host
     g = np.load(os.path.join(GOLDEN, "chain_shapes_80x64_N12_L64.npz"))
-    n_frames, levels = int(g["n_frames"]), int(g["levels"])
-    h, w = g["bgr1"].shape[:2]
-    cur_img, cur_pts = g["bgr1"], g["pts1"]
-    for j in range(n_frames):
-        s = host.chain_ratio(j, n_frames)
-        mp = host.morph_points(cur_pts, g["pts2"], s, w, h)
-        tri = host.triangulate(mp, w, h)
-        st = port.morph_frame(cur_img, g["bgr2"], g["gabor2"], cur_pts, g["pts2"], tri, s, s, levels)
-        assert bits_differ(st.morphed_points, g["points"][j]) == 0, j
-        assert (st.dst == g["frames"][j]).all(), j
-        cur_img, cur_pts = st.dst, st.morphed_points
+    frames, points = port.chain(g["bgr1"], g["bgr2"], g["gabor2"], g["pts1"], g["pts2"], int(g["n_frames"]), int(g["levels"]))
+    for j in range(int(g["n_frames"])):
+        assert bits_differ(points[j], g["points"][j]) == 0, j
+        assert (frames[j] == g["frames"][j]).all(), j
+
+
+@pytest.mark.parametrize("path", FRAME_FILES, ids=[os.path.basename(f)[:-4] for f in FRAME_FILES])
+def test_port_entry_points_reproduce_golden_frames(path):
+    """port.stages / port.morph_images, the stand-ins of the reference library in the GPU parity tests, with their own
+    triangulation: the same triangle lists, stages and frames as the reference."""
+    g = np.load(path)
+    args = (g["bgr1"], g["bgr2"], g["gabor2"], g["pts1"], g["pts2"], float(g["shape"]), float(g["mask_ratio"]), int(g["levels"]))
+    st = port.stages(*args)
+    assert (st.tri_idx == g["tri_idx"]).all()
+    for k in STAGE_KEYS:
+        assert bits_differ(getattr(st, k), g[k]) == 0, k
+    dst, mp = port.morph_images(*args)
+    assert (dst == g["dst"]).all() and bits_differ(mp, g["morphed_points"]) == 0
 
 
 def test_fixtures_come_from_the_avx2_fma_dispatch_of_the_reference():

@@ -1,5 +1,7 @@
 """GPU parity through the public API (Python mirror of the reference interface -> C ABI -> CUDA kernels):
-single frames, the chain recurrence, batched independent phases, the golden fixtures and error behaviour."""
+single frames, the chain recurrence, batched independent phases, the golden fixtures and error behaviour. Without the
+reference library the parity cases compare with the CPU restatement, whose triangle lists come from the product's host
+stage (see tests.util.reference); the golden fixtures below carry the reference's own triangle lists."""
 import ctypes as C
 import glob
 import os
@@ -8,7 +10,7 @@ import numpy as np
 import pytest
 
 from poppy_b200 import api, host, synth
-from tests.util import assert_frame_parity, bits_differ, flat_tri
+from tests.util import assert_frame_parity, bits_differ, flat_tri, reference as _ref
 
 pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -18,13 +20,6 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 def _fresh_api(native_lib):
     yield
     api.release()
-
-
-def _ref():
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("reference library not shipped")
-    return ref
 
 
 @pytest.mark.parametrize("kind,w,h,n,s,m,levels", [

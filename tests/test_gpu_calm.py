@@ -6,16 +6,9 @@ import pytest
 
 from poppy_b200 import host, synth
 from poppy_b200.renderer import MorphRenderer
-from tests.util import bits_differ
+from tests.util import bits_differ, reference as _ref
 
 pytestmark = pytest.mark.gpu
-
-
-def _ref():
-    from oracle import ref
-    if not ref.available():
-        pytest.skip("reference library not shipped")
-    return ref
 
 
 CASES = [

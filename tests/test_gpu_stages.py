@@ -1,10 +1,11 @@
 """GPU parity, stage by stage: every stage boundary of the CUDA path (through the C ABI) must equal the
-reference library's (oracle/_ref, the unmodified reference code) bit for bit on seeded inputs."""
+reference's (oracle/_ref, the unmodified reference code, or the CPU restatement pinned to it) bit for bit on
+seeded inputs."""
 import numpy as np
 import pytest
 
 from poppy_b200 import synth
-from tests.util import bits_differ, flat_tri
+from tests.util import bits_differ, flat_tri, reference
 
 pytestmark = pytest.mark.gpu
 
@@ -28,10 +29,10 @@ CASES = [
 
 @pytest.mark.parametrize("w,h,n,s,levels", CASES)
 def test_stage_parity_vs_reference(native_lib, w, h, n, s, levels):
-    from oracle import ref, port
+    from oracle import port
     from poppy_b200 import renderer as R
     inp = synth.make_inputs(w, h, n, 8.0, seed=7)
-    want = ref.stages(inp.bgr1, inp.bgr2, inp.gabor2, inp.pts1, inp.pts2, s, s, levels)
+    want = reference().stages(inp.bgr1, inp.bgr2, inp.gabor2, inp.pts1, inp.pts2, s, s, levels)
     tri = want.tri_idx
     with R.MorphRenderer(w, h, levels, len(inp.pts1), max(len(tri), 1), 1, keep_stages=True) as r:
         r.set_pair(inp.bgr1, inp.bgr2, inp.gabor2)
