@@ -73,15 +73,15 @@ void launch_pyramid_tail(cudaStream_t st, float* g_base, float* o_base, const Ta
 // resultSmallest = left*mask + right*(1-mask) at the coarsest level (blend.hpp:68-69)
 void launch_blend_coarsest(cudaStream_t st, const float* g, LevelDesc l, float* out, int frames);
 // out[k] = pyrUp(out[k+1]) + (G_l[k]-pyrUp(G_l[k+1]))*m[k] + (G_r[k]-pyrUp(G_r[k+1]))*(1-m[k])   (blend.hpp:45-77)
-// maps (nullable): tensor maps of the level's planes; with them interior tiles are fed by a TMA producer warp
+// maps (nullable): tensor maps of the level's planes; with them interior tiles are fed by a TMA producer warp, without them
+// (levels too small to have an interior tile) every tile runs the generic body
 void launch_collapse(cudaStream_t st, const float* g_fine, LevelDesc fl, const float* g_coarse, const float* out_coarse,
                      LevelDesc cl, float* out_fine, int frames, const CollapseMaps* maps);
 // same for level 0, whose Gaussian level is the warped 8-bit pair + the level-0 mask planes
 // tile_flags (nullable): per frame and 128x32 tile, 0 = the tile is not needed (calm, see below)
 void launch_collapse0(cudaStream_t st, const uint32_t* warped, int wpitch, size_t wstride, const float* mask0, int mpitch,
                       size_t m0stride, int w, int h, const float* g_coarse, const float* out_coarse, LevelDesc cl,
-                      float* out_fine, LevelDesc ol, int frames, const unsigned char* tile_flags, const CollapseMaps* maps,
-                      int map_frame0 = 0);     // map_frame0: chunk frame index of the launch's first frame (the maps span the chunk)
+                      float* out_fine, LevelDesc ol, int frames, const unsigned char* tile_flags, const CollapseMaps* maps);
 // level-0 collapse fused with convertTo(CV_8U, 255): stores cvRound(255 out[0]) into the frame ring (exactly the frame
 // wherever unsharp_mask() leaves the pixel untouched) and, per 4x8-pixel block and channel, whether out[0] left [0, 1] by
 // more than 0.001 there: ex[(f*3 + c) * ex_stride + by * ex_pitch + bx]

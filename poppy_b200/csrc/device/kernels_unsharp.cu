@@ -24,7 +24,6 @@
 //   M  8 rows x 30 groups: where no flagged group touches the 3x3 window the median cannot reach the 0.3 threshold
 //      (|median| <= max |diff| < 0.3/sqrt(3)), so the pixel is the input; otherwise the exact median/norm/sharpen runs.
 //      Rounding to 8 bits uses the magic-number trick of pixel_ops.cuh; rows are written as three 32-bit words per lane.
-#include <cstdlib>
 
 #include "common.cuh"
 #include "kernels.cuh"
@@ -565,12 +564,10 @@ void launch_unsharp_store(cudaStream_t st, const float* lap_blend, LevelDesc l, 
         while (__builtin_sqrt(s) < t) s = __builtin_nextafter(s, 1.0);
         return s;
     }();
-    // POPPY_CUDA_US_PAD: extra bytes of dynamic shared memory per CTA (caps the CTAs per SM: room for another lane's kernels)
-    static const size_t pad = [] { const char* e = getenv("POPPY_CUDA_US_PAD"); return e ? (size_t)atoi(e) : (size_t)0; }();
     static SmemAttrOnce done;
-    ensure_smem_attr(k_unsharp_strip, US_SMEM + pad, done);
+    ensure_smem_attr(k_unsharp_strip, US_SMEM, done);
     if (chunk_rows <= 0) chunk_rows = US_CHUNK;
-    k_unsharp_strip<<<dim3(div_up(l.w, US_W), div_up(l.h, chunk_rows), frames), 256, US_SMEM + pad, st>>>(
+    k_unsharp_strip<<<dim3(div_up(l.w, US_W), div_up(l.h, chunk_rows), frames), 256, US_SMEM, st>>>(
         lap_blend, l.w, l.h, l.pitch, l.plane_stride, fp, thr2, frames_base, frame_bytes, chunk_rows, chunk_flags);
 }
 

@@ -39,8 +39,7 @@ void* huge_alloc(size_t bytes) {
         if (c.ptr[i] && c.size[i] == size) { void* p = c.ptr[i]; c.ptr[i] = nullptr; return p; }
     void* p = std::aligned_alloc(kHugePage, size);
     if (!p) throw std::bad_alloc();
-    static const bool advise = [] { const char* e = std::getenv("POPPY_PLAN_HUGEPAGES"); return !(e && e[0] == '0'); }();   // A/B switch
-    if (advise) madvise(p, size, MADV_HUGEPAGE);          // advisory: ordinary pages serve equally well, only slower
+    madvise(p, size, MADV_HUGEPAGE);          // advisory: ordinary pages serve equally well, only slower
     return p;
 }
 
@@ -522,103 +521,6 @@ void DelaunayMesh::triangles(std::vector<int32_t>& ids) const {
         ids.push_back(b);
         ids.push_back(c);
     }
-}
-
-namespace {
-
-// One frame of a batch: its deduplicated points, its mesh and the walk of the point being inserted.
-struct BatchJob {
-    std::vector<Point2f> uniq;
-    std::vector<int32_t> first, owner;
-    DelaunayMesh* mesh = nullptr;
-    DelaunayMesh::Walk walk;
-    size_t next = 0;            // next point of `uniq` to insert
-    int slot = -1;              // index of the point set this job triangulates
-    bool alive = false, failed = false;
-    ~BatchJob() { delete mesh; }
-
-    void open(const std::vector<Point2f>& points, int index, int width, int height) {
-        std::vector<Point2f> clipped = points;
-        clip_points(clipped, width, height);
-        uniq.clear();
-        first.clear();
-        make_uniq(clipped, uniq, &first);
-        owner.assign(4, -1);
-        delete mesh;
-        mesh = new DelaunayMesh(width, height, (int)uniq.size());
-        next = 0;
-        slot = index;
-        failed = false;
-        alive = true;
-        start_next();
-    }
-    // begins the walk of the next point; alive = false when the set is exhausted or an insertion failed
-    void start_next() {
-        while (next < uniq.size()) {
-            if (mesh->begin_walk(uniq[next], walk)) return;
-            complete();                      // outside the rectangle: finish_insert reports it
-            if (!alive) return;
-        }
-        alive = false;
-    }
-    // the walk of point `next` has ended: update the topology
-    void complete() {
-        const int v = mesh->finish_insert(walk);
-        if (v < 0) { failed = true; alive = false; return; }
-        if (v >= (int)owner.size()) owner.resize(v + 1, -1);
-        if (owner[v] < 0) owner[v] = first[next];
-        ++next;
-    }
-    void close(std::vector<int32_t>& tri_idx, bool& ok, std::string& error) {
-        tri_idx.clear();
-        ok = !failed;
-        if (failed) { error = mesh->error(); return; }
-        std::vector<int32_t> ids;
-        mesh->triangles(ids);
-        tri_idx.resize(ids.size());
-        for (size_t i = 0; i < ids.size(); ++i) tri_idx[i] = owner[ids[i]];
-    }
-};
-
-template <int K>
-void run_batch(const std::vector<Point2f>* sets, int count, int width, int height, std::vector<int32_t>* tri_idx, bool* ok,
-               std::string* errors) {
-    BatchJob jobs[K];
-    int issued = 0, open_jobs = 0;
-    for (int k = 0; k < K && issued < count; ++k, ++issued, ++open_jobs) jobs[k].open(sets[issued], issued, width, height);
-    while (open_jobs > 0) {
-        // one walk step of every mesh per round: K independent dependency chains in flight
-#pragma GCC unroll 8
-        for (int k = 0; k < K; ++k) {
-            BatchJob& j = jobs[k];
-            if (j.slot < 0) continue;
-            if (j.alive && j.mesh->walk_step(j.walk)) continue;
-            if (j.alive) {
-                j.complete();
-                if (j.alive) j.start_next();
-                if (j.alive) continue;
-            }
-            j.close(tri_idx[j.slot], ok[j.slot], errors[j.slot]);
-            j.slot = -1;
-            --open_jobs;
-            if (issued < count) {
-                j.open(sets[issued], issued, width, height);
-                ++issued;
-                ++open_jobs;
-            }
-        }
-    }
-}
-
-}  // namespace
-
-void triangulate_points_batch(const std::vector<Point2f>* sets, int count, int width, int height,
-                              std::vector<int32_t>* tri_idx, bool* ok, std::string* errors, int ways) {
-    if (ways >= 8) run_batch<8>(sets, count, width, height, tri_idx, ok, errors);
-    else if (ways >= 6) run_batch<6>(sets, count, width, height, tri_idx, ok, errors);
-    else if (ways >= 4) run_batch<4>(sets, count, width, height, tri_idx, ok, errors);
-    else if (ways >= 2) run_batch<2>(sets, count, width, height, tri_idx, ok, errors);
-    else run_batch<1>(sets, count, width, height, tri_idx, ok, errors);
 }
 
 bool triangulate_points(std::vector<Point2f> points, int width, int height, std::vector<int32_t>& tri_idx,

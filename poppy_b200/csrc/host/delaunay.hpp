@@ -98,17 +98,6 @@ public:
         Where where;
     };
 
-    // The same insertion cut at the boundaries of its point-location walk, so that a caller can advance the walks of
-    // several independent meshes in one instruction stream (triangulate_points_batch): the walk is a chain of dependent
-    // loads and compares (~100 cycles per step, ~120 steps per point at 20k points) that leaves the core idle; the
-    // out-of-order window overlaps the chains of different meshes.
-    //   begin_walk(p, w)   false: p is outside the rectangle (w.where = kOutside)
-    //   walk_step(w)       one step of Subdiv2D::locate; false when the walk has ended
-    //   finish_insert(w)   classification of the final edge + the topology update; returns what insert() returns
-    bool begin_walk(Point2f pt, Walk& w) const;
-    bool walk_step(Walk& w) const;
-    int finish_insert(Walk& w);
-
     // The general-position steps of the same walk as one loop with the data dependences cut: while the two orientation
     // predicates of the current edge are evaluated, the links and end points of BOTH possible successors are already
     // being loaded and their coordinate differences formed, so a step costs one predicate latency instead of
@@ -145,6 +134,15 @@ public:
     const std::string& error() const { return err_; }
 
 private:
+    // insert() cut at the boundaries of its point-location walk, which insert() runs in between (walk_guided, walk_run,
+    // and walk_step wherever a predicate is degenerate):
+    //   begin_walk(p, w)   false: p is outside the rectangle (w.where = kOutside)
+    //   walk_step(w)       one step of Subdiv2D::locate, degenerate predicates included; false when the walk has ended
+    //   finish_insert(w)   classification of the final edge + the topology update; returns what insert() returns
+    bool begin_walk(Point2f pt, Walk& w) const;
+    bool walk_step(Walk& w) const;
+    int finish_insert(Walk& w);
+
     // One quad-edge record = half a cache line: the four onext links and a copy of the origin coordinates of the two
     // primal edges, so that the point-location walk (latency-bound pointer chasing, ~120 steps per inserted point at
     // 20k points; three records per step: the current edge's, its onext's and its dprev's) never chases vertex
@@ -196,10 +194,5 @@ bool triangulate_points(std::vector<Point2f> points, int width, int height, std:
 // morph_images() once per frame): each call is predicted by the calling thread's previous call and records for the next.
 bool triangulate_points_next(std::vector<Point2f> points, int width, int height, std::vector<int32_t>& tri_idx,
                              std::string* error = nullptr);
-
-// The same for `count` independent point sets (the frames of a sequence) on one thread, with the point-location walks
-// of up to `ways` meshes interleaved (see DelaunayMesh::walk_step). ok[i] / errors[i] as triangulate_points.
-void triangulate_points_batch(const std::vector<Point2f>* sets, int count, int width, int height,
-                              std::vector<int32_t>* tri_idx, bool* ok, std::string* errors, int ways = 4);
 
 }  // namespace poppy

@@ -2,9 +2,7 @@
 #include <atomic>
 #include <climits>
 #include <cmath>
-#include <cstdlib>
 #include <cstring>
-#include <functional>
 #include <memory>
 #include <mutex>
 #include <string>
@@ -147,69 +145,42 @@ int poppy_host_plan_create(poppy_host_plan** out, const float* p1, const float* 
     // triangulations are independent: fan out over host threads
     std::vector<std::vector<int32_t>> tris(n_frames);
     std::vector<std::string> errs(n_frames);
-    std::atomic<int> next{0}, failed{-1};
+    std::atomic<int> failed{-1};
     int nt = threads > 0 ? threads : (int)std::thread::hardware_concurrency();
     nt = std::max(1, std::min(nt, n_frames));
-    // POPPY_PLAN_WAYS > 1: a thread triangulates that many frames at once with their point-location walks interleaved
-    // (pays where the quad-edge tables of several meshes fit the core's cache; see delaunay.hpp)
-    const char* ways_env = std::getenv("POPPY_PLAN_WAYS");
-    const int ways = ways_env ? std::max(1, std::min(8, std::atoi(ways_env))) : 1;
-    // ways == 1 (default): worker t triangulates frames t, t + nt, t + 2 nt, ... Frame f is PREDICTED by frame f - 1
-    // (poppy::WalkTrace), which another worker is triangulating at the same time: frame f runs a few points behind it
-    // (poppy::WalkPace), so every frame but the first is guided by its immediate neighbour - the distance at which the
-    // prediction is nearly perfect - and all workers stay busy. Frame 0 is predicted by the last frame of the previous call
-    // (the previous slice of the same sequence, typically); a stale guide costs its own mispredictions, never the result.
-    const char* guide_env = std::getenv("POPPY_PLAN_GUIDE");            // A/B switch: 0 = unguided walks
-    const bool guided = !(guide_env && guide_env[0] == '0');
+    // Worker t triangulates frames t, t + nt, t + 2 nt, ... Frame f is PREDICTED by frame f - 1 (poppy::WalkTrace), which
+    // another worker is triangulating at the same time: frame f runs a few points behind it (poppy::WalkPace), so every
+    // frame but the first is guided by its immediate neighbour - the distance at which the prediction is nearly perfect -
+    // and all workers stay busy. Frame 0 is predicted by the last frame of the previous call (the previous slice of the
+    // same sequence, typically); a stale guide costs its own mispredictions, never the result.
     const int ring = 2 * nt + 1;
-    std::vector<poppy::WalkTrace> traces(guided ? ring : 0);
+    std::vector<poppy::WalkTrace> traces(ring);
     std::unique_ptr<std::atomic<int>[]> progress(new std::atomic<int>[n_frames + 1]);
     for (int f = 0; f <= n_frames; ++f) progress[f].store(0, std::memory_order_relaxed);
     poppy::WalkTrace carried;                                           // the previous call's last trace
-    if (guided) take_carried_trace(carried);
+    take_carried_trace(carried);
     std::atomic<int> worker_id{0};
-    auto work_single = [&] {
+    auto work = [&] {
         const int t = worker_id.fetch_add(1);
         for (int f = t; f < n_frames; f += nt) {
-            bool ok;
-            if (!guided) {
-                ok = poppy::triangulate_points(plan->points[f], w, h, tris[f], &errs[f]);
-                progress[f].store(INT_MAX, std::memory_order_release);
-            } else {
-                // the ring slot of frame f was last used by frame f - ring, which frame f - ring + 1 was reading
-                if (f - ring + 1 >= 0)
-                    while (progress[f - ring + 1].load(std::memory_order_acquire) != INT_MAX) std::this_thread::yield();
-                poppy::WalkPace pace;
-                pace.publish = &progress[f];
-                pace.follow = f > 0 ? &progress[f - 1] : nullptr;
-                const poppy::WalkTrace* guide = f > 0 ? &traces[(f - 1) % ring] : (carried.empty() ? nullptr : &carried);
-                ok = poppy::triangulate_points(plan->points[f], w, h, tris[f], &errs[f], guide, &traces[f % ring], &pace);
-            }
-            if (!ok) {
+            // the ring slot of frame f was last used by frame f - ring, which frame f - ring + 1 was reading
+            if (f - ring + 1 >= 0)
+                while (progress[f - ring + 1].load(std::memory_order_acquire) != INT_MAX) std::this_thread::yield();
+            poppy::WalkPace pace;
+            pace.publish = &progress[f];
+            pace.follow = f > 0 ? &progress[f - 1] : nullptr;
+            const poppy::WalkTrace* guide = f > 0 ? &traces[(f - 1) % ring] : (carried.empty() ? nullptr : &carried);
+            if (!poppy::triangulate_points(plan->points[f], w, h, tris[f], &errs[f], guide, &traces[f % ring], &pace)) {
                 int expected = -1;
                 failed.compare_exchange_strong(expected, f);
             }
         }
     };
-    auto work_batched = [&] {
-        std::unique_ptr<bool[]> ok(new bool[ways]);
-        for (int f0; (f0 = next.fetch_add(ways)) < n_frames;) {
-            const int cnt = std::min(ways, n_frames - f0);
-            poppy::triangulate_points_batch(&plan->points[f0], cnt, w, h, &tris[f0], ok.get(), &errs[f0], ways);
-            for (int i = 0; i < cnt; ++i)
-                if (!ok[i]) {
-                    int expected = -1;
-                    failed.compare_exchange_strong(expected, f0 + i);
-                }
-        }
-    };
-    std::function<void()> work = work_batched;
-    if (ways == 1) work = work_single;
     std::vector<std::thread> pool;
     for (int i = 1; i < nt; ++i) pool.emplace_back(work);
     work();
     for (auto& t : pool) t.join();
-    if (guided && ways == 1 && n_frames > 0) put_carried_trace(traces[(n_frames - 1) % ring]);
+    put_carried_trace(traces[(n_frames - 1) % ring]);
     if (failed.load() >= 0) {
         std::string msg = "frame " + std::to_string(failed.load()) + ": " + errs[failed.load()];
         delete plan;

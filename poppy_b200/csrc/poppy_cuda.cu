@@ -15,7 +15,6 @@
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -47,13 +46,17 @@ constexpr unsigned kCalmProbeEvery = 8;      // on the dense route: every n-th c
 // regions out of the exact path at the price of the 10-row warm-up per chunk)
 constexpr int kSparseChunkRows = 24;
 
+// Render lanes: consecutive chunks of a direct-mode render go round-robin to the lanes. Measured at 4K: 1 lane 2,694,
+// 2: 2,952, 3: 3,150, 4: 3,219-3,259, 8: 3,263 frames/s.
+constexpr int kRenderLanes = 4;
+
 }  // namespace
 
 struct poppy_cuda_ctx {
     int device = 0, w = 0, h = 0, levels = 0, max_points = 0, max_tri = 0, max_frames = 0;
     int chunk = 0;            // frames per kernel batch (0 = not yet allocated)
     int want_chunk = 0;
-    bool keep_stages = false, stage_timing = false, single_lane = false;
+    bool keep_stages = false, stage_timing = false;
     bool have_pair = false, have_points = false;
     bool have_image[3] = {false, false, false};
     uint8_t* d_stage_u8 = nullptr;       // upload staging of set_image, kept between calls
@@ -86,9 +89,9 @@ struct poppy_cuda_ctx {
     float2 *d_pts1_raw = nullptr, *d_pts2_raw = nullptr, *d_pts1 = nullptr, *d_pts2 = nullptr, *d_morphed = nullptr;
     uint8_t* d_frames = nullptr;
     unsigned long long* d_sum = nullptr;
-    // Chunk scratch. Up to four lanes (default three), each with its own stream and scratch: consecutive chunks of a
-    // direct-mode render go round-robin to the lanes, so the issue-bound kernels of one chunk overlap the latency- and
-    // bandwidth-bound kernels of the others.
+    // Chunk scratch of kRenderLanes lanes, each with its own stream: consecutive chunks of a direct-mode render go
+    // round-robin to the lanes, so the issue-bound kernels of one chunk overlap the latency- and bandwidth-bound kernels of
+    // the others.
     struct Lane {
         cudaStream_t stream = nullptr;
         cudaEvent_t ev_staged = nullptr, ev_done = nullptr;
@@ -107,14 +110,13 @@ struct poppy_cuda_ctx {
         int* h_calm_counts = nullptr;        // pinned: flagged strip chunks per frame of the lane's last calm-route chunk
         cudaEvent_t ev_calm = nullptr;
         int calm_pending = 0;                // frames whose counts are on their way to h_calm_counts
-        std::vector<CollapseMaps> maps;      // tensor maps of level k's collapse (index k); empty = no TMA path
+        std::vector<CollapseMaps> maps;      // tensor maps of level k's collapse (index k)
         FrameParams* h_fp = nullptr;         // pinned staging
         int32_t* h_tri = nullptr;
-    } lane[8];
-    int want_lanes = 4;                      // POPPY_CUDA_LANES (1..8); measured at 4K: 1 lane 2,694, 2: 2,952, 3: 3,150, 4: 3,219-3,259, 8: 3,263 frames/s
+    } lane[kRenderLanes];
     int n_lanes = 0;                         // lanes allocated (0 = none yet)
     int n_tiles = 0, list_cap = 0;
-    // levels tail_k0 .. L run in one launch (k_pyramid_tail); 0 = none (no level is small enough, or POPPY_CUDA_TAIL=0)
+    // levels tail_k0 .. L run in one launch (k_pyramid_tail); 0 = none (no level is small enough)
     int tail_k0 = 0;
     TailLevel* d_tail_levels = nullptr;
     // unsharp stage. Calm route: the fused level-0 collapse stores the frame and only the strip chunks that can reach the
@@ -122,8 +124,6 @@ struct poppy_cuda_ctx {
     // every pixel. 0 = adaptive (the calm route while the share of flagged chunks seen on recent frames stays low, the dense
     // route otherwise, probing the calm route now and then); 1 = dense always (forced by keep_stages); 2 = calm always.
     int unsharp_mode = 0;
-    int l0_group = 0;                        // POPPY_CUDA_L0_GROUP: frames per (level-0 collapse, unsharp) launch pair of the dense route
-    int l0_chunk_rows = 0;                   // POPPY_CUDA_US_ROWS: rows per CTA of the dense unsharp pass (0: 216)
     double calm_share = 1.0;                 // running share of flagged strip chunks (starts pessimistic: dense until a scan says otherwise)
     unsigned route_tick = kCalmProbeEvery - 1;   // the first dense chunk carries a scan
     unsigned probe_every = kCalmProbeEvery;
@@ -231,7 +231,7 @@ int ensure_chunk(poppy_cuda_ctx* c) {
     }
     want = std::max(1, std::min(want, c->max_frames));
     // a second lane only pays when a render spans several chunks
-    const int lanes = (c->keep_stages || c->single_lane || want >= c->max_frames) ? 1 : c->want_lanes;
+    const int lanes = (c->keep_stages || want >= c->max_frames) ? 1 : kRenderLanes;
     if (c->chunk == want && c->n_lanes == lanes) return 0;
     CU_TRY(c, cudaStreamSynchronize(c->stream));
     for (auto& l : c->lane) if (l.stream) CU_TRY(c, cudaStreamSynchronize(l.stream));
@@ -273,30 +273,33 @@ int ensure_chunk(poppy_cuda_ctx* c) {
         CU_TRY(c, dmalloc(&c->d_tail_levels, tl.size()));
         CU_TRY(c, cudaMemcpy(c->d_tail_levels, tl.data(), tl.size() * sizeof(TailLevel), cudaMemcpyHostToDevice));
     }
-    // tensor maps of every level's collapse (level k fine, level k+1 coarse); a level whose maps cannot be built keeps
-    // the per-warp staging kernel
+    // tensor maps of every level's collapse (level k fine, level k+1 coarse). A level too small for the boxes keeps an
+    // all-zero entry and runs k_collapse_roll: it has no interior tile.
     for (int i = 0; i < lanes; ++i) {
         auto& l = c->lane[i];
         l.maps.assign(c->levels, CollapseMaps());
-        bool ok = true;
-        for (int k = 0; k < c->levels && ok; ++k) {
+        for (int k = 0; k < c->levels; ++k) {
             const LevelDesc &fl = c->lv[k], &cl = c->lv[k + 1];
             CollapseMaps& m = l.maps[k];
+            bool ok;
             if (k == 0) {
                 ok = make_plane_map(&m.fine, l.d_warped, c->pitch0(), c->h, c->padded_pixels(), 2 * B, 128, 2, 2) &&
                      make_plane_map(&m.mask, l.d_mask0, c->pitch0(), c->h, c->padded_pixels(), B, 128, 2, 1);
             } else {
-                // levels too small for a 128 x 2 box have no interior tile anyway; keep the box inside the tensor
-                if (fl.pitch < 128 || fl.h < 2) { m = CollapseMaps(); continue; }
+                // keep the 128 x 2 box inside the tensor
+                if (fl.pitch < 128 || fl.h < 2) continue;
                 ok = make_plane_map(&m.fine, g_level(c, l, k), fl.pitch, fl.h, fl.plane_stride, 7 * B, 128, 2, 7);
                 m.mask = m.fine;
             }
-            if (!ok) break;
-            if (cl.pitch < 72) { m = CollapseMaps(); continue; }
-            ok = make_plane_map(&m.gc, g_level(c, l, k + 1), cl.pitch, cl.h, cl.plane_stride, 7 * B, 72, 1, 6) &&
+            if (ok && cl.pitch < 72) { m = CollapseMaps(); continue; }
+            ok = ok && make_plane_map(&m.gc, g_level(c, l, k + 1), cl.pitch, cl.h, cl.plane_stride, 7 * B, 72, 1, 6) &&
                  make_plane_map(&m.oc, o_level(c, l, k + 1), cl.pitch, cl.h, cl.plane_stride, 3 * B, 72, 1, 3);
+            if (!ok) {
+                free_chunk(c);       // the next render retries instead of running without the maps
+                return fail(c, POPPY_CUDA_ERR_CUDA, "cuTensorMapEncodeTiled %s for the collapse of level %d",
+                            tensor_map_encoder() ? "failed" : "is not available from the driver", k);
+            }
         }
-        if (!ok) l.maps.clear();
     }
     return 0;
 }
@@ -475,21 +478,13 @@ int render_chunk(poppy_cuda_ctx* c, int slot0, int first, int nb, const float* s
                                  ln.d_chunk_flags);
         }
     } else {
-        // Dense route in groups of `l0_group` frames: the level-0 collapse of a group writes lapBlend into one small scratch
-        // that the unsharp kernel reads right away and the next group overwrites, so the 12 B/px planes live in the 126 MB L2
-        // instead of crossing HBM twice (0: one launch pair for the whole chunk).
-        const int G = (c->l0_group > 0 && c->l0_group < nb) ? c->l0_group : nb;
-        const size_t pp = c->padded_pixels();
-        for (int f0 = 0; f0 < nb; f0 += G) {
-            const int n = std::min(G, nb - f0);
-            {   Scope s(c, KC_COLLAPSE, st);
-                launch_collapse0(st, ln.d_warped + (size_t)f0 * 2 * pp, c->pitch0(), pp, ln.d_mask0 + (size_t)f0 * pp, c->pitch0(), pp, w, h,
-                                 g_level(c, ln, 1) + (size_t)f0 * 7 * c->lv[1].plane_stride, o_level(c, ln, 1) + (size_t)f0 * 3 * c->lv[1].plane_stride,
-                                 c->lv[1], o_level(c, ln, 0), c->lv[0], n, nullptr, level_maps(ln, 0), f0);
-            }
-            {   Scope s(c, KC_UNSHARP, st);
-                launch_unsharp_store(st, o_level(c, ln, 0), c->lv[0], ln.d_fp + f0, c->d_frames, c->frame_bytes(), n, c->l0_chunk_rows, nullptr);
-            }
+        // dense route: the level-0 collapse of the whole chunk to float planes, then the exact unsharp pass on every pixel
+        {   Scope s(c, KC_COLLAPSE, st);
+            launch_collapse0(st, ln.d_warped, c->pitch0(), c->padded_pixels(), ln.d_mask0, c->pitch0(), c->padded_pixels(), w, h,
+                             g_level(c, ln, 1), o_level(c, ln, 1), c->lv[1], o_level(c, ln, 0), c->lv[0], nb, nullptr, level_maps(ln, 0));
+        }
+        {   Scope s(c, KC_UNSHARP, st);
+            launch_unsharp_store(st, o_level(c, ln, 0), c->lv[0], ln.d_fp, c->d_frames, c->frame_bytes(), nb, 0, nullptr);
         }
         c->dense_chunks_total += (uint64_t)nb * chunks_per_frame;
         if (c->unsharp_mode == 0 && !c->keep_stages && (++c->route_tick % c->probe_every) == 0 && !ln.calm_pending) {
@@ -544,10 +539,6 @@ int poppy_cuda_create(poppy_cuda_ctx** out, int device, int width, int height, i
     poppy_cuda_ctx* c = new poppy_cuda_ctx();
     c->device = device; c->w = width; c->h = height; c->levels = pyramid_levels;
     c->max_points = max_points; c->max_tri = max_triangles; c->max_frames = max_batch_frames;
-    if (const char* e = std::getenv("POPPY_CUDA_SINGLE_LANE")) c->single_lane = e[0] == '1';   // A/B switch for profiling
-    if (const char* e = std::getenv("POPPY_CUDA_LANES")) c->want_lanes = std::max(1, std::min(8, std::atoi(e)));
-    if (const char* e = std::getenv("POPPY_CUDA_L0_GROUP")) c->l0_group = std::max(0, std::atoi(e));
-    if (const char* e = std::getenv("POPPY_CUDA_US_ROWS")) c->l0_chunk_rows = std::max(0, std::atoi(e)) / 8 * 8;
     auto bail = [&](int rc) { g_create_error = c->err; poppy_cuda_destroy(c); return rc; };
 #define CR_TRY(expr) do { cudaError_t e_ = (expr); if (e_ != cudaSuccess) { \
         fail(c, POPPY_CUDA_ERR_CUDA, "%s failed: %s", #expr, cudaGetErrorString(e_)); return bail(POPPY_CUDA_ERR_CUDA); } } while (0)
@@ -579,12 +570,8 @@ int poppy_cuda_create(poppy_cuda_ctx** out, int device, int width, int height, i
         lw = (lw + 1) / 2; lh = (lh + 1) / 2;
     }
     // the pyramid's tail: from the first level no larger than 32 x 32 on, all levels run in one launch
-    {
-        const char* e = std::getenv("POPPY_CUDA_TAIL");
-        if (!(e && e[0] == '0'))
-            for (int k = 1; k < pyramid_levels; ++k)
-                if (c->lv[k].w <= 32 && c->lv[k].h <= 32) { c->tail_k0 = k; break; }
-    }
+    for (int k = 1; k < pyramid_levels; ++k)
+        if (c->lv[k].w <= 32 && c->lv[k].h <= 32) { c->tail_k0 = k; break; }
     // triangle binning: 64x32 screen tiles; list capacity per frame (a frame that needs more falls back to testing
     // every triangle in every tile, see k_raster_warp)
     {

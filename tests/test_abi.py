@@ -54,6 +54,20 @@ def test_product_does_not_reference_the_oracle():
     assert not bad, bad
 
 
+def test_library_reads_no_environment_variables():
+    """The native library and its integration layer have no hidden run-time switches: nothing under
+    poppy_b200/csrc/, include/ or integration/ calls getenv."""
+    bad = []
+    for top in ("poppy_b200/csrc", "include", "integration"):
+        for base, _, files in os.walk(os.path.join(ROOT, top)):
+            for f in files:
+                if f.endswith((".cu", ".cuh", ".cpp", ".hpp", ".h", ".c")):
+                    path = os.path.join(base, f)
+                    if re.search(r"\b(secure_)?getenv\s*\(", open(path, errors="replace").read()):
+                        bad.append(os.path.relpath(path, ROOT))
+    assert not bad, bad
+
+
 def test_kernels_are_compiled_for_sm_100a(native_lib):
     import shutil
     import subprocess

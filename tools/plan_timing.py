@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Host planning throughput (Delaunay per frame) for thread counts / POPPY_PLAN_WAYS. usage: plan_timing.py frames threads"""
+"""Host planning throughput (Delaunay per frame) for a thread count. usage: plan_timing.py frames threads"""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -11,4 +11,4 @@ best = 1e9
 for _ in range(2):
     t = time.perf_counter(); p = host.SequencePlan(inp.pts1, inp.pts2, c["w"], c["h"], ph, threads=thr); dt = time.perf_counter() - t; p.close()
     best = min(best, dt)
-print(f"ways={os.environ.get('POPPY_PLAN_WAYS','1')} threads={thr} frames={F}: {best:.3f} s -> {F/best:.1f} frames/s", flush=True)
+print(f"threads={thr} frames={F}: {best:.3f} s -> {F/best:.1f} frames/s", flush=True)
