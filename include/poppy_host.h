@@ -95,7 +95,10 @@ void poppy_host_writer_destroy(poppy_host_writer* w);
 /* The C++ shim (poppy_b200/csrc/host/morph_images.hpp: poppy::Settings, poppy::morph_images, poppy::morph_sequence with
  * the reference's argument order and semantics) behind C entry points, for callers and tests without a C++ toolchain:
  * the shim keeps its own device context (per frame size / pyramid levels), runs the host stages and, for a sequence, the
- * sliced chain render + writer ring; `write` receives the frames in order (reference src/poppy.hpp:177-243). */
+ * sliced chain render + writer ring; `write` receives the frames in order (reference src/poppy.hpp:177-243).
+ * poppy_shim_morph_sequence takes gabor2 == NULL (gstep ignored): gabor2 is then derived on the device from corrected2, as
+ * poppy::morph() derives it before its frame loop (src/poppy.hpp:119-122; poppy_cuda_set_pair). The per-frame entry points
+ * keep requiring gabor2, as the reference's morph_images() does. */
 int poppy_shim_morph_images(int width, int height, int pyramid_levels, const uint8_t* corrected1, size_t step1,
                             const uint8_t* corrected2, size_t step2, const float* gabor2, size_t gstep,
                             const float* src_points1_xy, const float* src_points2_xy, int n, double shape_ratio,

@@ -48,6 +48,12 @@ void launch_bin_triangles(cudaStream_t st, const TriRaster* rast, const FramePar
 void launch_bgr_to_bgrx(cudaStream_t st, const uint8_t* bgr, uchar4* out, int w, int h);
 // mask basis m2 = 1 - gray(gabor2)  (reference src/algo.cpp:250-252), rows `bpitch` floats apart
 void launch_mask_basis(cudaStream_t st, const float* gabor_bgr, float* m2, int bpitch, int w, int h);
+
+// ---- margin.cu ---------------------------------------------------------------------------------------------------
+// the same basis derived from the 8-bit corrected2 (BGR, tight rows) as the reference derives gabor2 from it:
+// 1 - gray(gabor_filter(corrected2 * 1/255)) with the default Gabor parameters (reference src/poppy.hpp:119-122); the first
+// call on a device uploads the filter taps and synchronises `st`
+cudaError_t launch_gabor_mask_basis(cudaStream_t st, const uint8_t* bgr, float* m2, int bpitch, int w, int h);
 // paint_triangles + create_map + remap for both images, one CTA per 64x32 screen tile (reference src/algo.cpp:95-106,
 // 146-176, 232-238). warped: per frame two planes of packed BGRX words (remap of image 1, of image 2), rows `wpitch`
 // words apart, `wstride` words per plane; tri_map_out (nullable) receives frame 0's ID map. src1/src2: point-sampled,

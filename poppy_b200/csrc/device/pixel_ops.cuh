@@ -18,6 +18,15 @@ __device__ __forceinline__ float unit_from_byte(uint32_t word, int c) {
     return fmaf(m, kInv255, -8388608.0f * kInv255);
 }
 
+// m2 = 1 - gray(gabor2) of one pixel, the mask basis (reference src/algo.cpp:250-252). RGB2Gray<float>
+// (OCV imgproc/src/color_rgb.simd.hpp:594-642) runs per row: the 8-lane vector body evaluates fma(r,cr, fma(g,cg, b*cb));
+// the scalar tail (last w%8 pixels) is contracted to fma(r,cr, fma(b,cb, g*cg)). body: x < (w & ~7).
+__device__ __forceinline__ float mask_basis_px(float b, float g, float r, bool body) {
+    const float gray = body ? fmaf(r, 0.299f, fmaf(g, 0.587f, __fmul_rn(b, 0.114f)))
+                            : fmaf(r, 0.299f, fmaf(b, 0.114f, __fmul_rn(g, 0.587f)));
+    return __fsub_rn(1.0f, gray);
+}
+
 // lbmask of one pixel (reference src/algo.cpp:255-258): addWeighted(ones, 1-mr, m2, -mr) evaluates
 // alpha + round(m2 * beta) in double and narrows (OCV core/src/arithm.simd.hpp:1161-1204,1721-1730), then the two
 // setTo() clamps.

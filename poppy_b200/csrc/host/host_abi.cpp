@@ -281,11 +281,11 @@ int poppy_shim_morph_images(int w, int h, int pyramid_levels, const uint8_t* c1,
 int poppy_shim_morph_sequence(int w, int h, int pyramid_levels, const uint8_t* c1, size_t step1, const uint8_t* c2, size_t step2,
                               const float* gabor2, size_t gstep, const float* sp1, const float* sp2, int n, int n_frames,
                               poppy_write_fn write, void* user) {
-    if (!c1 || !c2 || !gabor2 || !write || n < 0 || (n > 0 && (!sp1 || !sp2))) return host_fail(POPPY_CUDA_ERR_INVALID, "null argument");
+    if (!c1 || !c2 || !write || n < 0 || (n > 0 && (!sp1 || !sp2))) return host_fail(POPPY_CUDA_ERR_INVALID, "null argument");
     return shim_guard([&] {
         poppy::Settings::instance().pyramid_levels = (size_t)pyramid_levels;
-        poppy::Image32F g;
-        g.data = gabor2; g.cols = w; g.rows = h; g.step = gstep;
+        poppy::Image32F g;             // gabor2 == NULL: empty, derived on the device
+        if (gabor2) { g.data = gabor2; g.cols = w; g.rows = h; g.step = gstep; }
         int index = 0;
         poppy::morph_sequence(view8(c1, w, h, step1), view8(c2, w, h, step2), g, to_points(sp1, n), to_points(sp2, n), n_frames,
                               [&](const poppy::Image8& f) { write(user, index++, f.data, f.cols, f.rows, f.step); });

@@ -5,6 +5,7 @@
 #include <memory>
 #include <mutex>
 #include <thread>
+#include <utility>
 
 #include "../../../include/poppy_host.h"
 
@@ -66,6 +67,8 @@ double morph_images(const Image8& img1, const Image8& /*img2*/, const Image8& co
     if (corrected1.cols != w || corrected1.rows != h || corrected2.cols != w || corrected2.rows != h ||
         gabor2.cols != w || gabor2.rows != h)
         throw MorphError("morph_images: image sizes differ");
+    // per frame, gabor2 is the caller's (the reference's signature); deriving it here would repeat the filter every frame
+    if (!gabor2.data) throw MorphError("morph_images: gabor2 is empty");
     if (srcPoints1.size() != srcPoints2.size()) throw MorphError("morph_images: point sets differ in size");
     const int n = (int)srcPoints1.size();
 
@@ -126,6 +129,7 @@ void morph_sequence(const Image8& corrected1, const Image8& corrected2, const Im
 
     std::lock_guard<std::mutex> lock(g_mu);
     poppy_cuda_ctx* c = context_for(w, h, (int)Settings::instance().pyramid_levels, n, max_tri, N);
+    // gabor2.data == nullptr: set_pair derives the mask basis from corrected2
     cu(c, poppy_cuda_set_pair(c, corrected1.data, corrected1.step, corrected2.data, corrected2.step, gabor2.data, gabor2.step));
     cu(c, poppy_cuda_set_points(c, p1, p2, n));
     // The chain is rendered slice by slice (frame j-1 stays in HBM as frame j's source across the calls) and every finished
@@ -150,6 +154,11 @@ void morph_sequence(const Image8& corrected1, const Image8& corrected2, const Im
         if (poppy_host_writer_submit(wr, a, cnt, a) != 0) throw MorphError(std::string("morph_sequence: ") + poppy_cuda_last_error(c));
     }
     if (poppy_host_writer_flush(wr) != 0) throw MorphError("morph_sequence: a frame download failed");
+}
+
+void morph_sequence(const Image8& corrected1, const Image8& corrected2, std::vector<Point2f> srcPoints1,
+                    std::vector<Point2f> srcPoints2, int number_of_frames, const std::function<void(const Image8&)>& write) {
+    morph_sequence(corrected1, corrected2, Image32F(), std::move(srcPoints1), std::move(srcPoints2), number_of_frames, write);
 }
 
 }  // namespace poppy

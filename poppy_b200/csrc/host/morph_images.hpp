@@ -80,10 +80,14 @@ double morph_images(const Image8& img1, const Image8& img2, const Image8& correc
 
 // The frame loop of morph<Twriter>() (reference src/poppy.hpp:177-243, phase < 0) with the whole segment resident
 // on the GPU: points/topology of all frames are planned on host threads, the chain is rendered with frame j-1 kept
-// in HBM as frame j's source, and frames are handed to `write` in order.
+// in HBM as frame j's source, and frames are handed to `write` in order. An empty gabor2 (data == nullptr) has the
+// device derive it from corrected2, as poppy::morph() does before its frame loop (src/poppy.hpp:119-122).
 void morph_sequence(const Image8& corrected1, const Image8& corrected2, const Image32F& gabor2,
                     std::vector<Point2f> srcPoints1, std::vector<Point2f> srcPoints2, int number_of_frames,
                     const std::function<void(const Image8&)>& write);
+// The same with gabor2 derived on the device from corrected2: only the two 8-bit images cross PCIe.
+void morph_sequence(const Image8& corrected1, const Image8& corrected2, std::vector<Point2f> srcPoints1,
+                    std::vector<Point2f> srcPoints2, int number_of_frames, const std::function<void(const Image8&)>& write);
 
 // Releases the cached device context(s) held by morph_images()/morph_sequence().
 void release_cached_contexts();

@@ -60,7 +60,7 @@ struct poppy_cuda_ctx {
     bool have_pair = false, have_points = false;
     bool have_image[3] = {false, false, false};
     uint8_t* d_stage_u8 = nullptr;       // upload staging of set_image, kept between calls
-    float* d_stage_f32 = nullptr;
+    float* d_stage_f32 = nullptr;        // only for a caller-supplied gabor2 (selector 2)
     int n_points = 0, last_frames = 0;
     int chain_next_slot = -1;            // ring slot at which a sliced chain render may continue (-1: no chain in progress)
     std::vector<cudaEvent_t> tickets;    // download tickets (poppy_cuda_download_async), indexed ticket % size
@@ -710,31 +710,39 @@ int poppy_cuda_set_stage_timing(poppy_cuda_ctx* c, int enable) {
     return 0;
 }
 
-// upload staging of the pair, allocated on first use and kept (no cudaMalloc / cudaFree per call)
-static int ensure_pair_staging(poppy_cuda_ctx* c) {
-    if (!c->d_stage_u8) CU_TRY(c, dmalloc(&c->d_stage_u8, c->frame_bytes()));
-    if (!c->d_stage_f32) CU_TRY(c, dmalloc(&c->d_stage_f32, c->pixels() * 3));
+// upload staging of the pair, allocated on first use and kept (no cudaMalloc / cudaFree per call): 8-bit for the images,
+// float (99.5 MB at 4K) only once a caller supplies gabor2 itself
+static int ensure_pair_staging(poppy_cuda_ctx* c, int which) {
+    if (which != 2 && !c->d_stage_u8) CU_TRY(c, dmalloc(&c->d_stage_u8, c->frame_bytes()));
+    if (which == 2 && !c->d_stage_f32) CU_TRY(c, dmalloc(&c->d_stage_f32, c->pixels() * 3));
     return 0;
 }
 
 int poppy_cuda_set_image(poppy_cuda_ctx* c, int which, const void* data, size_t step) {
     if (!c) return POPPY_CUDA_ERR_INVALID;
-    if (!data || which < 0 || which > 2) return fail(c, POPPY_CUDA_ERR_INVALID, "bad image selector or null pointer");
+    if (!data || which < 0 || which > 3) return fail(c, POPPY_CUDA_ERR_INVALID, "bad image selector or null pointer");
     const size_t row = (size_t)c->w * 3, grow = row * sizeof(float), trow = (size_t)c->w * 4;
     if (step < (which == 2 ? grow : row)) return fail(c, POPPY_CUDA_ERR_INVALID, "row stride smaller than a row");
     CU_TRY(c, cudaSetDevice(c->device));
-    if (int rc = ensure_pair_staging(c)) return rc;
-    if (which < 2) {
+    if (int rc = ensure_pair_staging(c, which)) return rc;
+    if (which != 2) {
         CU_TRY(c, cudaMemcpy2DAsync(c->d_stage_u8, row, data, step, row, c->h, cudaMemcpyHostToDevice, c->stream));
         launch_bgr_to_bgrx(c->stream, c->d_stage_u8, c->d_src_stage, c->w, c->h);
-        CU_TRY(c, cudaMemcpy2DToArrayAsync(c->a_src[which], 0, 0, c->d_src_stage, trow, trow, c->h, cudaMemcpyDeviceToDevice, c->stream));
+        CU_TRY(c, cudaMemcpy2DToArrayAsync(c->a_src[which == 0 ? 0 : 1], 0, 0, c->d_src_stage, trow, trow, c->h,
+                                           cudaMemcpyDeviceToDevice, c->stream));
     } else {
         CU_TRY(c, cudaMemcpy2DAsync(c->d_stage_f32, grow, data, step, grow, c->h, cudaMemcpyHostToDevice, c->stream));
         launch_mask_basis(c->stream, c->d_stage_f32, c->d_mbasis, c->pitch0(), c->w, c->h);
     }
     c->launches++; c->class_launches[KC_MISC]++;
     CU_TRY(c, cudaGetLastError());
-    c->have_image[which] = true;
+    if (which == 3) {
+        // corrected2 is still in the 8-bit staging (same stream): the mask basis from it, gabor2 never stored
+        Scope s(c, KC_MISC, c->stream);
+        CU_TRY(c, launch_gabor_mask_basis(c->stream, c->d_stage_u8, c->d_mbasis, c->pitch0(), c->w, c->h));
+        c->have_image[1] = true;
+    }
+    c->have_image[which == 3 ? 2 : which] = true;
     c->have_pair = c->have_image[0] && c->have_image[1] && c->have_image[2];
     return 0;
 }
@@ -742,11 +750,12 @@ int poppy_cuda_set_image(poppy_cuda_ctx* c, int which, const void* data, size_t 
 int poppy_cuda_set_pair(poppy_cuda_ctx* c, const uint8_t* bgr1, size_t step1, const uint8_t* bgr2, size_t step2,
                         const float* gabor, size_t gstep) {
     if (!c) return POPPY_CUDA_ERR_INVALID;
-    if (!bgr1 || !bgr2 || !gabor) return fail(c, POPPY_CUDA_ERR_INVALID, "null image pointer");
+    if (!bgr1 || !bgr2) return fail(c, POPPY_CUDA_ERR_INVALID, "null image pointer");
     int rc;
-    if ((rc = poppy_cuda_set_image(c, 0, bgr1, step1)) != 0 || (rc = poppy_cuda_set_image(c, 1, bgr2, step2)) != 0 ||
-        (rc = poppy_cuda_set_image(c, 2, gabor, gstep)) != 0)
-        return rc;
+    if ((rc = poppy_cuda_set_image(c, 0, bgr1, step1)) != 0) return rc;
+    if (!gabor) rc = poppy_cuda_set_image(c, 3, bgr2, step2);      // no gabor2: derive the mask basis from corrected2
+    else if ((rc = poppy_cuda_set_image(c, 1, bgr2, step2)) == 0) rc = poppy_cuda_set_image(c, 2, gabor, gstep);
+    if (rc != 0) return rc;
     // the host arrays may be pinned (a truly asynchronous copy) and reused by the caller right after this call
     CU_TRY(c, cudaStreamSynchronize(c->stream));
     return 0;
@@ -1040,6 +1049,16 @@ int poppy_cuda_stage_times(poppy_cuda_ctx* c, const char** names, float* ms, uin
 int poppy_cuda_debug_read(poppy_cuda_ctx* c, int stage, int frame, void* dst, size_t bytes) {
     if (!c) return POPPY_CUDA_ERR_INVALID;
     if (!dst) return fail(c, POPPY_CUDA_ERR_INVALID, "dst is null");
+    if (stage == POPPY_STAGE_MASK_BASIS) {     // a property of the pair, not of a frame
+        if (!c->keep_stages) return fail(c, POPPY_CUDA_ERR_STATE, "stage buffers need set_keep_stages(1)");
+        if (!c->have_image[2]) return fail(c, POPPY_CUDA_ERR_STATE, "no mask basis: set_pair or set_image(2 or 3) first");
+        if (bytes != c->pixels() * 4)
+            return fail(c, POPPY_CUDA_ERR_INVALID, "stage %d holds %zu bytes, caller gave %zu", stage, c->pixels() * 4, bytes);
+        CU_TRY(c, cudaSetDevice(c->device));
+        CU_TRY(c, cudaStreamSynchronize(c->stream));
+        CU_TRY(c, cudaMemcpy2D(dst, (size_t)c->w * 4, c->d_mbasis, (size_t)c->pitch0() * 4, (size_t)c->w * 4, c->h, cudaMemcpyDeviceToHost));
+        return 0;
+    }
     if (!c->keep_stages || c->chunk != 1) return fail(c, POPPY_CUDA_ERR_STATE, "stage buffers need set_keep_stages(1) before render");
     if (frame != c->last_frames - 1 && stage != POPPY_STAGE_MORPHED_POINTS)
         return fail(c, POPPY_CUDA_ERR_STATE, "only the last rendered frame's stage buffers are resident");
