@@ -654,8 +654,8 @@ __device__ __forceinline__ void fine_from_rows(float4 l, float4 r, float4 m, Fin
 // unsharp_mask() leaves a pixel untouched unless the 3x3 median of d = x - GaussianBlur(x, sigma 1) reaches norm 0.3
 // (src/util.cpp:135-145). With the symmetric 9-tap kernel, d = (I - Bx) x + Bx (I - By) x and
 //     (I - Bx) x (p) = - sum_{a>0} w_a [x(p+a) + x(p-a) - 2 x(p)],   |x(p+a) + x(p-a) - 2 x(p)| <= a^2 max |d2x|,
-// so |d| <= 0.5 (max |d2x| + max |d2y|) over the pixel's footprint (sum_{a>0} w_a a^2 = 0.49996), d2 being the unit second
-// differences of x (reflected at the image border like the blur). Where that bound stays below 0.1732 in every channel no
+// so |d| <= 0.5 (max |d2x| + max |d2y|) over the pixel's footprint (sum_{a>0} w_a a^2 = 0.499964 <= 0.49997), d2 being
+// the unit second differences of x (reflected at the image border like the blur). Where that bound stays below 0.1732 in every channel no
 // median can reach the threshold (3 * 0.1732^2 < 0.09) and the frame pixel is exactly cvRound(255 x): neither blur nor
 // median have to be evaluated. The level-0 collapse therefore stores the 8-bit frame itself; k_calm_scan
 // (kernels_unsharp.cu) bounds the second differences from the stored bytes (|x - byte/255| <= 0.5/255 unless x was clamped,

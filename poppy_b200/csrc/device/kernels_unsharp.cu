@@ -414,11 +414,11 @@ __global__ void k_checksum(const uint8_t* __restrict__ data, size_t bytes, unsig
 // where the block's clamp excess is tolerated), so the second differences of x are below (2 h + 3.02) / 255. A pixel is
 // calm when, over the blocks within 2 block columns / 1 block row (8 pixels each way; its median + blur footprint spans 5
 // columns and 4 rows of second differences), max hx + max hy <= CALM_SUM: then
-//     |x - blur| <= 0.49996 ((2 hx + 3.02) + (2 hy + 3.02)) / 255 + rounding (< 1e-5) < 0.1732,
+//     |x - blur| <= 0.49997 ((2 hx + 3.02) + (2 hy + 3.02)) / 255 + rounding (< 1e-5) < 0.1732,
 // and no 3x3 median can reach norm 0.3 (3 * 0.1732^2 < 0.09).
 constexpr int CALM_SUM = 40;
 static_assert(UNSHARP_STRIP_W == US_W, "strip width");
-static_assert((2 * CALM_SUM + 2 * 3.02) / 255.0 * 0.49996 < 0.1731, "calm bound");
+static_assert((2 * CALM_SUM + 2 * 3.02) / 255.0 * 0.49997 < 0.1731, "calm bound");
 
 // |floor-avg(a, c) - b| of four bytes at once
 __device__ __forceinline__ unsigned calm_dev4(unsigned a, unsigned b, unsigned c) {
