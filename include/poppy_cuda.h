@@ -138,6 +138,35 @@ int poppy_cuda_set_plan(poppy_cuda_ctx* ctx, const int32_t* tri_idx, const int32
 int poppy_cuda_render_planned(poppy_cuda_ctx* ctx, int first_slot, int plan_first, int n_frames, const float* shape_ratio,
                               const double* mask_ratio, int chain);
 
+/* ---- segments of a multi-image sequence ---------------------------------------------------------------------------------
+ * The reference's run() (src/poppy.cpp:266-328) morphs each consecutive pair of a list of images as one segment: a chain of
+ * number_of_frames frames (src/poppy.hpp:177-243). Segments have the same frame size and depend on no rendered frame of
+ * each other, so they can be rendered together: a kernel batch holds step j of up to chunk-frames segments, and the
+ * launches per step do not grow with the number of segments. This state lives beside the single pair and leaves it,
+ * the points and the resident plan as they are.
+ *
+ * poppy_cuda_set_segments: room for n_segments segments (each with its own corrected1, corrected2, chain source, mask
+ * basis and point sets in HBM) and a ring window of `window` slots per segment: step j of segment s lands in ring slot
+ * s * window + j % window. window >= 2 (step j reads step j-1's points); n_segments * window <= max_batch_frames
+ * (POPPY_CUDA_ERR_CAPACITY). Replaces any earlier segments.
+ * poppy_cuda_set_segment: poppy_cuda_set_pair + poppy_cuda_set_points for segment s (gabor2 == NULL: the mask basis is
+ * derived from corrected2 on the device); n <= max_points. Synchronous. */
+int poppy_cuda_set_segments(poppy_cuda_ctx* ctx, int n_segments, int window);
+int poppy_cuda_set_segment(poppy_cuda_ctx* ctx, int s, const uint8_t* bgr1, size_t step1, const uint8_t* bgr2, size_t step2,
+                           const float* gabor2_bgr32f, size_t gstep, const float* pts1_xy, const float* pts2_xy, int n);
+/* Render steps [first_step, first_step + n_steps) of every segment as chains (frame j from frame j-1 and its morphed
+ * points). shape_ratio / mask_ratio: one entry per step, indexed from 0 for the call. tri_offsets has n_steps * K + 1
+ * entries: the list of step first_step + r of segment s is entry r * K + s (step-major), with vertex indices into that
+ * segment's points (checked against its own n). A call with first_step > 0 continues where the previous segment render
+ * ended (POPPY_CUDA_ERR_STATE otherwise); every segment must have been set. Segments go in groups of at most chunk-frames
+ * segments; all steps of a group run on one render lane and the groups go round-robin over the lanes. Not on keep_stages
+ * contexts. Frames are read with the slot-based calls (download, checksum, frame_device_ptr); poppy_cuda_last_render_ms
+ * times the call. A pair render afterwards ends the segment render (and a segment render a sliced pair chain). */
+int poppy_cuda_render_segments(poppy_cuda_ctx* ctx, int first_step, int n_steps, const float* shape_ratio,
+                               const double* mask_ratio, const int32_t* tri_idx, const int32_t* tri_offsets);
+/* morphedPoints of step `step` of segment s (its own n x 2 float), while the step is still in the segment's window. */
+int poppy_cuda_get_segment_points(poppy_cuda_ctx* ctx, int s, int step, float* xy);
+
 /* Copy frames [first, first+count) (8UC3 BGR) to host memory: row stride `step` bytes, `frame_stride` bytes
  * between frames. Ordered after every render queued so far, on a separate copy stream (renders of other slots are not
  * held up; a render of slots with a download pending waits for it). Asynchronous if dst is pinned;

@@ -107,6 +107,22 @@ int poppy_shim_morph_sequence(int width, int height, int pyramid_levels, const u
                               const uint8_t* corrected2, size_t step2, const float* gabor2, size_t gstep,
                               const float* src_points1_xy, const float* src_points2_xy, int n, int number_of_frames,
                               poppy_write_fn write, void* user);
+/* The segments of a multi-image sequence (reference run(), src/poppy.cpp:266-328): segment i morphs one consecutive pair as
+ * poppy_shim_morph_sequence does, and all segments (same frame size) are rendered together. `write` receives the
+ * n_segments * number_of_frames frames in the reference's order: every frame of segment 0, then of segment 1, ... */
+typedef struct poppy_shim_segment {
+    const uint8_t* corrected1;
+    size_t step1;
+    const uint8_t* corrected2;
+    size_t step2;
+    const float* gabor2;          /* NULL: derived on the device from corrected2 */
+    size_t gstep;
+    const float* pts1_xy;
+    const float* pts2_xy;
+    int n;
+} poppy_shim_segment;
+int poppy_shim_morph_segments(int width, int height, int pyramid_levels, const poppy_shim_segment* segments, int n_segments,
+                              int number_of_frames, poppy_write_fn write, void* user);
 void poppy_shim_release(void);
 
 const char* poppy_host_last_error(void);

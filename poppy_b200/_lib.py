@@ -70,6 +70,11 @@ def load():
         "poppy_cuda_render_range": (i32, [vp, i32, i32, vp, vp, vp, vp, i32]),
         "poppy_cuda_set_plan": (i32, [vp, vp, vp, i32]),
         "poppy_cuda_render_planned": (i32, [vp, i32, i32, i32, vp, vp, i32]),
+        "poppy_cuda_set_segments": (i32, [vp, i32, i32]),
+        "poppy_cuda_set_segment": (i32, [vp, i32, vp, C.c_size_t, vp, C.c_size_t, vp, C.c_size_t, vp, vp, i32]),
+        "poppy_cuda_render_segments": (i32, [vp, i32, i32, vp, vp, vp, vp]),
+        "poppy_cuda_get_segment_points": (i32, [vp, i32, i32, vp]),
+        "poppy_shim_morph_segments": (i32, [i32, i32, i32, vp, i32, i32, vp, vp]),
         "poppy_cuda_download": (i32, [vp, i32, i32, vp, C.c_size_t, C.c_size_t]),
         "poppy_cuda_download_async": (i32, [vp, i32, i32, vp, C.c_size_t, C.c_size_t, u64p]),
         "poppy_cuda_download_wait": (i32, [vp, C.c_uint64]),
@@ -110,11 +115,12 @@ CUDA_ABI_SYMBOLS = [
     "poppy_cuda_unsharp_stats", "poppy_cuda_set_image", "poppy_cuda_set_source1_from_slot",
     "poppy_cuda_download_async", "poppy_cuda_download_wait", "poppy_cuda_alloc_pinned", "poppy_cuda_free_pinned",
     "poppy_cuda_blur_margin", "poppy_cuda_blur_margin_last_error", "poppy_cuda_gabor_filter",
+    "poppy_cuda_set_segments", "poppy_cuda_set_segment", "poppy_cuda_render_segments", "poppy_cuda_get_segment_points",
 ]
 HOST_ABI_SYMBOLS = [
     "poppy_host_morph_points", "poppy_host_triangulate", "poppy_host_triangulate_next", "poppy_host_chain_ratio", "poppy_host_plan_create",
     "poppy_host_plan_triangles", "poppy_host_plan_points", "poppy_host_plan_destroy", "poppy_morph_images",
     "poppy_host_last_error", "poppy_host_writer_create", "poppy_host_writer_create_io", "poppy_host_writer_submit",
     "poppy_host_writer_flush", "poppy_host_writer_destroy", "poppy_host_writer_destroy_cuda",
-    "poppy_shim_morph_images", "poppy_shim_morph_sequence", "poppy_shim_release",
+    "poppy_shim_morph_images", "poppy_shim_morph_sequence", "poppy_shim_morph_segments", "poppy_shim_release",
 ]

@@ -8,6 +8,8 @@
   morph_sequence(...)     the frame loop of poppy::morph<Twriter>() (reference src/poppy.hpp:177-243, phase < 0):
                           the chain recurrence kept resident on the GPU, frames handed to writer.write() in order
   render_phases(...)      direct mode: N independent phases of one pair ("-f 1 -p s", src/poppy.hpp:186-200)
+  morph_segments(...)     the segments of a multi-image sequence (reference run(), src/poppy.cpp:266-328): one chain per
+                          consecutive pair, rendered together (step j of every segment in one kernel batch)
 
 morph_sequence and render_phases take gabor2=None: the GPU then derives it from corrected2 exactly as poppy::morph()
 does before its frame loop (gabor_filter(corrected2 * 1/255), src/poppy.hpp:119-122), and the float image never exists.
@@ -204,3 +206,62 @@ def render_phases(corrected1, corrected2, gabor2, src_points1, src_points2, phas
         return r.download(0, len(phases))
     finally:
         plan.close()
+
+
+def interleave_segment_plans(plans, n_steps):
+    """Triangle lists of chain plans in the step-major order of MorphRenderer.render_segments: entry j * K + s is step j of
+    segment s. Returns (tri_idx, tri_offsets)."""
+    K = len(plans)
+    counts = np.array([[p.tri_offsets[j + 1] - p.tri_offsets[j] for p in plans] for j in range(n_steps)], np.int64).reshape(-1)
+    offsets = np.zeros(n_steps * K + 1, np.int32)
+    np.cumsum(counts, out=offsets[1:])
+    parts = [plans[s].triangles(j) for j in range(n_steps) for s in range(K)]
+    tri = np.concatenate(parts).astype(np.int32, copy=False) if parts else np.zeros((0, 3), np.int32)
+    return tri.reshape(-1, 3), offsets
+
+
+# ring memory one morph_segments batch may take: segments that do not fit are rendered in further batches
+_SEGMENT_RING_BYTES = 8 << 30
+
+
+def morph_segments(segments, number_of_frames=None, writer=None, threads=0):
+    """The segments of a multi-image sequence: segments[i] = (corrected1, corrected2, gabor2 or None, pts1, pts2) of one
+    consecutive pair, all of one frame size. Each is the chain morph_sequence renders, and they are rendered together.
+    Returns the frames as a (K, N, H, W, 3) array and calls writer.write(frame) in the reference's order: the N frames of
+    segment 0, then those of segment 1, and so on (one video, as run() writes it)."""
+    n_frames = int(number_of_frames if number_of_frames is not None else Settings.instance().number_of_frames)
+    K = len(segments)
+    if K == 0:
+        raise ValueError("morph_segments: no segments")
+    h, w = segments[0][0].shape[:2]
+    for c1, c2, _, p1, p2 in segments:
+        if c1.shape[:2] != (h, w) or c2.shape[:2] != (h, w):
+            raise ValueError("morph_segments: all segments must have the same frame size")
+        if np.shape(p1) != np.shape(p2):
+            raise ValueError("morph_segments: point sets differ in size")
+    ratio = np.array([host.chain_ratio(j, n_frames) for j in range(n_frames)], np.float64)
+    shape = ratio.astype(np.float32)
+    plans = [host.SequencePlan(np.reshape(p1, (-1, 2)), np.reshape(p2, (-1, 2)), w, h, shape, chain=True, threads=threads)
+             for _, _, _, p1, p2 in segments]
+    frames = np.empty((K, n_frames, h, w, 3), np.uint8)
+    try:
+        per_batch = max(1, min(K, _SEGMENT_RING_BYTES // (n_frames * w * h * 3)))
+        r = _renderer(w, h, max(p.n for p in plans), max(p.max_triangles for p in plans), per_batch * n_frames)
+        for b0 in range(0, K, per_batch):
+            batch = range(b0, min(K, b0 + per_batch))
+            r.set_segments(len(batch), n_frames)
+            for i, s in enumerate(batch):
+                c1, c2, g2, p1, p2 = segments[s]
+                r.set_segment(i, np.ascontiguousarray(c1), np.ascontiguousarray(c2), _optional(g2), np.reshape(p1, (-1, 2)),
+                              np.reshape(p2, (-1, 2)))
+            tri, offs = interleave_segment_plans([plans[s] for s in batch], n_frames)
+            r.render_segments(0, shape, ratio, tri, offs)
+            r.download(0, len(batch) * n_frames, out=frames[b0:b0 + len(batch)].reshape(-1, h, w, 3))
+    finally:
+        for p in plans:
+            p.close()
+    if writer is not None:
+        for seg in frames:
+            for f in seg:
+                writer.write(f)
+    return frames

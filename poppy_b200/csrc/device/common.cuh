@@ -23,6 +23,18 @@ struct FrameParams {
     int dst_slot;       // frame ring slot written by the last stage
 };
 
+// Per-frame inputs of a segment render (poppy_cuda_render_segments): a chunk holds one step of several segments, and
+// each frame reads its own segment's pair, mask basis and end points. Uploaded with the chunk's FrameParams.
+struct __align__(8) SegFrame {
+    cudaTextureObject_t src1;   // the segment's corrected1 at step 0, its chain array (the previous step's frame) after
+    cudaTextureObject_t src2;   // the segment's corrected2
+    const float* basis;         // the segment's mask basis, rows pitch0 floats apart
+    const float2* pts2;         // the segment's clipped pts2
+    int n_points;               // the segment's point count
+    int pad;
+};
+static_assert(sizeof(SegFrame) == 40, "SegFrame layout");
+
 // Raster record of one morphed triangle: integer vertices and the closed form of cv::FillConvexPoly's two edge
 // walkers (OCV imgproc/src/drawing.cpp:1093-1255). 64 bytes.
 struct __align__(16) TriRaster {

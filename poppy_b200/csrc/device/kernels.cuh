@@ -37,6 +37,14 @@ void launch_tri_geometry(cudaStream_t st, const int3* tri_idx, const FrameParams
                          size_t p1_frame_stride, const float2* p2, const float2* morphed, size_t morphed_frame_stride,
                          int max_tri, int tri_in_chunk_max, int frames, int img_w, int img_h, TriInverse* inv_out,
                          TriRaster* rast_out, int* tile_counts);
+// Segment renders: frame f of the chunk takes pts2 and its point count from seg[f] (n_max: the largest count of the chunk)
+void launch_lerp_points_seg(cudaStream_t st, const float2* p1, size_t p1_frame_stride, const SegFrame* seg,
+                            const FrameParams* fp, float2* out, size_t out_frame_stride, int n_max, int frames, int cols,
+                            int rows);
+void launch_tri_geometry_seg(cudaStream_t st, const int3* tri_idx, const FrameParams* fp, const float2* p1,
+                             size_t p1_frame_stride, const SegFrame* seg, const float2* morphed, size_t morphed_frame_stride,
+                             int max_tri, int tri_in_chunk_max, int frames, int img_w, int img_h, TriInverse* inv_out,
+                             TriRaster* rast_out, int* tile_counts);
 // tile_counts (frames x n_tiles, filled by launch_tri_geometry) -> tile_off (frames x (n_tiles+1)), overflow (frames),
 // tile_list (frames x cap)
 void launch_bin_triangles(cudaStream_t st, const TriRaster* rast, const FrameParams* fp, int max_tri, int tri_in_chunk_max,
@@ -46,6 +54,9 @@ void launch_bin_triangles(cudaStream_t st, const TriRaster* rast, const FramePar
 // ---- kernels_warp.cu ---------------------------------------------------------------------------------------------
 // BGR (3 bytes/px, tight rows) -> BGRX uchar4
 void launch_bgr_to_bgrx(cudaStream_t st, const uint8_t* bgr, uchar4* out, int w, int h);
+// every frame of a chunk: ring slot fp[f].dst_slot (BGR) -> out + f * w * h (BGRX)
+void launch_bgr_to_bgrx_frames(cudaStream_t st, const uint8_t* frames_base, size_t frame_bytes, const FrameParams* fp, uchar4* out,
+                               int w, int h, int frames);
 // mask basis m2 = 1 - gray(gabor2)  (reference src/algo.cpp:250-252), rows `bpitch` floats apart
 void launch_mask_basis(cudaStream_t st, const float* gabor_bgr, float* m2, int bpitch, int w, int h);
 
@@ -62,6 +73,10 @@ void launch_raster_warp(cudaStream_t st, const TriRaster* rast, const TriInverse
                         const int* tile_off, const int* tile_list, int cap, const int* overflow,
                         cudaTextureObject_t src1, cudaTextureObject_t src2, uint32_t* warped, int wpitch, size_t wstride, int* tri_map_out, int w, int h,
                         int frames);
+// the same with frame f sampling its segment's textures seg[f].src1 / seg[f].src2 (no ID-map dump)
+void launch_raster_warp_seg(cudaStream_t st, const TriRaster* rast, const TriInverse* inv, const FrameParams* fp, int max_tri,
+                            const int* tile_off, const int* tile_list, int cap, const int* overflow, const SegFrame* seg,
+                            uint32_t* warped, int wpitch, size_t wstride, int w, int h, int frames);
 
 // ---- kernels_pyramid.cu ------------------------------------------------------------------------------------------
 // level 0 -> 1: sources are the warped 8-bit pair (converted on the fly, algo.cpp:247-248) and the frame's blend
@@ -70,6 +85,10 @@ void launch_raster_warp(cudaStream_t st, const TriRaster* rast, const TriInverse
 void launch_pyr_down0(cudaStream_t st, const uint32_t* warped, int wpitch, size_t wstride, const float* basis, int bpitch,
                       const FrameParams* fp, int w, int h, float* mask0, size_t m0stride, float* dst, LevelDesc dl,
                       int frames);
+// the same with frame f's mask basis seg[f].basis (rows bpitch floats apart)
+void launch_pyr_down0_seg(cudaStream_t st, const uint32_t* warped, int wpitch, size_t wstride, const SegFrame* seg, int bpitch,
+                          const FrameParams* fp, int w, int h, float* mask0, size_t m0stride, float* dst, LevelDesc dl,
+                          int frames);
 // level k -> k+1 for the 7 planes (left BGR, right BGR, mask)
 void launch_pyr_down(cudaStream_t st, const float* src, LevelDesc sl, float* dst, LevelDesc dl, int frames);
 // Levels k0 .. L of a chunk in one launch (one CTA per frame): pyrDown k0 -> ... -> L, resultSmallest, collapse L-1 .. k0.

@@ -34,18 +34,35 @@ __device__ __forceinline__ float lerp_coord(float a, float b, float s) {
 }
 
 // grid (ceil(n/256), frames). Frame f reads p1 + f * p1_frame_stride (0: every frame starts from the same set)
-// and writes out + f * out_frame_stride.
-__global__ void k_lerp_points(const float2* __restrict__ p1, size_t p1_frame_stride, const float2* __restrict__ p2,
-                              const FrameParams* __restrict__ fp, float2* __restrict__ out, size_t out_frame_stride, int n,
-                              int cols, int rows) {
+// and writes out + f * out_frame_stride. SEG: frame f's pts2 and point count are its segment's (seg[f]); n is their maximum.
+template <bool SEG>
+__device__ __forceinline__ void lerp_points_body(const float2* __restrict__ p1, size_t p1_frame_stride, const float2* __restrict__ p2,
+                                                 const FrameParams* __restrict__ fp, const SegFrame* __restrict__ seg,
+                                                 float2* __restrict__ out, size_t out_frame_stride, int n, int cols, int rows) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     int f = blockIdx.y;
+    if (SEG) {
+        n = seg[f].n_points;
+        p2 = seg[f].pts2;
+    }
     if (i >= n) return;
     float s = fp[f].shape;
     float2 a = p1[(size_t)f * p1_frame_stride + i], b = p2[i], r;
     r.x = lerp_coord(a.x, b.x, s);
     r.y = lerp_coord(a.y, b.y, s);
     out[(size_t)f * out_frame_stride + i] = clip_point(r, cols, rows);
+}
+
+__global__ void k_lerp_points(const float2* __restrict__ p1, size_t p1_frame_stride, const float2* __restrict__ p2,
+                              const FrameParams* __restrict__ fp, float2* __restrict__ out, size_t out_frame_stride, int n,
+                              int cols, int rows) {
+    lerp_points_body<false>(p1, p1_frame_stride, p2, fp, nullptr, out, out_frame_stride, n, cols, rows);
+}
+
+__global__ void k_lerp_points_seg(const float2* __restrict__ p1, size_t p1_frame_stride, const SegFrame* __restrict__ seg,
+                                  const FrameParams* __restrict__ fp, float2* __restrict__ out, size_t out_frame_stride, int n,
+                                  int cols, int rows) {
+    lerp_points_body<true>(p1, p1_frame_stride, nullptr, fp, seg, out, out_frame_stride, n, cols, rows);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -148,16 +165,19 @@ __device__ __forceinline__ bool tile_bbox(const TriRaster& r, int w, int h, int&
 }
 
 // grid (ceil(max_tri/128), frames). tile_counts (frames x n_tiles, zeroed by the caller) receives, per screen tile,
-// the number of triangles whose bounding box touches it.
-__global__ void k_tri_geometry(const int3* __restrict__ tri_idx, const FrameParams* __restrict__ fp,
-                               const float2* __restrict__ p1, size_t p1_frame_stride, const float2* __restrict__ p2,
-                               const float2* __restrict__ morphed, size_t morphed_frame_stride, int max_tri, int img_w,
-                               int img_h, TriInverse* __restrict__ inv_out, TriRaster* __restrict__ rast_out,
-                               int* __restrict__ tile_counts, int tiles_x, int n_tiles) {
+// the number of triangles whose bounding box touches it. SEG: frame f's pts2 is its segment's (seg[f]).
+template <bool SEG>
+__device__ __forceinline__ void tri_geometry_body(const int3* __restrict__ tri_idx, const FrameParams* __restrict__ fp,
+                                                  const float2* __restrict__ p1, size_t p1_frame_stride, const float2* __restrict__ p2,
+                                                  const SegFrame* __restrict__ seg, const float2* __restrict__ morphed,
+                                                  size_t morphed_frame_stride, int max_tri, int img_w, int img_h,
+                                                  TriInverse* __restrict__ inv_out, TriRaster* __restrict__ rast_out,
+                                                  int* __restrict__ tile_counts, int tiles_x, int n_tiles) {
     int t = blockIdx.x * blockDim.x + threadIdx.x;
     int f = blockIdx.y;
     FrameParams P = fp[f];
     if (t >= P.n_tri) return;
+    if (SEG) p2 = seg[f].pts2;
     int3 id = tri_idx[P.tri_base + t];
     const float2* s1 = p1 + (size_t)f * p1_frame_stride;
     const float2* mp = morphed + (size_t)f * morphed_frame_stride;
@@ -197,6 +217,24 @@ __global__ void k_tri_geometry(const int3* __restrict__ tri_idx, const FramePara
     inv3(M2, out.b);
     out.pad_a[0] = out.pad_a[1] = out.pad_a[2] = out.pad_b[0] = out.pad_b[1] = out.pad_b[2] = 0.f;
     inv_out[(size_t)f * max_tri + t] = out;
+}
+
+__global__ void k_tri_geometry(const int3* __restrict__ tri_idx, const FrameParams* __restrict__ fp,
+                               const float2* __restrict__ p1, size_t p1_frame_stride, const float2* __restrict__ p2,
+                               const float2* __restrict__ morphed, size_t morphed_frame_stride, int max_tri, int img_w,
+                               int img_h, TriInverse* __restrict__ inv_out, TriRaster* __restrict__ rast_out,
+                               int* __restrict__ tile_counts, int tiles_x, int n_tiles) {
+    tri_geometry_body<false>(tri_idx, fp, p1, p1_frame_stride, p2, nullptr, morphed, morphed_frame_stride, max_tri, img_w, img_h,
+                             inv_out, rast_out, tile_counts, tiles_x, n_tiles);
+}
+
+__global__ void k_tri_geometry_seg(const int3* __restrict__ tri_idx, const FrameParams* __restrict__ fp,
+                                   const float2* __restrict__ p1, size_t p1_frame_stride, const SegFrame* __restrict__ seg,
+                                   const float2* __restrict__ morphed, size_t morphed_frame_stride, int max_tri, int img_w,
+                                   int img_h, TriInverse* __restrict__ inv_out, TriRaster* __restrict__ rast_out,
+                                   int* __restrict__ tile_counts, int tiles_x, int n_tiles) {
+    tri_geometry_body<true>(tri_idx, fp, p1, p1_frame_stride, nullptr, seg, morphed, morphed_frame_stride, max_tri, img_w, img_h,
+                            inv_out, rast_out, tile_counts, tiles_x, n_tiles);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -288,6 +326,25 @@ void launch_tri_geometry(cudaStream_t st, const int3* tri_idx, const FrameParams
     if (tri_in_chunk_max > 0)
         k_tri_geometry<<<dim3(div_up(tri_in_chunk_max, 128), frames), 128, 0, st>>>(
             tri_idx, fp, p1, p1_frame_stride, p2, morphed, morphed_frame_stride, max_tri, img_w, img_h, inv_out, rast_out,
+            tile_counts, tiles_x, n_tiles);
+}
+
+void launch_lerp_points_seg(cudaStream_t st, const float2* p1, size_t p1_frame_stride, const SegFrame* seg,
+                            const FrameParams* fp, float2* out, size_t out_frame_stride, int n_max, int frames, int cols,
+                            int rows) {
+    if (n_max > 0)
+        k_lerp_points_seg<<<dim3(div_up(n_max, 256), frames), 256, 0, st>>>(p1, p1_frame_stride, seg, fp, out, out_frame_stride,
+                                                                            n_max, cols, rows);
+}
+
+void launch_tri_geometry_seg(cudaStream_t st, const int3* tri_idx, const FrameParams* fp, const float2* p1,
+                             size_t p1_frame_stride, const SegFrame* seg, const float2* morphed, size_t morphed_frame_stride,
+                             int max_tri, int tri_in_chunk_max, int frames, int img_w, int img_h, TriInverse* inv_out,
+                             TriRaster* rast_out, int* tile_counts) {
+    const int tiles_x = div_up(img_w, RW_TW), n_tiles = tiles_x * div_up(img_h, RW_TH);
+    if (tri_in_chunk_max > 0)
+        k_tri_geometry_seg<<<dim3(div_up(tri_in_chunk_max, 128), frames), 128, 0, st>>>(
+            tri_idx, fp, p1, p1_frame_stride, seg, morphed, morphed_frame_stride, max_tri, img_w, img_h, inv_out, rast_out,
             tile_counts, tiles_x, n_tiles);
 }
 

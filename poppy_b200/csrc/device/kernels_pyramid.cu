@@ -460,10 +460,12 @@ __device__ __forceinline__ void down0_bulk_mask(const Down0Feed<float>& F, int b
 // warped: per frame two planes of packed BGRX words (image 1, image 2), rows wpitch words apart, wstride words per
 // plane. mask0: per-frame level-0 mask planes (rows bpitch floats apart, m0stride floats per frame) written here for the
 // level-0 collapse. Interior tiles stage their source rows through a Down0Feed ring, border tiles run the generic bodies.
-__global__ void __launch_bounds__(96)
-k_pyr_down0_roll(const uint32_t* __restrict__ warped, int wpitch, size_t wstride, const float* __restrict__ basis, int bpitch,
-                 const FrameParams* __restrict__ fp, int sw, int sh, float* __restrict__ mask0, size_t m0stride,
-                 float* __restrict__ dst, int dw, int dh, int dpitch, size_t dstride) {
+// SEG: frame f's mask basis is its segment's, seg[f].basis (same pitch; every basis starts 128-byte aligned).
+template <bool SEG>
+__device__ __forceinline__ void
+pyr_down0_body(const uint32_t* __restrict__ warped, int wpitch, size_t wstride, const float* __restrict__ basis, int bpitch,
+               const SegFrame* __restrict__ seg, const FrameParams* __restrict__ fp, int sw, int sh, float* __restrict__ mask0,
+               size_t m0stride, float* __restrict__ dst, int dw, int dh, int dpitch, size_t dstride) {
     extern __shared__ __align__(128) unsigned char smem_down0[];
     // blockIdx.z = role * frames + f: CTAs that are resident together run the same role, i.e. the same hot loop, which
     // keeps the per-scheduler instruction cache from thrashing between the (large, fully unrolled) role bodies. The three
@@ -492,6 +494,7 @@ k_pyr_down0_roll(const uint32_t* __restrict__ warped, int wpitch, size_t wstride
     } else {
         const DownFlags fl = down_flags(sel, x, false, 0);
         const double alpha = fp[f].mask_alpha, beta = fp[f].mask_beta;
+        if (SEG) basis = seg[f].basis;
         float* __restrict__ m0 = mask0 + (size_t)f * m0stride;
         const bool interior = __all_sync(FULL, rows_in && down_lane_interior(x, sw, dw, fl)) &&
                               (2 * X0 - 4 >= 0 && 2 * X0 - 4 + D0_SEG <= bpitch);
@@ -503,6 +506,20 @@ k_pyr_down0_roll(const uint32_t* __restrict__ warped, int wpitch, size_t wstride
             down0_body_mask(basis, bpitch, alpha, beta, sw, sh, m0, dframe + 6 * dstride, dh, dpitch, x, y0, fl);
         }
     }
+}
+
+__global__ void __launch_bounds__(96)
+k_pyr_down0_roll(const uint32_t* __restrict__ warped, int wpitch, size_t wstride, const float* __restrict__ basis, int bpitch,
+                 const FrameParams* __restrict__ fp, int sw, int sh, float* __restrict__ mask0, size_t m0stride,
+                 float* __restrict__ dst, int dw, int dh, int dpitch, size_t dstride) {
+    pyr_down0_body<false>(warped, wpitch, wstride, basis, bpitch, nullptr, fp, sw, sh, mask0, m0stride, dst, dw, dh, dpitch, dstride);
+}
+
+__global__ void __launch_bounds__(96)
+k_pyr_down0_roll_seg(const uint32_t* __restrict__ warped, int wpitch, size_t wstride, const SegFrame* __restrict__ seg, int bpitch,
+                     const FrameParams* __restrict__ fp, int sw, int sh, float* __restrict__ mask0, size_t m0stride,
+                     float* __restrict__ dst, int dw, int dh, int dpitch, size_t dstride) {
+    pyr_down0_body<true>(warped, wpitch, wstride, nullptr, bpitch, seg, fp, sw, sh, mask0, m0stride, dst, dw, dh, dpitch, dstride);
 }
 
 // block 256; grid (ceil(w*h/256), frames)
@@ -1074,6 +1091,16 @@ void launch_pyr_down0(cudaStream_t st, const uint32_t* warped, int wpitch, size_
     ensure_smem_attr(k_pyr_down0_roll, D0_SMEM, done);
     k_pyr_down0_roll<<<grid, block, D0_SMEM, st>>>(warped, wpitch, wstride, basis, bpitch, fp, w, h, mask0, m0stride, dst, dl.w, dl.h,
                                                    dl.pitch, dl.plane_stride);
+}
+
+void launch_pyr_down0_seg(cudaStream_t st, const uint32_t* warped, int wpitch, size_t wstride, const SegFrame* seg, int bpitch,
+                          const FrameParams* fp, int w, int h, float* mask0, size_t m0stride, float* dst, LevelDesc dl,
+                          int frames) {
+    const dim3 grid(div_up(dl.w, 128), div_up(dl.h, 3 * DN_R), 3 * frames), block(32, 3);
+    static SmemAttrOnce done;
+    ensure_smem_attr(k_pyr_down0_roll_seg, D0_SMEM, done);
+    k_pyr_down0_roll_seg<<<grid, block, D0_SMEM, st>>>(warped, wpitch, wstride, seg, bpitch, fp, w, h, mask0, m0stride, dst, dl.w,
+                                                       dl.h, dl.pitch, dl.plane_stride);
 }
 
 void launch_pyr_down(cudaStream_t st, const float* src, LevelDesc sl, float* dst, LevelDesc dl, int frames) {

@@ -292,6 +292,28 @@ int poppy_shim_morph_sequence(int w, int h, int pyramid_levels, const uint8_t* c
     });
 }
 
+int poppy_shim_morph_segments(int w, int h, int pyramid_levels, const poppy_shim_segment* segs, int n_segments, int n_frames,
+                              poppy_write_fn write, void* user) {
+    if (!segs || !write || n_segments < 1) return host_fail(POPPY_CUDA_ERR_INVALID, "null argument");
+    for (int s = 0; s < n_segments; ++s)
+        if (!segs[s].corrected1 || !segs[s].corrected2 || segs[s].n < 0 || (segs[s].n > 0 && (!segs[s].pts1_xy || !segs[s].pts2_xy)))
+            return host_fail(POPPY_CUDA_ERR_INVALID, "segment " + std::to_string(s) + ": null argument");
+    return shim_guard([&] {
+        poppy::Settings::instance().pyramid_levels = (size_t)pyramid_levels;
+        std::vector<poppy::Segment> v(n_segments);
+        for (int s = 0; s < n_segments; ++s) {
+            const poppy_shim_segment& g = segs[s];
+            v[s].corrected1 = view8(g.corrected1, w, h, g.step1);
+            v[s].corrected2 = view8(g.corrected2, w, h, g.step2);
+            if (g.gabor2) { v[s].gabor2.data = g.gabor2; v[s].gabor2.cols = w; v[s].gabor2.rows = h; v[s].gabor2.step = g.gstep; }
+            v[s].srcPoints1 = to_points(g.pts1_xy, g.n);
+            v[s].srcPoints2 = to_points(g.pts2_xy, g.n);
+        }
+        int index = 0;
+        poppy::morph_segments(v, n_frames, [&](const poppy::Image8& f) { write(user, index++, f.data, f.cols, f.rows, f.step); });
+    });
+}
+
 void poppy_shim_release(void) { poppy::release_cached_contexts(); }
 
 }  // extern "C"

@@ -161,4 +161,86 @@ void morph_sequence(const Image8& corrected1, const Image8& corrected2, std::vec
     morph_sequence(corrected1, corrected2, Image32F(), std::move(srcPoints1), std::move(srcPoints2), number_of_frames, write);
 }
 
+void morph_segments(const std::vector<Segment>& segments, int number_of_frames, const std::function<void(const Image8&)>& write) {
+    const int K = (int)segments.size(), N = number_of_frames;
+    if (K == 0 || N < 1) return;
+    const int w = segments[0].corrected1.cols, h = segments[0].corrected1.rows;
+    for (const Segment& s : segments) {
+        if (s.corrected1.cols != w || s.corrected1.rows != h || s.corrected2.cols != w || s.corrected2.rows != h)
+            throw MorphError("morph_segments: all segments must have the same frame size");
+        if (s.srcPoints1.size() != s.srcPoints2.size()) throw MorphError("morph_segments: point sets differ in size");
+    }
+    std::vector<float> ratio(N);
+    std::vector<double> mask(N);
+    for (int j = 0; j < N; ++j) { mask[j] = poppy_host_chain_ratio(j, N); ratio[j] = (float)mask[j]; }
+    // every segment's chain is planned as morph_sequence plans it
+    struct Plans { std::vector<poppy_host_plan*> p; ~Plans() { for (auto* q : p) poppy_host_plan_destroy(q); } } plans;
+    std::vector<const int32_t*> tri(K), offs(K);
+    int n_max = 0, tri_max = 0;
+    static const float none[2] = {0.f, 0.f};
+    for (int s = 0; s < K; ++s) {
+        const int n = (int)segments[s].srcPoints1.size();
+        poppy_host_plan* plan = nullptr;
+        if (poppy_host_plan_create(&plan, n ? &segments[s].srcPoints1.data()->x : none, n ? &segments[s].srcPoints2.data()->x : none,
+                                   n, w, h, N, ratio.data(), 1, 0) != 0)
+            throw MorphError("morph_segments: segment " + std::to_string(s) + ": " + poppy_host_last_error());
+        plans.p.push_back(plan);
+        int mt = 0;
+        poppy_host_plan_triangles(plan, &tri[s], &offs[s], &mt);
+        n_max = std::max(n_max, n);
+        tri_max = std::max(tri_max, mt);
+    }
+
+    std::lock_guard<std::mutex> lock(g_mu);
+    // as many segments per batch as fit the ring at once (all N frames of each stay resident until written)
+    const size_t frame_bytes = (size_t)w * h * 3, ring_bytes = 8ull << 30;
+    const int per_batch = (int)std::max<size_t>(1, std::min<size_t>(K, ring_bytes / (frame_bytes * N)));
+    poppy_cuda_ctx* c = context_for(w, h, (int)Settings::instance().pyramid_levels, n_max, tri_max, per_batch * N);
+    // a kernel batch holds one step of a group of segments; the cached context goes back to one frame per batch after
+    cu(c, poppy_cuda_set_chunk_frames(c, std::min(per_batch, 32)));
+    struct ChunkGuard { poppy_cuda_ctx* c; ~ChunkGuard() { poppy_cuda_set_chunk_frames(c, 1); } } cguard{c};
+    struct Sink { const std::function<void(const Image8&)>* write; } sink{&write};
+    auto deliver = [](void* u, int, uint8_t* bgr, int fw, int fh, size_t step) {
+        Image8 f;
+        f.data = bgr; f.cols = fw; f.rows = fh; f.step = step;
+        (*static_cast<Sink*>(u)->write)(f);
+    };
+    poppy_host_writer* wr = nullptr;
+    if (poppy_host_writer_create(&wr, c, std::min(N, 8), deliver, nullptr, 0, &sink) != 0)
+        throw MorphError("morph_segments: cannot create the writer ring");
+    struct WriterGuard { poppy_host_writer* w; ~WriterGuard() { poppy_host_writer_destroy_cuda(w); } } wguard{wr};
+    const int S = 4;                                  // steps per render call
+    std::vector<int32_t> st, so;
+    for (int b0 = 0; b0 < K; b0 += per_batch) {
+        const int kb = std::min(per_batch, K - b0);
+        cu(c, poppy_cuda_set_segments(c, kb, N));
+        for (int i = 0; i < kb; ++i) {
+            const Segment& g = segments[b0 + i];
+            const int n = (int)g.srcPoints1.size();
+            cu(c, poppy_cuda_set_segment(c, i, g.corrected1.data, g.corrected1.step, g.corrected2.data, g.corrected2.step, g.gabor2.data,
+                                         g.gabor2.step, n ? &g.srcPoints1.data()->x : none, n ? &g.srcPoints2.data()->x : none, n));
+        }
+        for (int a = 0; a < N; a += S) {
+            const int cnt = std::min(S, N - a);
+            // the slice's lists, step-major: entry r * kb + i is step a + r of segment b0 + i
+            st.clear();
+            so.assign(1, 0);
+            for (int r = 0; r < cnt; ++r)
+                for (int i = 0; i < kb; ++i) {
+                    const int32_t* o = offs[b0 + i];
+                    st.insert(st.end(), tri[b0 + i] + (size_t)o[a + r] * 3, tri[b0 + i] + (size_t)o[a + r + 1] * 3);
+                    so.push_back((int32_t)(st.size() / 3));
+                }
+            cu(c, poppy_cuda_render_segments(c, a, cnt, ratio.data() + a, mask.data() + a, st.data(), so.data()));
+            // the batch's first segment is written as it renders (its step j is ring slot j)
+            if (poppy_host_writer_submit(wr, a, cnt, b0 * N + a) != 0) throw MorphError(std::string("morph_segments: ") + poppy_cuda_last_error(c));
+        }
+        for (int i = 1; i < kb; ++i)
+            if (poppy_host_writer_submit(wr, i * N, N, (b0 + i) * N) != 0)
+                throw MorphError(std::string("morph_segments: ") + poppy_cuda_last_error(c));
+        // the next batch's segment data and frames replace this batch's: wait until every frame of it is written
+        if (poppy_host_writer_flush(wr) != 0) throw MorphError("morph_segments: a frame download failed");
+    }
+}
+
 }  // namespace poppy

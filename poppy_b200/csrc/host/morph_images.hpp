@@ -89,6 +89,17 @@ void morph_sequence(const Image8& corrected1, const Image8& corrected2, const Im
 void morph_sequence(const Image8& corrected1, const Image8& corrected2, std::vector<Point2f> srcPoints1,
                     std::vector<Point2f> srcPoints2, int number_of_frames, const std::function<void(const Image8&)>& write);
 
+// One segment of a multi-image sequence: the arguments of morph_sequence for one consecutive pair.
+struct Segment {
+    Image8 corrected1, corrected2;
+    Image32F gabor2;                   // empty: derived on the device
+    std::vector<Point2f> srcPoints1, srcPoints2;
+};
+// The segments of run() (reference src/poppy.cpp:266-328), each the chain morph_sequence renders, rendered together on the
+// GPU (step j of a group of segments per kernel batch). Frames go to `write` in the reference's order: all
+// number_of_frames frames of segment 0, then segment 1, ...; segment 0's are written while later steps still render.
+void morph_segments(const std::vector<Segment>& segments, int number_of_frames, const std::function<void(const Image8&)>& write);
+
 // Releases the cached device context(s) held by morph_images()/morph_sequence().
 void release_cached_contexts();
 

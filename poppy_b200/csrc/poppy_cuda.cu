@@ -8,6 +8,9 @@
 //   chunk scratch (xB): FrameParams; triangle indices; TriInverse / TriRaster records; triangle-ID map int32 [H][W];
 //                       warped pair 2 x uint32 BGRX [H][pitch0]; Gaussian levels 1..L (7 planes); collapsed levels 0..L
 //                       (3 planes); level-0 blend mask float [H][pitch0]
+//   segments (optional, poppy_cuda_set_segments): per segment the pair's resident data - corrected1, corrected2 and chain
+//                       arrays, a mask basis (one allocation, padded_pixels() floats each), raw and clipped point sets;
+//                       per lane a SegFrame table and a BGRX staging plane per frame of a chunk
 #include <cuda.h>
 #include <cuda_runtime.h>
 
@@ -113,6 +116,11 @@ struct poppy_cuda_ctx {
         std::vector<CollapseMaps> maps;      // tensor maps of level k's collapse (index k)
         FrameParams* h_fp = nullptr;         // pinned staging
         int32_t* h_tri = nullptr;
+        // segment renders: the chunk's per-frame sources (d_seg, pinned staging h_seg) and the BGRX staging of its frames
+        // for the chain arrays, seg_cap frames each
+        SegFrame *d_seg = nullptr, *h_seg = nullptr;
+        uchar4* d_seg_stage = nullptr;
+        int seg_cap = 0;
     } lane[kRenderLanes];
     int n_lanes = 0;                         // lanes allocated (0 = none yet)
     int n_tiles = 0, list_cap = 0;
@@ -137,6 +145,20 @@ struct poppy_cuda_ctx {
     unsigned long long* d_calm_total = nullptr;      // flagged strip chunks since the last stats read
     unsigned long long* d_probe_total = nullptr;     // sink of the statistic-only scans
     uint64_t calm_chunks_total = 0, dense_chunks_total = 0;
+
+    // Segments of a multi-image sequence (poppy_cuda_set_segments): independent chains of the same frame size, rendered
+    // together. Step j of segment s lands in ring slot s * seg_window + j % seg_window.
+    struct Segment {
+        cudaArray_t a[3] = {nullptr, nullptr, nullptr};      // corrected1, corrected2, chain source (the previous step's frame)
+        cudaTextureObject_t t[3] = {0, 0, 0};
+        int n = 0;                                           // points
+        bool set = false;
+    };
+    std::vector<Segment> seg;
+    int seg_window = 0;
+    int seg_next_step = -1;                  // step at which a segment render may continue (-1: none in progress)
+    float* d_seg_basis = nullptr;            // n_seg x padded_pixels()
+    float2 *d_seg_raw = nullptr, *d_seg_pts1 = nullptr, *d_seg_pts2 = nullptr;   // raw: 2 x max_points, clipped: max_points per segment
 
     std::vector<TimedLaunch> timed;
     std::vector<cudaEvent_t> event_pool;
@@ -177,12 +199,67 @@ void free_chunk(poppy_cuda_ctx* c) {
         cudaFree(l.d_warped); cudaFree(l.d_mask0); cudaFree(l.d_g); cudaFree(l.d_o);
         cudaFree(l.d_excess); cudaFree(l.d_block_dev); cudaFree(l.d_block_flags); cudaFree(l.d_chunk_flags); cudaFree(l.d_tile_flags); cudaFree(l.d_calm_counts);
         cudaFreeHost(l.h_fp); cudaFreeHost(l.h_tri); cudaFreeHost(l.h_calm_counts);
+        cudaFree(l.d_seg); cudaFreeHost(l.h_seg); cudaFree(l.d_seg_stage);
         cudaStream_t st = l.stream; cudaEvent_t e1 = l.ev_staged, e2 = l.ev_done, e3 = l.ev_calm;
         l = poppy_cuda_ctx::Lane();
         l.stream = st; l.ev_staged = e1; l.ev_done = e2; l.ev_calm = e3;
     }
     c->chunk = 0;
     c->n_lanes = 0;
+}
+
+void free_segments(poppy_cuda_ctx* c) {
+    for (auto& S : c->seg)
+        for (int i = 0; i < 3; ++i) {
+            if (S.t[i]) cudaDestroyTextureObject(S.t[i]);
+            if (S.a[i]) cudaFreeArray(S.a[i]);
+        }
+    c->seg.clear();
+    cudaFree(c->d_seg_basis); cudaFree(c->d_seg_raw); cudaFree(c->d_seg_pts1); cudaFree(c->d_seg_pts2);
+    c->d_seg_basis = nullptr; c->d_seg_raw = c->d_seg_pts1 = c->d_seg_pts2 = nullptr;
+    c->seg_window = 0;
+    c->seg_next_step = -1;
+}
+
+// uchar4 array with a point-sampled, border-addressed (zero) texture over it, as the pair's sources
+cudaError_t make_source_array(int w, int h, cudaArray_t* a, cudaTextureObject_t* t) {
+    const cudaChannelFormatDesc fmt = cudaCreateChannelDesc<uchar4>();
+    cudaError_t e = cudaMallocArray(a, &fmt, (size_t)w, (size_t)h, cudaArrayTextureGather);
+    if (e != cudaSuccess) return e;
+    cudaResourceDesc res{};
+    res.resType = cudaResourceTypeArray;
+    res.res.array.array = *a;
+    cudaTextureDesc td{};
+    td.addressMode[0] = td.addressMode[1] = cudaAddressModeBorder;      // BORDER_CONSTANT(0)
+    td.filterMode = cudaFilterModePoint;
+    td.readMode = cudaReadModeElementType;
+    td.normalizedCoords = 0;
+    return cudaCreateTextureObject(t, &res, &td, nullptr);
+}
+
+// 8-bit BGR host image -> BGRX array, through the pair's upload staging on the context's stream
+int upload_source(poppy_cuda_ctx* c, const uint8_t* data, size_t step, cudaArray_t dst) {
+    const size_t row = (size_t)c->w * 3, trow = (size_t)c->w * 4;
+    CU_TRY(c, cudaMemcpy2DAsync(c->d_stage_u8, row, data, step, row, c->h, cudaMemcpyHostToDevice, c->stream));
+    launch_bgr_to_bgrx(c->stream, c->d_stage_u8, c->d_src_stage, c->w, c->h);
+    c->launches++; c->class_launches[KC_MISC]++;
+    CU_TRY(c, cudaMemcpy2DToArrayAsync(dst, 0, 0, c->d_src_stage, trow, trow, c->h, cudaMemcpyDeviceToDevice, c->stream));
+    return 0;
+}
+
+// per-lane segment tables and chain staging for groups of up to `frames` segments
+int ensure_seg_lanes(poppy_cuda_ctx* c, int frames) {
+    for (int i = 0; i < c->n_lanes; ++i) {
+        auto& l = c->lane[i];
+        if (l.seg_cap >= frames) continue;
+        cudaFree(l.d_seg); cudaFreeHost(l.h_seg); cudaFree(l.d_seg_stage);
+        l.d_seg = nullptr; l.h_seg = nullptr; l.d_seg_stage = nullptr; l.seg_cap = 0;
+        CU_TRY(c, dmalloc(&l.d_seg, (size_t)frames));
+        CU_TRY(c, cudaMallocHost((void**)&l.h_seg, (size_t)frames * sizeof(SegFrame)));
+        CU_TRY(c, dmalloc(&l.d_seg_stage, (size_t)frames * c->pixels()));
+        l.seg_cap = frames;
+    }
+    return 0;
 }
 
 // ---- TMA tensor maps (cuTensorMapEncodeTiled through the runtime's driver entry point: no libcuda link dependency) ----
@@ -363,34 +440,52 @@ void harvest_calm_stats(poppy_cuda_ctx* c, bool wait) {
     }
 }
 
+// One step of a group of segments (poppy_cuda_render_segments): frame i of the chunk is step `step` of segment s0 + i, its
+// shape / mask ratio is entry `row` of the call's arrays and its triangle list entry row * n_seg + s0 + i.
+struct SegChunk { int s0, step, row; };
+
 // tri_idx == nullptr: the triangles come from the resident plan, tri_off pointing into its offsets (frame `first` of this call
 // is plan frame plan_first + first)
 int render_chunk(poppy_cuda_ctx* c, int slot0, int first, int nb, const float* shape, const double* mask, const int32_t* tri_idx,
-                 const int32_t* tri_off, bool chain, poppy_cuda_ctx::Lane& ln) {
+                 const int32_t* tri_off, bool chain, poppy_cuda_ctx::Lane& ln, const SegChunk* sg = nullptr) {
     cudaStream_t st = ln.stream;
     CU_TRY(c, cudaEventSynchronize(ln.ev_staged));       // the lane's staging buffers are free again
     FrameParams* hp = ln.h_fp;
     int32_t* ht = ln.h_tri;
-    int tri_total = 0, tri_max = 0;
+    int tri_total = 0, tri_max = 0, seg_n_max = 0;
+    const int K = (int)c->seg.size(), W = c->seg_window;
     for (int i = 0; i < nb; ++i) {
-        const int f = first + i;
+        const int f = sg ? sg->row * K + sg->s0 + i : first + i;       // triangle list entry
+        const int r = sg ? sg->row : f;                                 // ratio entry
         const int nt = tri_off[f + 1] - tri_off[f];
         if (nt < 0 || nt > c->max_tri) return fail(c, POPPY_CUDA_ERR_CAPACITY, "frame %d has %d triangles (max %d)", f, nt, c->max_tri);
         if (tri_idx && nt)         // validated by poppy_cuda_render_range
             std::memcpy(ht + (size_t)tri_total * 3, tri_idx + (size_t)tri_off[f] * 3, (size_t)nt * 3 * sizeof(int32_t));
         FrameParams& p = hp[i];
-        p.shape = shape[f];
+        p.shape = shape[r];
         p.one_minus_r = (float)(1.0 - (double)p.shape);
-        p.mask_alpha = 1.0 - mask[f];
-        p.mask_beta = -mask[f];
-        p.amount = (float)(1.0 - std::sin(mask[f] * M_PI));
+        p.mask_alpha = 1.0 - mask[r];
+        p.mask_beta = -mask[r];
+        p.amount = (float)(1.0 - std::sin(mask[r] * M_PI));
         p.n_tri = nt;
         p.tri_base = tri_total;
-        p.dst_slot = slot0 + f;
+        p.dst_slot = sg ? (sg->s0 + i) * W + sg->step % W : slot0 + f;
         tri_total += nt;
         tri_max = std::max(tri_max, nt);
+        if (sg) {
+            const poppy_cuda_ctx::Segment& S = c->seg[sg->s0 + i];
+            SegFrame& q = ln.h_seg[i];
+            q.src1 = sg->step == 0 ? S.t[0] : S.t[2];
+            q.src2 = S.t[1];
+            q.basis = c->d_seg_basis + (size_t)(sg->s0 + i) * c->padded_pixels();
+            q.pts2 = c->d_seg_pts2 + (size_t)(sg->s0 + i) * c->max_points;
+            q.n_points = S.n;
+            q.pad = 0;
+            seg_n_max = std::max(seg_n_max, S.n);
+        }
     }
     CU_TRY(c, cudaMemcpyAsync(ln.d_fp, hp, nb * sizeof(FrameParams), cudaMemcpyHostToDevice, st));
+    if (sg) CU_TRY(c, cudaMemcpyAsync(ln.d_seg, ln.h_seg, nb * sizeof(SegFrame), cudaMemcpyHostToDevice, st));
     if (tri_idx && tri_total)
         CU_TRY(c, cudaMemcpyAsync(ln.d_tri, ht, (size_t)tri_total * 3 * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     CU_TRY(c, cudaEventRecord(ln.ev_staged, st));
@@ -405,13 +500,27 @@ int render_chunk(poppy_cuda_ctx* c, int slot0, int first, int nb, const float* s
     float2* morphed = c->d_morphed + (size_t)(slot0 + first) * c->max_points;
     const int n = c->n_points, w = c->w, h = c->h, L = c->levels;
 
+    // segments: the chunk's frames are consecutive segments, so their previous steps' points and their outputs lie a
+    // constant W * max_points apart in the ring, their step-0 points max_points apart
+    const size_t ring_stride = (size_t)W * c->max_points;
+    const float2* sp1 = !sg ? nullptr
+                      : sg->step == 0 ? c->d_seg_pts1 + (size_t)sg->s0 * c->max_points
+                                      : c->d_morphed + ((size_t)sg->s0 * W + (sg->step - 1) % W) * c->max_points;
+    const size_t sp1_stride = sg && sg->step == 0 ? (size_t)c->max_points : ring_stride;
+    float2* smorphed = sg ? c->d_morphed + ((size_t)sg->s0 * W + sg->step % W) * c->max_points : nullptr;
+
     {   Scope s(c, KC_POINTS, st);
-        launch_lerp_points(st, p1, 0, c->d_pts2, ln.d_fp, morphed, c->max_points, n, nb, w, h);
+        if (sg) launch_lerp_points_seg(st, sp1, sp1_stride, ln.d_seg, ln.d_fp, smorphed, ring_stride, seg_n_max, nb, w, h);
+        else launch_lerp_points(st, p1, 0, c->d_pts2, ln.d_fp, morphed, c->max_points, n, nb, w, h);
     }
     CU_TRY(c, cudaMemsetAsync(ln.d_tile_cnt, 0, (size_t)nb * c->n_tiles * sizeof(int), st));
     {   Scope s(c, KC_GEOMETRY, st);
-        launch_tri_geometry(st, chunk_tri, ln.d_fp, p1, 0, c->d_pts2, morphed, c->max_points, c->max_tri, tri_max, nb, w, h,
-                            ln.d_inv, ln.d_rast, ln.d_tile_cnt);
+        if (sg)
+            launch_tri_geometry_seg(st, chunk_tri, ln.d_fp, sp1, sp1_stride, ln.d_seg, smorphed, ring_stride, c->max_tri, tri_max, nb,
+                                    w, h, ln.d_inv, ln.d_rast, ln.d_tile_cnt);
+        else
+            launch_tri_geometry(st, chunk_tri, ln.d_fp, p1, 0, c->d_pts2, morphed, c->max_points, c->max_tri, tri_max, nb, w, h,
+                                ln.d_inv, ln.d_rast, ln.d_tile_cnt);
     }
     {   Scope s(c, KC_BIN, st);
         c->launches++;          // scan + fill
@@ -419,14 +528,21 @@ int render_chunk(poppy_cuda_ctx* c, int slot0, int first, int nb, const float* s
                              ln.d_overflow, ln.d_tile_list, c->list_cap);
     }
     {   Scope s(c, KC_WARP, st);
-        launch_raster_warp(st, ln.d_rast, ln.d_inv, ln.d_fp, c->max_tri, ln.d_tile_off, ln.d_tile_list, c->list_cap,
-                           ln.d_overflow, src1, c->t_src[1], ln.d_warped, c->pitch0(), c->padded_pixels(),
-                           c->keep_stages ? ln.d_trimap : nullptr,
-                           w, h, nb);
+        if (sg)
+            launch_raster_warp_seg(st, ln.d_rast, ln.d_inv, ln.d_fp, c->max_tri, ln.d_tile_off, ln.d_tile_list, c->list_cap,
+                                   ln.d_overflow, ln.d_seg, ln.d_warped, c->pitch0(), c->padded_pixels(), w, h, nb);
+        else
+            launch_raster_warp(st, ln.d_rast, ln.d_inv, ln.d_fp, c->max_tri, ln.d_tile_off, ln.d_tile_list, c->list_cap,
+                               ln.d_overflow, src1, c->t_src[1], ln.d_warped, c->pitch0(), c->padded_pixels(),
+                               c->keep_stages ? ln.d_trimap : nullptr, w, h, nb);
     }
     {   Scope s(c, KC_PYR_DOWN, st);
-        launch_pyr_down0(st, ln.d_warped, c->pitch0(), c->padded_pixels(), c->d_mbasis, c->pitch0(), ln.d_fp, w, h, ln.d_mask0,
-                         c->padded_pixels(), g_level(c, ln, 1), c->lv[1], nb);
+        if (sg)
+            launch_pyr_down0_seg(st, ln.d_warped, c->pitch0(), c->padded_pixels(), ln.d_seg, c->pitch0(), ln.d_fp, w, h, ln.d_mask0,
+                                 c->padded_pixels(), g_level(c, ln, 1), c->lv[1], nb);
+        else
+            launch_pyr_down0(st, ln.d_warped, c->pitch0(), c->padded_pixels(), c->d_mbasis, c->pitch0(), ln.d_fp, w, h, ln.d_mask0,
+                             c->padded_pixels(), g_level(c, ln, 1), c->lv[1], nb);
     }
     const int k0 = c->tail_k0;                  // levels k0 .. L: one launch
     for (int k = 1; k < (k0 ? k0 : L); ++k) {
@@ -500,7 +616,14 @@ int render_chunk(poppy_cuda_ctx* c, int slot0, int first, int nb, const float* s
             ln.calm_pending = nb;
         }
     }
-    if (chain) {
+    if (sg) {
+        // every segment's chain source becomes this step's frame: one conversion for the chunk, one array copy per segment
+        Scope s(c, KC_MISC, st);
+        launch_bgr_to_bgrx_frames(st, c->d_frames, c->frame_bytes(), ln.d_fp, ln.d_seg_stage, w, h, nb);
+        for (int i = 0; i < nb; ++i)
+            CU_TRY(c, cudaMemcpy2DToArrayAsync(c->seg[sg->s0 + i].a[2], 0, 0, ln.d_seg_stage + (size_t)i * c->pixels(), (size_t)w * 4,
+                                               (size_t)w * 4, h, cudaMemcpyDeviceToDevice, st));
+    } else if (chain) {
         Scope s(c, KC_MISC, st);
         launch_bgr_to_bgrx(st, c->d_frames + (size_t)(slot0 + first + nb - 1) * c->frame_bytes(), c->d_src_stage, w, h);
         CU_TRY(c, cudaMemcpy2DToArrayAsync(c->a_src[2], 0, 0, c->d_src_stage, (size_t)w * 4, (size_t)w * 4, h,
@@ -624,6 +747,7 @@ void poppy_cuda_destroy(poppy_cuda_ctx* c) {
     for (cudaEvent_t e : c->event_pool) cudaEventDestroy(e);
     for (cudaEvent_t e : c->tickets) if (e) cudaEventDestroy(e);
     free_chunk(c);
+    free_segments(c);
     cudaFree(c->d_src_stage); cudaFree(c->d_mbasis); cudaFree(c->d_stage_u8); cudaFree(c->d_stage_f32);
     for (int i = 0; i < 3; ++i) {
         if (c->t_src[i]) cudaDestroyTextureObject(c->t_src[i]);
@@ -912,9 +1036,159 @@ int render_impl(poppy_cuda_ctx* c, int first_slot, int n_frames, const float* sh
     CU_TRY(c, cudaEventRecord(c->ev_end, c->stream));
     c->last_frames = first_slot + n_frames;
     c->chain_next_slot = chain ? first_slot + n_frames : -1;
+    c->seg_next_step = -1;          // the ring slots and points a segment render would continue from may be overwritten
     return 0;
 }
+
 }  // namespace
+
+int poppy_cuda_set_segments(poppy_cuda_ctx* c, int n_segments, int window) {
+    if (!c) return POPPY_CUDA_ERR_INVALID;
+    if (n_segments < 1) return fail(c, POPPY_CUDA_ERR_INVALID, "n_segments must be >= 1");
+    if (window < 2) return fail(c, POPPY_CUDA_ERR_INVALID, "window %d < 2: step j-1's points must survive step j", window);
+    if ((long long)n_segments * window > c->max_frames)
+        return fail(c, POPPY_CUDA_ERR_CAPACITY, "%d segments x %d slots exceed the ring (max %d)", n_segments, window, c->max_frames);
+    CU_TRY(c, cudaSetDevice(c->device));
+    // nothing queued may still read the segments being replaced
+    CU_TRY(c, cudaStreamSynchronize(c->stream));
+    for (auto& l : c->lane) if (l.stream) CU_TRY(c, cudaStreamSynchronize(l.stream));
+    free_segments(c);
+    c->seg.resize(n_segments);
+    for (auto& S : c->seg)
+        for (int i = 0; i < 3; ++i)
+            if (cudaError_t e = make_source_array(c->w, c->h, &S.a[i], &S.t[i])) {
+                free_segments(c);
+                return fail(c, POPPY_CUDA_ERR_CUDA, "segment source array: %s", cudaGetErrorString(e));
+            }
+    const size_t K = (size_t)n_segments, P = (size_t)c->max_points;
+    if (dmalloc(&c->d_seg_basis, K * c->padded_pixels()) != cudaSuccess || dmalloc(&c->d_seg_raw, 2 * K * P) != cudaSuccess ||
+        dmalloc(&c->d_seg_pts1, K * P) != cudaSuccess || dmalloc(&c->d_seg_pts2, K * P) != cudaSuccess) {
+        free_segments(c);
+        return fail(c, POPPY_CUDA_ERR_CUDA, "cannot allocate the resident data of %d segments", n_segments);
+    }
+    c->seg_window = window;
+    return 0;
+}
+
+int poppy_cuda_set_segment(poppy_cuda_ctx* c, int s, const uint8_t* bgr1, size_t step1, const uint8_t* bgr2, size_t step2,
+                           const float* gabor, size_t gstep, const float* pts1, const float* pts2, int n) {
+    if (!c) return POPPY_CUDA_ERR_INVALID;
+    if (s < 0 || s >= (int)c->seg.size()) return fail(c, POPPY_CUDA_ERR_INVALID, "segment %d not in [0,%d)", s, (int)c->seg.size());
+    if (!bgr1 || !bgr2) return fail(c, POPPY_CUDA_ERR_INVALID, "null image pointer");
+    const size_t row = (size_t)c->w * 3;
+    if (step1 < row || step2 < row || (gabor && gstep < row * sizeof(float)))
+        return fail(c, POPPY_CUDA_ERR_INVALID, "row stride smaller than a row");
+    if ((n > 0 && (!pts1 || !pts2)) || n < 0) return fail(c, POPPY_CUDA_ERR_INVALID, "bad point sets");
+    if (n > c->max_points) return fail(c, POPPY_CUDA_ERR_CAPACITY, "%d points (max %d)", n, c->max_points);
+    CU_TRY(c, cudaSetDevice(c->device));
+    if (int rc = ensure_pair_staging(c, 0)) return rc;
+    if (gabor) if (int rc = ensure_pair_staging(c, 2)) return rc;
+    poppy_cuda_ctx::Segment& S = c->seg[s];
+    S.set = false;
+    c->seg_next_step = -1;          // a chain cannot continue across a change of its inputs
+    float* basis = c->d_seg_basis + (size_t)s * c->padded_pixels();
+    if (int rc = upload_source(c, bgr1, step1, S.a[0])) return rc;
+    if (int rc = upload_source(c, bgr2, step2, S.a[1])) return rc;
+    if (!gabor) {
+        // corrected2 is still in the 8-bit staging (same stream): the mask basis from it, as poppy_cuda_set_image(3)
+        Scope sc(c, KC_MISC, c->stream);
+        CU_TRY(c, launch_gabor_mask_basis(c->stream, c->d_stage_u8, basis, c->pitch0(), c->w, c->h));
+    } else {
+        CU_TRY(c, cudaMemcpy2DAsync(c->d_stage_f32, row * sizeof(float), gabor, gstep, row * sizeof(float), c->h,
+                                    cudaMemcpyHostToDevice, c->stream));
+        Scope sc(c, KC_MISC, c->stream);
+        launch_mask_basis(c->stream, c->d_stage_f32, basis, c->pitch0(), c->w, c->h);
+    }
+    const size_t P = (size_t)c->max_points;
+    float2* raw = c->d_seg_raw + 2 * (size_t)s * P;
+    if (n > 0) {
+        CU_TRY(c, cudaMemcpyAsync(raw, pts1, (size_t)n * 8, cudaMemcpyHostToDevice, c->stream));
+        CU_TRY(c, cudaMemcpyAsync(raw + P, pts2, (size_t)n * 8, cudaMemcpyHostToDevice, c->stream));
+    }
+    launch_clip_points(c->stream, raw, c->d_seg_pts1 + (size_t)s * P, n, c->w, c->h);
+    launch_clip_points(c->stream, raw + P, c->d_seg_pts2 + (size_t)s * P, n, c->w, c->h);
+    c->launches += 2; c->class_launches[KC_MISC] += 2;
+    CU_TRY(c, cudaGetLastError());
+    CU_TRY(c, cudaStreamSynchronize(c->stream));   // the host arrays may be pageable and reused by the caller
+    S.n = n;
+    S.set = true;
+    return 0;
+}
+
+int poppy_cuda_render_segments(poppy_cuda_ctx* c, int first_step, int n_steps, const float* shape, const double* mask,
+                               const int32_t* tri_idx, const int32_t* tri_off) {
+    if (!c) return POPPY_CUDA_ERR_INVALID;
+    const int K = (int)c->seg.size(), W = c->seg_window;
+    if (K == 0) return fail(c, POPPY_CUDA_ERR_STATE, "poppy_cuda_set_segments must precede render_segments");
+    for (int s = 0; s < K; ++s)
+        if (!c->seg[s].set) return fail(c, POPPY_CUDA_ERR_STATE, "segment %d has not been set (poppy_cuda_set_segment)", s);
+    if (c->keep_stages) return fail(c, POPPY_CUDA_ERR_STATE, "segment renders keep no stage buffers (set_keep_stages(0))");
+    if (first_step < 0 || n_steps < 1) return fail(c, POPPY_CUDA_ERR_INVALID, "bad step range [%d, %d)", first_step, first_step + n_steps);
+    if (first_step > 0 && first_step != c->seg_next_step)
+        return fail(c, POPPY_CUDA_ERR_STATE, "a segment render continues at the step after its last rendered one (%d), not at %d",
+                    c->seg_next_step, first_step);
+    if (!shape || !mask || !tri_off) return fail(c, POPPY_CUDA_ERR_INVALID, "null argument");
+    const int entries = n_steps * K;
+    if (!tri_idx && tri_off[entries] != tri_off[0]) return fail(c, POPPY_CUDA_ERR_INVALID, "null triangle list");
+    // validate every list against its own segment's points before anything is enqueued
+    for (int e = 0; e < entries; ++e) {
+        const int s = e % K, nt = tri_off[e + 1] - tri_off[e];
+        if (nt < 0 || nt > c->max_tri)
+            return fail(c, POPPY_CUDA_ERR_CAPACITY, "step %d of segment %d has %d triangles (max %d)", first_step + e / K, s, nt, c->max_tri);
+        const int32_t* src = tri_idx ? tri_idx + (size_t)tri_off[e] * 3 : nullptr;
+        for (int j = 0; j < nt * 3; ++j)
+            if ((unsigned)src[j] >= (unsigned)c->seg[s].n)
+                return fail(c, POPPY_CUDA_ERR_INVALID, "step %d of segment %d: vertex index %d out of range [0,%d)", first_step + e / K, s,
+                            src[j], c->seg[s].n);
+    }
+    static const int32_t none[3] = {0, 0, 0};
+    if (!tri_idx) tri_idx = none;
+    CU_TRY(c, cudaSetDevice(c->device));
+    if (int rc = ensure_chunk(c)) return rc;
+    const int G = std::min(c->chunk, K);            // segments per group
+    if (int rc = ensure_seg_lanes(c, G)) return rc;
+    if (c->copy_hi > c->copy_lo && c->copy_lo < K * W)       // slots with a download in flight
+        CU_TRY(c, cudaStreamWaitEvent(c->stream, c->ev_copied, 0));
+    collect_timing(c);
+    std::fill(c->class_ms, c->class_ms + KC_COUNT, 0.f);
+    std::fill(c->class_launches, c->class_launches + KC_COUNT, 0ull);
+    CU_TRY(c, cudaEventRecord(c->ev_begin, c->stream));
+    // every step of a group runs on one lane (its chain is a recurrence); the groups go round-robin over the lanes
+    const int lanes = c->stage_timing ? 1 : c->n_lanes;
+    for (int i = 0; i < lanes; ++i) CU_TRY(c, cudaStreamWaitEvent(c->lane[i].stream, c->ev_begin, 0));
+    int rc = 0;
+    c->seg_next_step = -1;
+    for (int r = 0; r < n_steps && !rc; ++r)
+        for (int g = 0; g * G < K && !rc; ++g) {
+            const SegChunk sg{g * G, first_step + r, r};
+            rc = render_chunk(c, 0, 0, std::min(G, K - g * G), shape, mask, tri_idx, tri_off, true, c->lane[g % lanes], &sg);
+        }
+    for (int i = 0; i < lanes; ++i) {
+        cudaEventRecord(c->lane[i].ev_done, c->lane[i].stream);
+        cudaStreamWaitEvent(c->stream, c->lane[i].ev_done, 0);
+    }
+    cudaEventRecord(c->ev_end, c->stream);
+    if (rc) return rc;
+    CU_TRY(c, cudaGetLastError());
+    c->chain_next_slot = -1;        // the pair's chain slots are overwritten
+    c->last_frames = 0;
+    c->seg_next_step = first_step + n_steps;
+    return 0;
+}
+
+int poppy_cuda_get_segment_points(poppy_cuda_ctx* c, int s, int step, float* xy) {
+    if (!c) return POPPY_CUDA_ERR_INVALID;
+    if (!xy || s < 0 || s >= (int)c->seg.size()) return fail(c, POPPY_CUDA_ERR_INVALID, "bad segment %d or null pointer", s);
+    const int W = c->seg_window;
+    if (c->seg_next_step < 0 || step >= c->seg_next_step || step < std::max(0, c->seg_next_step - W))
+        return fail(c, POPPY_CUDA_ERR_INVALID, "step %d of segment %d is not in the ring", step, s);
+    CU_TRY(c, cudaSetDevice(c->device));
+    if (c->seg[s].n > 0)
+        CU_TRY(c, cudaMemcpyAsync(xy, c->d_morphed + ((size_t)s * W + step % W) * c->max_points, (size_t)c->seg[s].n * 8,
+                                  cudaMemcpyDeviceToHost, c->stream));
+    CU_TRY(c, cudaStreamSynchronize(c->stream));
+    return 0;
+}
 
 int poppy_cuda_download(poppy_cuda_ctx* c, int first, int count, uint8_t* dst, size_t step, size_t frame_stride) {
     if (!c) return POPPY_CUDA_ERR_INVALID;

@@ -36,6 +36,7 @@ class MorphRenderer:
         self.width, self.height, self.levels = width, height, pyramid_levels
         self.max_points, self.max_triangles, self.max_batch_frames = max_points, max_triangles, max_batch_frames
         self.n_points = 0
+        self.n_segments, self.segment_window, self._segment_n = 0, 0, []
         if keep_stages:
             self._check(self._lib.poppy_cuda_set_keep_stages(self._ctx, 1))
         if chunk_frames:
@@ -133,6 +134,53 @@ class MorphRenderer:
         self._check(self._lib.poppy_cuda_render_planned(self._ctx, int(first_slot), int(plan_first), n, _ptr(shape_ratio),
                                                         _ptr(mask_ratio), 1 if chain else 0))
         return n
+
+    # -- segments of a multi-image sequence (poppy_cuda_set_segments) -------------------------------------------------
+    def set_segments(self, n_segments: int, window: int):
+        """Room for n_segments independent chains; step j of segment s lands in ring slot s * window + j % window."""
+        self._check(self._lib.poppy_cuda_set_segments(self._ctx, int(n_segments), int(window)))
+        self.n_segments, self.segment_window = int(n_segments), int(window)
+        self._segment_n = [0] * self.n_segments
+
+    def set_segment(self, s: int, bgr1: np.ndarray, bgr2: np.ndarray, gabor2: np.ndarray | None, pts1, pts2):
+        """corrected1, corrected2, gabor2 (None: derived on the GPU) and the point sets of segment s."""
+        images = ((bgr1, np.uint8), (bgr2, np.uint8)) + (() if gabor2 is None else ((gabor2, np.float32),))
+        for a, dt in images:
+            if a.dtype != dt or a.shape[:2] != (self.height, self.width) or a.ndim != 3 or a.shape[2] != 3 \
+                    or a.strides[2] != a.itemsize or a.strides[1] != 3 * a.itemsize:
+                raise ValueError("images must be HxWx3, pixel-contiguous, uint8 (bgr) / float32 (gabor2)")
+        pts1 = np.ascontiguousarray(pts1, np.float32).reshape(-1, 2)
+        pts2 = np.ascontiguousarray(pts2, np.float32).reshape(-1, 2)
+        if pts1.shape != pts2.shape:
+            raise ValueError("point sets must both be N x 2")
+        gab, gstep = (None, 0) if gabor2 is None else (_ptr(gabor2), gabor2.strides[0])
+        self._check(self._lib.poppy_cuda_set_segment(self._ctx, int(s), _ptr(bgr1), bgr1.strides[0], _ptr(bgr2), bgr2.strides[0],
+                                                     gab, gstep, _ptr(pts1), _ptr(pts2), pts1.shape[0]))
+        self._segment_n[s] = pts1.shape[0]
+
+    def render_segments(self, first_step, shape_ratio, mask_ratio, tri_idx, tri_offsets):
+        """Steps first_step .. first_step + len(shape_ratio) - 1 of every segment. tri_offsets: n_steps * K + 1 entries, the
+        list of step first_step + r of segment s being entry r * K + s."""
+        shape_ratio = np.ascontiguousarray(shape_ratio, np.float32)
+        mask_ratio = np.ascontiguousarray(mask_ratio, np.float64)
+        tri_idx = np.ascontiguousarray(tri_idx, np.int32).reshape(-1, 3)
+        tri_offsets = np.ascontiguousarray(tri_offsets, np.int32)
+        n = shape_ratio.shape[0]
+        if mask_ratio.shape[0] != n or tri_offsets.shape[0] != n * self.n_segments + 1 or tri_offsets[-1] > tri_idx.shape[0]:
+            raise ValueError("inconsistent step / triangle-offset arrays")
+        self._check(self._lib.poppy_cuda_render_segments(self._ctx, int(first_step), n, _ptr(shape_ratio), _ptr(mask_ratio),
+                                                         _ptr(tri_idx), _ptr(tri_offsets)))
+        return n
+
+    def segment_slot(self, s: int, step: int) -> int:
+        """Ring slot of step `step` of segment s."""
+        return int(s) * self.segment_window + int(step) % self.segment_window
+
+    def segment_points(self, s: int, step: int) -> np.ndarray:
+        """morphedPoints of step `step` of segment s (its own n x 2), while the step is in the segment's window."""
+        out = np.empty((self._segment_n[s] if 0 <= s < len(self._segment_n) else 0, 2), np.float32)
+        self._check(self._lib.poppy_cuda_get_segment_points(self._ctx, int(s), int(step), _ptr(out)))
+        return out
 
     def download(self, first, count, out: np.ndarray | None = None) -> np.ndarray:
         if out is None:
