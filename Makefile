@@ -11,7 +11,7 @@ NVCCFLAGS := -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -f
 # host stages: no implicit FMA contraction (the Delaunay predicates mirror a non-FMA build of cv::Subdiv2D)
 CXXFLAGS  := -O2 -std=c++17 -fPIC -ffp-contract=off -Wall -pthread -Iinclude
 
-CU_SRC   := poppy_cuda.cu device/kernels_geometry.cu device/kernels_warp.cu device/kernels_pyramid.cu device/kernels_unsharp.cu margin.cu
+CU_SRC   := poppy_cuda.cu device/kernels_geometry.cu device/kernels_warp.cu device/kernels_pyramid.cu device/kernels_unsharp.cu margin.cu denoise.cu
 CPP_SRC  := host/delaunay.cpp host/morph_images.cpp host/host_abi.cpp host/writer.cpp
 OBJS     := $(addprefix $(OBJDIR)/,$(CU_SRC:.cu=.cu.o) $(CPP_SRC:.cpp=.cpp.o))
 HEADERS  := $(wildcard $(CSRC)/*.cuh $(CSRC)/device/*.cuh $(CSRC)/host/*.hpp include/*.h)

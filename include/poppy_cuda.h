@@ -224,7 +224,7 @@ const char* poppy_cuda_version(void);
  * one and with POPPY_CUDA_ERR_INVALID where the reference's cv::Mat ROI assertions would throw. */
 int poppy_cuda_blur_margin(int device, const uint8_t* src, size_t src_step, int cols, int rows, int union_w, int union_h,
                            uint8_t* dst, size_t dst_step);
-const char* poppy_cuda_blur_margin_last_error(void);      /* of the calling thread's last blur_margin / gabor_filter call */
+const char* poppy_cuda_blur_margin_last_error(void);      /* of the calling thread's last blur_margin / gabor_filter / denoise call */
 
 /* poppy::gabor_filter(src, dst) with the reference's defaults (src/util.cpp:40-60, src/util.hpp:95, called at
  * src/poppy.hpp:122): src / dst are float BGR (rows x cols x 3), dst = mean over 16 orientations of the clamped 13 x 13 Gabor
@@ -233,6 +233,17 @@ const char* poppy_cuda_blur_margin_last_error(void);      /* of the calling thre
  * (|diff| <= 1.2e-7 everywhere; on textured images at most 20 values per million differ by more than the DFT's own round-off
  * around zero, 1e-12; tests/test_margin.py), not bit-exact. */
 int poppy_cuda_gabor_filter(int device, const float* src, size_t src_step, int cols, int rows, float* dst, size_t dst_step);
+
+/* cv::fastNlMeansDenoising(src, dst, h, template_window_size, search_window_size) of an 8-bit BGR image (NORM_L2), as the
+ * reference's run() calls it under --denoise (src/poppy.cpp:172, 269-311), reproduced bit for bit: the weight table is built
+ * on the host with std::exp as OpenCV builds it, and every per-pixel step is exact integer arithmetic. OpenCV's defaults are
+ * h = 3, 7, 21; even window sizes round up to the next odd size, and only h * h counts. Stand-alone (no context), host
+ * input and output (src_step / dst_step: row strides in bytes); dst may equal src. Supported range, after rounding:
+ * template_window_size <= 15 and search_window_size <= 63. POPPY_CUDA_ERR_INVALID for a null pointer, cols or rows < 1,
+ * a step below cols * 3, a window size < 1 or beyond that range, or a non-finite h; POPPY_CUDA_ERR_NO_DEVICE without a
+ * GPU. Error text: poppy_cuda_blur_margin_last_error(). */
+int poppy_cuda_denoise(int device, const uint8_t* src, size_t src_step, int cols, int rows, float h, int template_window_size,
+                       int search_window_size, uint8_t* dst, size_t dst_step);
 
 #ifdef __cplusplus
 }

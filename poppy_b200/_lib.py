@@ -83,6 +83,7 @@ def load():
         "poppy_cuda_blur_margin": (i32, [i32, vp, C.c_size_t, i32, i32, i32, i32, vp, C.c_size_t]),
         "poppy_cuda_blur_margin_last_error": (C.c_char_p, []),
         "poppy_cuda_gabor_filter": (i32, [i32, vp, C.c_size_t, i32, i32, vp, C.c_size_t]),
+        "poppy_cuda_denoise": (i32, [i32, vp, C.c_size_t, i32, i32, C.c_float, i32, i32, vp, C.c_size_t]),
         "poppy_cuda_get_morphed_points": (i32, [vp, i32, vp]),
         "poppy_cuda_frame_device_ptr": (i32, [vp, i32, C.POINTER(vp), C.POINTER(C.c_size_t)]),
         "poppy_cuda_checksum": (i32, [vp, i32, i32, u64p]),
@@ -115,7 +116,7 @@ CUDA_ABI_SYMBOLS = [
     "poppy_cuda_unsharp_stats", "poppy_cuda_set_image", "poppy_cuda_set_source1_from_slot",
     "poppy_cuda_download_async", "poppy_cuda_download_wait", "poppy_cuda_alloc_pinned", "poppy_cuda_free_pinned",
     "poppy_cuda_blur_margin", "poppy_cuda_blur_margin_last_error", "poppy_cuda_gabor_filter",
-    "poppy_cuda_set_segments", "poppy_cuda_set_segment", "poppy_cuda_render_segments", "poppy_cuda_get_segment_points",
+    "poppy_cuda_denoise", "poppy_cuda_set_segments", "poppy_cuda_set_segment", "poppy_cuda_render_segments", "poppy_cuda_get_segment_points",
 ]
 HOST_ABI_SYMBOLS = [
     "poppy_host_morph_points", "poppy_host_triangulate", "poppy_host_triangulate_next", "poppy_host_chain_ratio", "poppy_host_plan_create",

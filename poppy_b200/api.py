@@ -164,6 +164,27 @@ def gabor_filter(src):
     return dst
 
 
+def denoise(src, h=3.0, template_window_size=7, search_window_size=21):
+    """cv::fastNlMeansDenoising(src, dst, h, template_window_size, search_window_size) on the GPU, bit for bit, with the same
+    defaults: the --denoise step the reference's run() applies to every input image (src/poppy.cpp:172, 269-311).
+    src: H x W x 3 uint8 (rows may be strided, as in a ROI). Returns a new H x W x 3 uint8 array."""
+    from . import _lib
+    import ctypes as C
+    src = np.asarray(src)
+    if src.dtype != np.uint8 or src.ndim != 3 or src.shape[2] != 3:
+        raise ValueError("denoise: expected an H x W x 3 uint8 image")
+    if src.strides[1:] != (3, 1) or src.strides[0] < 0:
+        src = np.ascontiguousarray(src)
+    dst = np.empty(src.shape, np.uint8)
+    lib = _lib.load()
+    rc = lib.poppy_cuda_denoise(Settings.instance().cuda_device, src.ctypes.data_as(C.c_void_p), src.strides[0], src.shape[1],
+                                src.shape[0], float(h), int(template_window_size), int(search_window_size),
+                                dst.ctypes.data_as(C.c_void_p), dst.strides[0])
+    if rc != 0:
+        raise RuntimeError(f"poppy_cuda_denoise failed ({rc}): {lib.poppy_cuda_blur_margin_last_error().decode()}")
+    return dst
+
+
 def _optional(gabor2):
     return None if gabor2 is None else np.ascontiguousarray(gabor2)
 

@@ -19,6 +19,7 @@ CUDA_SOURCES = [
     "device/kernels_pyramid.cu",
     "device/kernels_unsharp.cu",
     "margin.cu",
+    "denoise.cu",
 ]
 HOST_SOURCES = [
     "host/delaunay.cpp",

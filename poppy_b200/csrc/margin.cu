@@ -211,6 +211,8 @@ struct Rect { int x, y, w, h; };
 
 }  // namespace
 
+void margin_set_error(const std::string& msg) { g_margin_error = msg; }
+
 cudaError_t launch_gabor_mask_basis(cudaStream_t st, const uint8_t* bgr, float* m2, int bpitch, int w, int h) {
     // c_gabor_taps: written once per device. The copy is complete before the flag is raised, so a context on another stream
     // of the same device never launches ahead of it (poppy_cuda_gabor_filter rewrites the same values).
