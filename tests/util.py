@@ -15,6 +15,34 @@ def reference():
     return ref if ref.available() else port
 
 
+def any_size_inputs(w, h, seed=0, smooth=False):
+    """(bgr1, bgr2, gabor2, pts1, pts2) at any frame size, down to 1 x 1 (poppy_b200.synth needs about 8 x 8).
+    Images: seeded random bytes, or with smooth=True slow sinusoids in 70..190, whose lapBlend leaves most strip chunks
+    calm for the calm unsharp route. gabor2: a smooth field. Points: a few interior ones, points outside the frame
+    (clip_points moves them to the border), repeated points where w or h is 1, and the four corners."""
+    rng = np.random.Generator(np.random.PCG64(seed * 7919 + w * 31 + h))
+    y, x = np.mgrid[0:h, 0:w].astype(np.float64)
+    if smooth:
+        bgr1, bgr2 = (np.stack([130 + 60 * np.sin(x / (17.0 + 4 * c + k) + y / (23.0 + 3 * c) + c + 2 * k) for c in range(3)],
+                               -1).round().astype(np.uint8) for k in range(2))
+    else:
+        bgr1 = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
+        bgr2 = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
+    gab = np.stack([0.5 + 0.45 * np.sin(x / (7.0 + 3 * c) + y / (5.0 + 2 * c) + c) for c in range(3)], -1).astype(np.float32)
+    corners = np.array([[0, 0], [w - 1, 0], [0, h - 1], [w - 1, h - 1]], np.float32)
+    inner = rng.uniform(0.0, 1.0, (6, 2)) * [w - 1, h - 1]
+    outside = np.array([[-2.5, 0.3 * (h - 1)], [w + 3.25, 0.6 * (h - 1)], [0.5 * (w - 1), -1.75], [0.4 * (w - 1), h + 2.5]])
+    pts1 = np.concatenate([inner, outside]).astype(np.float32)
+    pts2 = (pts1 + rng.uniform(-2.0, 2.0, pts1.shape)).astype(np.float32)
+    pts2[:len(inner)] = np.clip(pts2[:len(inner)], 0, [w - 1, h - 1])
+    if w == 1 or h == 1:
+        pts1 = np.concatenate([pts1, pts1[:2]])
+        pts2 = np.concatenate([pts2, pts2[:2]])
+    pts1 = np.concatenate([pts1, corners])
+    pts2 = np.concatenate([pts2, corners])
+    return bgr1, bgr2, gab, pts1, pts2
+
+
 def bits_differ(a: np.ndarray, b: np.ndarray) -> int:
     """Number of elements whose bit patterns differ (floats compared as uint32, so -0/+0 and NaNs count)."""
     assert a.shape == b.shape, (a.shape, b.shape)
