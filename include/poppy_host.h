@@ -94,8 +94,8 @@ void poppy_host_writer_destroy(poppy_host_writer* w);
 
 /* The C++ shim (poppy_b200/csrc/host/morph_images.hpp: poppy::Settings, poppy::morph_images, poppy::morph_sequence with
  * the reference's argument order and semantics) behind C entry points, for callers and tests without a C++ toolchain:
- * the shim keeps its own device context (per frame size / pyramid levels), runs the host stages and, for a sequence, the
- * sliced chain render + writer ring; `write` receives the frames in order (reference src/poppy.hpp:177-243).
+ * the shim keeps its own device context per GPU (for the last frame size / pyramid levels), runs the host stages and, for
+ * a sequence, the sliced chain render + writer ring; `write` receives the frames in order (reference src/poppy.hpp:177-243).
  * poppy_shim_morph_sequence takes gabor2 == NULL (gstep ignored): gabor2 is then derived on the device from corrected2, as
  * poppy::morph() derives it before its frame loop (src/poppy.hpp:119-122; poppy_cuda_set_pair). The per-frame entry points
  * keep requiring gabor2, as the reference's morph_images() does. */
@@ -123,7 +123,16 @@ typedef struct poppy_shim_segment {
 } poppy_shim_segment;
 int poppy_shim_morph_segments(int width, int height, int pyramid_levels, const poppy_shim_segment* segments, int n_segments,
                               int number_of_frames, poppy_write_fn write, void* user);
-void poppy_shim_release(void);
+/* The same on several GPUs of one box: the segments are sharded over the first G = min(n_devices, n_segments) entries of
+ * `devices`, devices[g] rendering segments [g * K / G, (g + 1) * K / G) on its own context and host thread (the others stay
+ * idle). The frames and the order of the `write` calls equal poppy_shim_morph_segments's; `write` is called from a library
+ * thread, one call at a time. Before anything is planned or rendered: POPPY_CUDA_ERR_INVALID for devices == NULL,
+ * n_devices < 1, a duplicate or a negative index, then POPPY_CUDA_ERR_NO_DEVICE without a GPU, then POPPY_CUDA_ERR_INVALID
+ * for an index >= poppy_cuda_device_count(). */
+int poppy_shim_morph_segments_devices(const int* devices, int n_devices, int width, int height, int pyramid_levels,
+                                      const poppy_shim_segment* segments, int n_segments, int number_of_frames, poppy_write_fn write,
+                                      void* user);
+void poppy_shim_release(void);            /* frees the shim's cached contexts, one per device used */
 
 const char* poppy_host_last_error(void);
 

@@ -75,6 +75,7 @@ def load():
         "poppy_cuda_render_segments": (i32, [vp, i32, i32, vp, vp, vp, vp]),
         "poppy_cuda_get_segment_points": (i32, [vp, i32, i32, vp]),
         "poppy_shim_morph_segments": (i32, [i32, i32, i32, vp, i32, i32, vp, vp]),
+        "poppy_shim_morph_segments_devices": (i32, [vp, i32, i32, i32, i32, vp, i32, i32, vp, vp]),
         "poppy_cuda_download": (i32, [vp, i32, i32, vp, C.c_size_t, C.c_size_t]),
         "poppy_cuda_download_async": (i32, [vp, i32, i32, vp, C.c_size_t, C.c_size_t, u64p]),
         "poppy_cuda_download_wait": (i32, [vp, C.c_uint64]),
@@ -123,5 +124,6 @@ HOST_ABI_SYMBOLS = [
     "poppy_host_plan_triangles", "poppy_host_plan_points", "poppy_host_plan_destroy", "poppy_morph_images",
     "poppy_host_last_error", "poppy_host_writer_create", "poppy_host_writer_create_io", "poppy_host_writer_submit",
     "poppy_host_writer_flush", "poppy_host_writer_destroy", "poppy_host_writer_destroy_cuda",
-    "poppy_shim_morph_images", "poppy_shim_morph_sequence", "poppy_shim_morph_segments", "poppy_shim_release",
+    "poppy_shim_morph_images", "poppy_shim_morph_sequence", "poppy_shim_morph_segments", "poppy_shim_morph_segments_devices",
+    "poppy_shim_release",
 ]

@@ -9,7 +9,8 @@
                           the chain recurrence kept resident on the GPU, frames handed to writer.write() in order
   render_phases(...)      direct mode: N independent phases of one pair ("-f 1 -p s", src/poppy.hpp:186-200)
   morph_segments(...)     the segments of a multi-image sequence (reference run(), src/poppy.cpp:266-328): one chain per
-                          consecutive pair, rendered together (step j of every segment in one kernel batch)
+                          consecutive pair, rendered together (step j of every segment in one kernel batch); with
+                          devices=[...] sharded by segment over several GPUs of one box
 
 morph_sequence and render_phases take gabor2=None: the GPU then derives it from corrected2 exactly as poppy::morph()
 does before its frame loop (gabor_filter(corrected2 * 1/255), src/poppy.hpp:119-122), and the float image never exists.
@@ -21,12 +22,13 @@ from __future__ import annotations
 
 from dataclasses import dataclass
 
+import operator
 import threading
 
 import numpy as np
 
-from . import host
-from .renderer import MorphRenderer
+from . import host, shard
+from .renderer import MorphRenderer, device_count
 
 
 @dataclass
@@ -85,10 +87,29 @@ def _renderer(w, h, n_points, n_tri, n_frames) -> MorphRenderer:
     return r
 
 
+# renderers of morph_segments(devices=...) on the listed GPUs other than Settings.cuda_device, one per device: they neither evict
+# nor replace the renderer in _cache, which the single-device entry points share
+_device_cache: dict = {}
+
+
+def _device_renderer(device, w, h, n_points, n_tri, n_frames) -> MorphRenderer:
+    levels = int(Settings.instance().pyramid_levels)
+    r = _device_cache.get(device)
+    if r is None or (r.width, r.height, r.levels) != (w, h, levels) or r.max_points < n_points or r.max_triangles < n_tri \
+            or r.max_batch_frames < n_frames:
+        if r is not None:
+            r.close()
+            del _device_cache[device]
+        r = MorphRenderer(w, h, levels, max(n_points, 64), max(n_tri, 2 * n_points + 16), n_frames, device=device)
+        _device_cache[device] = r
+    return r
+
+
 def release():
-    for r in _cache.values():
+    for r in list(_cache.values()) + list(_device_cache.values()):
         r.close()
     _cache.clear()
+    _device_cache.clear()
 
 
 def morph_images(img1, img2, corrected1, corrected2, gabor2, src_points1, src_points2, shape_ratio, mask_ratio,
@@ -245,12 +266,54 @@ def interleave_segment_plans(plans, n_steps):
 _SEGMENT_RING_BYTES = 8 << 30
 
 
-def morph_segments(segments, number_of_frames=None, writer=None, threads=0):
+def _check_devices(devices):
+    """The device list of morph_segments, checked before anything is planned or rendered."""
+    devices = [operator.index(d) for d in devices]
+    if not devices:
+        raise ValueError("morph_segments: the device list is empty")
+    if any(d < 0 for d in devices):
+        raise ValueError(f"morph_segments: negative device index in {devices}")
+    if len(set(devices)) != len(devices):
+        raise ValueError(f"morph_segments: a device is listed twice in {devices}")
+    n = device_count()
+    if n <= 0:
+        raise RuntimeError("morph_segments: no CUDA device: the morph renderer has no CPU fallback")
+    if any(d >= n for d in devices):
+        raise ValueError(f"morph_segments: device index out of [0, {n}) in {devices}")
+    return devices
+
+
+def _render_segment_range(r, segments, plans, lo, hi, per_batch, shape, ratio, frames, stop=None):
+    """Segments [lo, hi) on renderer r, per_batch at a time, downloaded into frames[lo:hi]."""
+    n_frames, h, w = frames.shape[1:4]
+    for b0 in range(lo, hi, per_batch):
+        if stop is not None and stop.is_set():
+            return
+        batch = range(b0, min(hi, b0 + per_batch))
+        r.set_segments(len(batch), n_frames)
+        for i, s in enumerate(batch):
+            c1, c2, g2, p1, p2 = segments[s]
+            r.set_segment(i, np.ascontiguousarray(c1), np.ascontiguousarray(c2), _optional(g2), np.reshape(p1, (-1, 2)),
+                          np.reshape(p2, (-1, 2)))
+        tri, offs = interleave_segment_plans([plans[s] for s in batch], n_frames)
+        r.render_segments(0, shape, ratio, tri, offs)
+        r.download(0, len(batch) * n_frames, out=frames[b0:b0 + len(batch)].reshape(-1, h, w, 3))
+
+
+def morph_segments(segments, number_of_frames=None, writer=None, threads=0, devices=None):
     """The segments of a multi-image sequence: segments[i] = (corrected1, corrected2, gabor2 or None, pts1, pts2) of one
     consecutive pair, all of one frame size. Each is the chain morph_sequence renders, and they are rendered together.
     Returns the frames as a (K, N, H, W, 3) array and calls writer.write(frame) in the reference's order: the N frames of
-    segment 0, then those of segment 1, and so on (one video, as run() writes it)."""
+    segment 0, then those of segment 1, and so on (one video, as run() writes it).
+
+    devices=None renders on Settings.cuda_device. devices=[d0, d1, ...] shards the K segments over the first
+    G = min(len(devices), K) of those GPUs: devices[g] renders the contiguous range shard.phase_range(g, G, K) on its own
+    renderer and Python thread, each as the single-device call does with its own ring budget. The result and the writer
+    calls are the same as with one device. An empty list, a duplicate, a negative index or an index >= device_count()
+    raises ValueError, and RuntimeError is raised without a GPU, before anything is planned or rendered."""
     n_frames = int(number_of_frames if number_of_frames is not None else Settings.instance().number_of_frames)
+    if devices is not None:
+        devices = _check_devices(devices)
     K = len(segments)
     if K == 0:
         raise ValueError("morph_segments: no segments")
@@ -265,19 +328,36 @@ def morph_segments(segments, number_of_frames=None, writer=None, threads=0):
     plans = [host.SequencePlan(np.reshape(p1, (-1, 2)), np.reshape(p2, (-1, 2)), w, h, shape, chain=True, threads=threads)
              for _, _, _, p1, p2 in segments]
     frames = np.empty((K, n_frames, h, w, 3), np.uint8)
+    n_max, tri_max = max(p.n for p in plans), max(p.max_triangles for p in plans)
+
+    def per_batch(count):
+        return max(1, min(count, _SEGMENT_RING_BYTES // (n_frames * w * h * 3)))
+
     try:
-        per_batch = max(1, min(K, _SEGMENT_RING_BYTES // (n_frames * w * h * 3)))
-        r = _renderer(w, h, max(p.n for p in plans), max(p.max_triangles for p in plans), per_batch * n_frames)
-        for b0 in range(0, K, per_batch):
-            batch = range(b0, min(K, b0 + per_batch))
-            r.set_segments(len(batch), n_frames)
-            for i, s in enumerate(batch):
-                c1, c2, g2, p1, p2 = segments[s]
-                r.set_segment(i, np.ascontiguousarray(c1), np.ascontiguousarray(c2), _optional(g2), np.reshape(p1, (-1, 2)),
-                              np.reshape(p2, (-1, 2)))
-            tri, offs = interleave_segment_plans([plans[s] for s in batch], n_frames)
-            r.render_segments(0, shape, ratio, tri, offs)
-            r.download(0, len(batch) * n_frames, out=frames[b0:b0 + len(batch)].reshape(-1, h, w, 3))
+        if devices is None:
+            r = _renderer(w, h, n_max, tri_max, per_batch(K) * n_frames)
+            _render_segment_range(r, segments, plans, 0, K, per_batch(K), shape, ratio, frames)
+        else:
+            G = min(len(devices), K)
+            stop, errors = threading.Event(), []
+
+            def run(g):
+                try:
+                    lo, hi = shard.phase_range(g, G, K)
+                    d, b = devices[g], per_batch(hi - lo)
+                    r = _renderer(w, h, n_max, tri_max, b * n_frames) if d == Settings.instance().cuda_device \
+                        else _device_renderer(d, w, h, n_max, tri_max, b * n_frames)
+                    _render_segment_range(r, segments, plans, lo, hi, b, shape, ratio, frames, stop)
+                except BaseException as e:      # the other devices stop before their next batch; re-raised below
+                    errors.append(e)
+                    stop.set()
+            workers = [threading.Thread(target=run, args=(g,)) for g in range(G)]
+            for t in workers:
+                t.start()
+            for t in workers:
+                t.join()
+            if errors:
+                raise errors[0]
     finally:
         for p in plans:
             p.close()

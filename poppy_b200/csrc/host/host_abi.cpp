@@ -54,12 +54,34 @@ struct poppy_host_plan {
 namespace {
 template <class F> int shim_guard(F&& f) {
     try { f(); return 0; }
+    catch (const poppy::NoDeviceError& e) { return host_fail(POPPY_CUDA_ERR_NO_DEVICE, e.what()); }
     catch (const poppy::MorphError& e) { return host_fail(POPPY_CUDA_ERR_INVALID, e.what()); }
     catch (const std::exception& e) { return host_fail(POPPY_CUDA_ERR_INVALID, e.what()); }
 }
 poppy::Image8 view8(const uint8_t* p, int w, int h, size_t step) {
     poppy::Image8 v;
     v.data = const_cast<uint8_t*>(p); v.cols = w; v.rows = h; v.step = step;
+    return v;
+}
+
+int check_shim_segments(const poppy_shim_segment* segs, int n_segments, poppy_write_fn write) {
+    if (!segs || !write || n_segments < 1) return host_fail(POPPY_CUDA_ERR_INVALID, "null argument");
+    for (int s = 0; s < n_segments; ++s)
+        if (!segs[s].corrected1 || !segs[s].corrected2 || segs[s].n < 0 || (segs[s].n > 0 && (!segs[s].pts1_xy || !segs[s].pts2_xy)))
+            return host_fail(POPPY_CUDA_ERR_INVALID, "segment " + std::to_string(s) + ": null argument");
+    return 0;
+}
+
+std::vector<poppy::Segment> shim_segments(int w, int h, const poppy_shim_segment* segs, int n_segments) {
+    std::vector<poppy::Segment> v(n_segments);
+    for (int s = 0; s < n_segments; ++s) {
+        const poppy_shim_segment& g = segs[s];
+        v[s].corrected1 = view8(g.corrected1, w, h, g.step1);
+        v[s].corrected2 = view8(g.corrected2, w, h, g.step2);
+        if (g.gabor2) { v[s].gabor2.data = g.gabor2; v[s].gabor2.cols = w; v[s].gabor2.rows = h; v[s].gabor2.step = g.gstep; }
+        v[s].srcPoints1 = to_points(g.pts1_xy, g.n);
+        v[s].srcPoints2 = to_points(g.pts2_xy, g.n);
+    }
     return v;
 }
 }  // namespace
@@ -294,23 +316,25 @@ int poppy_shim_morph_sequence(int w, int h, int pyramid_levels, const uint8_t* c
 
 int poppy_shim_morph_segments(int w, int h, int pyramid_levels, const poppy_shim_segment* segs, int n_segments, int n_frames,
                               poppy_write_fn write, void* user) {
-    if (!segs || !write || n_segments < 1) return host_fail(POPPY_CUDA_ERR_INVALID, "null argument");
-    for (int s = 0; s < n_segments; ++s)
-        if (!segs[s].corrected1 || !segs[s].corrected2 || segs[s].n < 0 || (segs[s].n > 0 && (!segs[s].pts1_xy || !segs[s].pts2_xy)))
-            return host_fail(POPPY_CUDA_ERR_INVALID, "segment " + std::to_string(s) + ": null argument");
+    if (int rc = check_shim_segments(segs, n_segments, write)) return rc;
     return shim_guard([&] {
         poppy::Settings::instance().pyramid_levels = (size_t)pyramid_levels;
-        std::vector<poppy::Segment> v(n_segments);
-        for (int s = 0; s < n_segments; ++s) {
-            const poppy_shim_segment& g = segs[s];
-            v[s].corrected1 = view8(g.corrected1, w, h, g.step1);
-            v[s].corrected2 = view8(g.corrected2, w, h, g.step2);
-            if (g.gabor2) { v[s].gabor2.data = g.gabor2; v[s].gabor2.cols = w; v[s].gabor2.rows = h; v[s].gabor2.step = g.gstep; }
-            v[s].srcPoints1 = to_points(g.pts1_xy, g.n);
-            v[s].srcPoints2 = to_points(g.pts2_xy, g.n);
-        }
         int index = 0;
-        poppy::morph_segments(v, n_frames, [&](const poppy::Image8& f) { write(user, index++, f.data, f.cols, f.rows, f.step); });
+        poppy::morph_segments(shim_segments(w, h, segs, n_segments), n_frames,
+                              [&](const poppy::Image8& f) { write(user, index++, f.data, f.cols, f.rows, f.step); });
+    });
+}
+
+int poppy_shim_morph_segments_devices(const int* devices, int n_devices, int w, int h, int pyramid_levels, const poppy_shim_segment* segs,
+                                      int n_segments, int n_frames, poppy_write_fn write, void* user) {
+    if (!devices || n_devices < 1) return host_fail(POPPY_CUDA_ERR_INVALID, "no devices");
+    if (int rc = check_shim_segments(segs, n_segments, write)) return rc;
+    return shim_guard([&] {
+        poppy::Settings::instance().pyramid_levels = (size_t)pyramid_levels;
+        int index = 0;
+        poppy::morph_segments(shim_segments(w, h, segs, n_segments), n_frames,
+                              [&](const poppy::Image8& f) { write(user, index++, f.data, f.cols, f.rows, f.step); },
+                              std::vector<int>(devices, devices + n_devices));
     });
 }
 

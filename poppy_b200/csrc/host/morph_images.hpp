@@ -70,6 +70,11 @@ class MorphError : public std::runtime_error {
 public:
     using std::runtime_error::runtime_error;
 };
+// thrown by calls that check for a CUDA device up front when the machine has none
+class NoDeviceError : public MorphError {
+public:
+    using MorphError::MorphError;
+};
 
 // reference src/algo.hpp:26 / src/algo.cpp:178-273. img1 supplies only the frame size; goodFeatures1/2, img2, last
 // and linear are unused exactly as in the reference. dst is (re)allocated when its size differs.
@@ -99,8 +104,16 @@ struct Segment {
 // GPU (step j of a group of segments per kernel batch). Frames go to `write` in the reference's order: all
 // number_of_frames frames of segment 0, then segment 1, ...; segment 0's are written while later steps still render.
 void morph_segments(const std::vector<Segment>& segments, int number_of_frames, const std::function<void(const Image8&)>& write);
+// The same on several GPUs of one box: the K segments are sharded over the first G = min(devices.size(), K) listed devices,
+// devices[g] rendering the contiguous range [g * K / G, (g + 1) * K / G) on its own context and host thread; the other
+// listed devices stay idle. The frames and the order of the `write` calls equal the single-device call's: `write` is
+// called from a library thread, one call at a time. The device list is checked before anything is planned or rendered:
+// MorphError for an empty list, a duplicate, a negative index or an index >= the device count, NoDeviceError without a GPU.
+// If one device fails, the others stop at their next render call and the first error is thrown once all have stopped.
+void morph_segments(const std::vector<Segment>& segments, int number_of_frames, const std::function<void(const Image8&)>& write,
+                    const std::vector<int>& devices);
 
-// Releases the cached device context(s) held by morph_images()/morph_sequence().
+// Releases the cached device contexts (one per device) held by morph_images()/morph_sequence()/morph_segments().
 void release_cached_contexts();
 
 }  // namespace poppy
