@@ -179,6 +179,18 @@ int poppy_cuda_download(poppy_cuda_ctx* ctx, int first, int count, uint8_t* dst,
 int poppy_cuda_download_async(poppy_cuda_ctx* ctx, int first, int count, uint8_t* dst, size_t step, size_t frame_stride,
                               uint64_t* ticket);
 int poppy_cuda_download_wait(poppy_cuda_ctx* ctx, uint64_t ticket);
+
+/* Frames [first, first+count) as I420 (YUV 4:2:0, BT.601 limited range), byte for byte what
+ * cv::cvtColor(bgr, out, COLOR_BGR2YUV_I420) gives for the BGR frame: per frame the Y plane (W x H), then U and V ((W/2) x (H/2)
+ * each), every row tightly packed, W*H*3/2 bytes; frame i lands at dst + i * frame_stride. Chroma is the top-left pixel of each
+ * 2 x 2 block. The conversion runs on the device, so half the bytes of a BGR download cross PCIe. Ordering is that of
+ * poppy_cuda_download: the conversion and the copies run on the copy stream after every render queued so far, and a later
+ * render of these slots waits for both. Device staging of a few frames is allocated on the first call; a larger count goes
+ * through it in pieces. POPPY_CUDA_ERR_INVALID for an odd W or H (cv::cvtColor throws there too), a null dst, a bad range or
+ * frame_stride < W*H*3/2. Asynchronous if dst is pinned; poppy_cuda_sync() before reading. The _async flavour returns a ticket
+ * of the same pool as poppy_cuda_download_async, for poppy_cuda_download_wait. */
+int poppy_cuda_download_i420(poppy_cuda_ctx* ctx, int first, int count, uint8_t* dst, size_t frame_stride);
+int poppy_cuda_download_i420_async(poppy_cuda_ctx* ctx, int first, int count, uint8_t* dst, size_t frame_stride, uint64_t* ticket);
 /* Page-locked host memory for download targets (asynchronous copies need it). */
 int poppy_cuda_alloc_pinned(size_t bytes, void** out);
 void poppy_cuda_free_pinned(void* p);

@@ -76,6 +76,12 @@ int poppy_host_writer_create(poppy_host_writer** out, poppy_cuda_ctx* ctx, int r
 int poppy_host_writer_submit(poppy_host_writer* w, int first_slot, int count, int first_frame_index);
 int poppy_host_writer_flush(poppy_host_writer* w);          /* returns once every submitted frame has been written */
 void poppy_host_writer_destroy_cuda(poppy_host_writer* w);  /* flushes, joins the threads, frees the ring */
+/* The same ring delivering I420 frames (poppy_cuda_download_i420_async: converted on the GPU, W*H*3/2 bytes per buffer), the
+ * pixel format of encoders fed yuv420p. `write` / `convert` receive a pointer to the Y plane with step = W; the U plane follows
+ * at +W*H and the V plane at +W*H*5/4, (W/2) x (H/2) bytes each with rows of W/2 bytes. POPPY_CUDA_ERR_INVALID for an odd frame
+ * size. Destroy it with poppy_host_writer_destroy_cuda. */
+int poppy_host_writer_create_i420(poppy_host_writer** out, poppy_cuda_ctx* ctx, int ring_frames, poppy_write_fn write,
+                                  poppy_write_fn convert /* may be NULL */, int workers, void* user);
 
 /* The same machinery over a caller-supplied transport (tests run it without a GPU; another source of frames can reuse it). */
 typedef struct poppy_host_writer_io {

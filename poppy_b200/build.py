@@ -18,6 +18,7 @@ CUDA_SOURCES = [
     "device/kernels_warp.cu",
     "device/kernels_pyramid.cu",
     "device/kernels_unsharp.cu",
+    "device/kernels_yuv.cu",
     "margin.cu",
     "denoise.cu",
 ]

@@ -137,4 +137,10 @@ constexpr int CALM_BLOCK_W = 4, CALM_BLOCK_H = 8;
 // order-dependent checksum of a byte range
 void launch_checksum(cudaStream_t st, const uint8_t* data, size_t bytes, unsigned long long* out);
 
+// ---- kernels_yuv.cu ----------------------------------------------------------------------------------------------
+// ring slots [first_slot, first_slot + frames) (BGR, frame_bytes apart) -> packed I420 frames at out, w * h * 3 / 2 bytes
+// apart, as cv::cvtColor(COLOR_BGR2YUV_I420). w and h even; frames <= 65535.
+void launch_bgr_to_i420(cudaStream_t st, const uint8_t* ring, size_t frame_bytes, int first_slot, int frames, uint8_t* out, int w,
+                        int h);
+
 }  // namespace poppy

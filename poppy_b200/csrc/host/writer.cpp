@@ -18,7 +18,7 @@
 struct poppy_host_writer {
     poppy_host_writer_io io{};
     int width = 0, height = 0, ring = 0, workers = 0;
-    size_t frame_bytes = 0;
+    size_t row_bytes = 0, frame_bytes = 0;      // of one ring buffer: BGR rows (width * 3), or the Y rows of an I420 frame
     std::vector<uint8_t*> buffers;              // page-locked frame buffers
     struct Item { int frame_index; int buffer; uint64_t ticket; bool converted; };
     std::mutex mu;
@@ -45,7 +45,7 @@ struct poppy_host_writer {
             if (workers == 0) {
                 if (io.wait && io.wait(io.user, it.ticket) != 0) { std::lock_guard<std::mutex> lk(mu); error = POPPY_CUDA_ERR_CUDA; }
             }
-            if (io.write) io.write(io.user, it.frame_index, buffers[it.buffer], width, height, (size_t)width * 3);
+            if (io.write) io.write(io.user, it.frame_index, buffers[it.buffer], width, height, row_bytes);
             {
                 std::lock_guard<std::mutex> lk(mu);
                 pending.pop_front();
@@ -70,7 +70,7 @@ struct poppy_host_writer {
                 it = pending[idx];
             }
             if (io.wait && io.wait(io.user, it.ticket) != 0) { std::lock_guard<std::mutex> lk(mu); error = POPPY_CUDA_ERR_CUDA; }
-            if (io.convert) io.convert(io.user, it.frame_index, buffers[it.buffer], width, height, (size_t)width * 3);
+            if (io.convert) io.convert(io.user, it.frame_index, buffers[it.buffer], width, height, row_bytes);
             {
                 std::lock_guard<std::mutex> lk(mu);
                 // entries only leave at the front, and only after they are converted: find ours by frame index
@@ -82,10 +82,9 @@ struct poppy_host_writer {
     }
 };
 
-extern "C" {
-
-int poppy_host_writer_create_io(poppy_host_writer** out, const poppy_host_writer_io* io, int width, int height, int ring_frames,
-                                int workers) {
+namespace {
+int writer_create(poppy_host_writer** out, const poppy_host_writer_io* io, int width, int height, size_t row_bytes, size_t frame_bytes,
+                  int ring_frames, int workers) {
     if (!out) return POPPY_CUDA_ERR_INVALID;
     *out = nullptr;
     if (!io || !io->download || !io->write || !io->alloc || !io->release || width <= 0 || height <= 0 || ring_frames < 1 || workers < 0)
@@ -93,7 +92,7 @@ int poppy_host_writer_create_io(poppy_host_writer** out, const poppy_host_writer
     poppy_host_writer* w = new poppy_host_writer();
     w->io = *io;
     w->width = width; w->height = height; w->ring = ring_frames; w->workers = io->convert ? workers : 0;
-    w->frame_bytes = (size_t)width * height * 3;
+    w->row_bytes = row_bytes; w->frame_bytes = frame_bytes;
     for (int i = 0; i < ring_frames; ++i) {
         void* p = nullptr;
         if (io->alloc(io->user, w->frame_bytes, &p) != 0 || !p) {
@@ -109,6 +108,14 @@ int poppy_host_writer_create_io(poppy_host_writer** out, const poppy_host_writer
     *out = w;
     return 0;
 }
+}  // namespace
+
+extern "C" {
+
+int poppy_host_writer_create_io(poppy_host_writer** out, const poppy_host_writer_io* io, int width, int height, int ring_frames,
+                                int workers) {
+    return writer_create(out, io, width, height, (size_t)width * 3, (size_t)width * height * 3, ring_frames, workers);
+}
 
 int poppy_host_writer_submit(poppy_host_writer* w, int first_slot, int count, int first_frame_index) {
     if (!w || count < 0) return POPPY_CUDA_ERR_INVALID;
@@ -121,7 +128,7 @@ int poppy_host_writer_submit(poppy_host_writer* w, int first_slot, int count, in
             w->free_buffers.pop_front();
         }
         uint64_t ticket = 0;
-        const int rc = w->io.download(w->io.user, first_slot + i, w->buffers[buf], (size_t)w->width * 3, &ticket);
+        const int rc = w->io.download(w->io.user, first_slot + i, w->buffers[buf], w->row_bytes, &ticket);
         if (rc != 0) {
             std::lock_guard<std::mutex> lk(w->mu);
             w->free_buffers.push_back(buf);
@@ -165,28 +172,45 @@ int ct_download(void* u, int slot, uint8_t* dst, size_t step, uint64_t* ticket) 
     auto* t = (CudaTransport*)u;
     return poppy_cuda_download_async(t->ctx, slot, 1, dst, step, step * (size_t)t->h, ticket);
 }
+int ct_download_i420(void* u, int slot, uint8_t* dst, size_t, uint64_t* ticket) {
+    auto* t = (CudaTransport*)u;
+    return poppy_cuda_download_i420_async(t->ctx, slot, 1, dst, (size_t)t->w * t->h * 3 / 2, ticket);
+}
 int ct_wait(void* u, uint64_t ticket) { return poppy_cuda_download_wait(((CudaTransport*)u)->ctx, ticket); }
 int ct_alloc(void*, size_t bytes, void** out) { return poppy_cuda_alloc_pinned(bytes, out); }
 void ct_release(void*, void* p) { poppy_cuda_free_pinned(p); }
 void ct_write(void* u, int idx, uint8_t* bgr, int w, int h, size_t step) { auto* t = (CudaTransport*)u; t->write(t->user, idx, bgr, w, h, step); }
 void ct_convert(void* u, int idx, uint8_t* bgr, int w, int h, size_t step) { auto* t = (CudaTransport*)u; t->convert(t->user, idx, bgr, w, h, step); }
-}  // namespace
 
-int poppy_host_writer_create(poppy_host_writer** out, poppy_cuda_ctx* ctx, int ring_frames, poppy_write_fn write,
-                             poppy_write_fn convert, int workers, void* user) {
+int cuda_writer_create(poppy_host_writer** out, poppy_cuda_ctx* ctx, int ring_frames, poppy_write_fn write, poppy_write_fn convert,
+                       int workers, void* user, bool i420) {
     if (!out || !ctx || !write) return POPPY_CUDA_ERR_INVALID;
     int w = 0, h = 0;
     if (int rc = poppy_cuda_get_info(ctx, &w, &h, nullptr, nullptr, nullptr, nullptr)) return rc;
+    if (i420 && ((w | h) & 1)) return POPPY_CUDA_ERR_INVALID;         // I420 needs an even frame size
     // at most 64 download tickets may be outstanding (poppy_cuda.h)
     if (ring_frames > 48) ring_frames = 48;
     auto* t = new CudaTransport{ctx, write, convert, user, w, h};
     poppy_host_writer_io io{};
-    io.user = t; io.download = ct_download; io.wait = ct_wait; io.alloc = ct_alloc; io.release = ct_release; io.write = ct_write;
+    io.user = t; io.download = i420 ? ct_download_i420 : ct_download; io.wait = ct_wait; io.alloc = ct_alloc; io.release = ct_release;
+    io.write = ct_write;
     io.convert = convert ? ct_convert : nullptr;
-    const int rc = poppy_host_writer_create_io(out, &io, w, h, ring_frames, workers);
+    const int rc = i420 ? writer_create(out, &io, w, h, (size_t)w, (size_t)w * h * 3 / 2, ring_frames, workers)
+                        : poppy_host_writer_create_io(out, &io, w, h, ring_frames, workers);
     if (rc != 0) { delete t; return rc; }
     (*out)->io.owned_transport = t;
     return 0;
+}
+}  // namespace
+
+int poppy_host_writer_create(poppy_host_writer** out, poppy_cuda_ctx* ctx, int ring_frames, poppy_write_fn write,
+                             poppy_write_fn convert, int workers, void* user) {
+    return cuda_writer_create(out, ctx, ring_frames, write, convert, workers, user, false);
+}
+
+int poppy_host_writer_create_i420(poppy_host_writer** out, poppy_cuda_ctx* ctx, int ring_frames, poppy_write_fn write,
+                                  poppy_write_fn convert, int workers, void* user) {
+    return cuda_writer_create(out, ctx, ring_frames, write, convert, workers, user, true);
 }
 
 void poppy_host_writer_destroy_cuda(poppy_host_writer* w) {

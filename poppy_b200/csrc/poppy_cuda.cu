@@ -8,6 +8,7 @@
 //   chunk scratch (xB): FrameParams; triangle indices; TriInverse / TriRaster records; triangle-ID map int32 [H][W];
 //                       warped pair 2 x uint32 BGRX [H][pitch0]; Gaussian levels 1..L (7 planes); collapsed levels 0..L
 //                       (3 planes); level-0 blend mask float [H][pitch0]
+//   I420 staging      : (optional, poppy_cuda_download_i420) up to kI420StageFrames x W*H*3/2 bytes, allocated on first use
 //   segments (optional, poppy_cuda_set_segments): per segment the pair's resident data - corrected1, corrected2 and chain
 //                       arrays, a mask basis (one allocation, padded_pixels() floats each), raw and clipped point sets;
 //                       per lane a SegFrame table and a BGRX staging plane per frame of a chunk
@@ -53,6 +54,9 @@ constexpr int kSparseChunkRows = 24;
 // 2: 2,952, 3: 3,150, 4: 3,219-3,259, 8: 3,263 frames/s.
 constexpr int kRenderLanes = 4;
 
+// I420 downloads convert at most this many frames per piece into device staging (a 4K frame is 12.4 MB in I420)
+constexpr int kI420StageFrames = 8;
+
 }  // namespace
 
 struct poppy_cuda_ctx {
@@ -75,6 +79,8 @@ struct poppy_cuda_ctx {
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t ev_rendered = nullptr, ev_copied = nullptr;
     int copy_lo = 0, copy_hi = 0;        // ring slots [lo, hi) with a download enqueued since the last sync
+    uint8_t* d_i420 = nullptr;           // I420 staging of poppy_cuda_download_i420 (copy stream only)
+    int i420_frames = 0;                 // frames d_i420 holds
     std::string err;
     uint64_t launches = 0;
 
@@ -755,7 +761,7 @@ void poppy_cuda_destroy(poppy_cuda_ctx* c) {
     }
     cudaFree(c->d_pts1_raw); cudaFree(c->d_pts2_raw); cudaFree(c->d_pts1); cudaFree(c->d_pts2); cudaFree(c->d_morphed);
     cudaFree(c->d_tail_levels);
-    cudaFree(c->d_frames); cudaFree(c->d_sum); cudaFree(c->d_calm_total); cudaFree(c->d_probe_total); cudaFree(c->d_plan_tri);
+    cudaFree(c->d_frames); cudaFree(c->d_i420); cudaFree(c->d_sum); cudaFree(c->d_calm_total); cudaFree(c->d_probe_total); cudaFree(c->d_plan_tri);
     if (c->ev_begin) cudaEventDestroy(c->ev_begin);
     if (c->ev_end) cudaEventDestroy(c->ev_end);
     if (c->ev_rendered) cudaEventDestroy(c->ev_rendered);
@@ -1190,34 +1196,25 @@ int poppy_cuda_get_segment_points(poppy_cuda_ctx* c, int s, int step, float* xy)
     return 0;
 }
 
-int poppy_cuda_download(poppy_cuda_ctx* c, int first, int count, uint8_t* dst, size_t step, size_t frame_stride) {
-    if (!c) return POPPY_CUDA_ERR_INVALID;
-    const size_t row = (size_t)c->w * 3;
-    if (!dst || first < 0 || count < 1 || first + count > c->max_frames || step < row || frame_stride < step * c->h)
-        return fail(c, POPPY_CUDA_ERR_INVALID, "bad download range or strides");
-    CU_TRY(c, cudaSetDevice(c->device));
-    // after everything queued on the context's stream so far (the renders that produce these slots), but on the copy
-    // stream: later renders of other slots are not held up by the transfer
+namespace {
+
+// Downloads run after everything queued on the context's stream so far (the renders that produce their slots), but on the
+// copy stream: later renders of other slots are not held up by the transfer.
+int copy_after_renders(poppy_cuda_ctx* c) {
     CU_TRY(c, cudaEventRecord(c->ev_rendered, c->stream));
     CU_TRY(c, cudaStreamWaitEvent(c->copy_stream, c->ev_rendered, 0));
-    if (step == row && frame_stride == c->frame_bytes()) {
-        CU_TRY(c, cudaMemcpyAsync(dst, c->d_frames + (size_t)first * c->frame_bytes(), (size_t)count * c->frame_bytes(),
-                                  cudaMemcpyDeviceToHost, c->copy_stream));
-    } else {
-        for (int i = 0; i < count; ++i)
-            CU_TRY(c, cudaMemcpy2DAsync(dst + (size_t)i * frame_stride, step, c->d_frames + (size_t)(first + i) * c->frame_bytes(),
-                                        row, row, c->h, cudaMemcpyDeviceToHost, c->copy_stream));
-    }
+    return 0;
+}
+
+// After the copy-stream work of a download of slots [first, first + count): a later render of those slots waits for it.
+int copies_enqueued(poppy_cuda_ctx* c, int first, int count) {
     CU_TRY(c, cudaEventRecord(c->ev_copied, c->copy_stream));
     if (c->copy_hi <= c->copy_lo) { c->copy_lo = first; c->copy_hi = first + count; }
     else { c->copy_lo = std::min(c->copy_lo, first); c->copy_hi = std::max(c->copy_hi, first + count); }
     return 0;
 }
 
-int poppy_cuda_download_async(poppy_cuda_ctx* c, int first, int count, uint8_t* dst, size_t step, size_t frame_stride,
-                              uint64_t* ticket) {
-    if (!c || !ticket) return POPPY_CUDA_ERR_INVALID;
-    if (int rc = poppy_cuda_download(c, first, count, dst, step, frame_stride)) return rc;
+int issue_ticket(poppy_cuda_ctx* c, uint64_t* ticket) {
     if (c->tickets.empty()) {
         c->tickets.resize(64, nullptr);
         for (auto& e : c->tickets) CU_TRY(c, cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -1226,6 +1223,74 @@ int poppy_cuda_download_async(poppy_cuda_ctx* c, int first, int count, uint8_t* 
     CU_TRY(c, cudaEventRecord(c->tickets[t % c->tickets.size()], c->copy_stream));
     *ticket = t;
     return 0;
+}
+
+}  // namespace
+
+int poppy_cuda_download(poppy_cuda_ctx* c, int first, int count, uint8_t* dst, size_t step, size_t frame_stride) {
+    if (!c) return POPPY_CUDA_ERR_INVALID;
+    const size_t row = (size_t)c->w * 3;
+    if (!dst || first < 0 || count < 1 || first + count > c->max_frames || step < row || frame_stride < step * c->h)
+        return fail(c, POPPY_CUDA_ERR_INVALID, "bad download range or strides");
+    CU_TRY(c, cudaSetDevice(c->device));
+    if (int rc = copy_after_renders(c)) return rc;
+    if (step == row && frame_stride == c->frame_bytes()) {
+        CU_TRY(c, cudaMemcpyAsync(dst, c->d_frames + (size_t)first * c->frame_bytes(), (size_t)count * c->frame_bytes(),
+                                  cudaMemcpyDeviceToHost, c->copy_stream));
+    } else {
+        for (int i = 0; i < count; ++i)
+            CU_TRY(c, cudaMemcpy2DAsync(dst + (size_t)i * frame_stride, step, c->d_frames + (size_t)(first + i) * c->frame_bytes(),
+                                        row, row, c->h, cudaMemcpyDeviceToHost, c->copy_stream));
+    }
+    return copies_enqueued(c, first, count);
+}
+
+int poppy_cuda_download_i420(poppy_cuda_ctx* c, int first, int count, uint8_t* dst, size_t frame_stride) {
+    if (!c) return POPPY_CUDA_ERR_INVALID;
+    if ((c->w | c->h) & 1)
+        return fail(c, POPPY_CUDA_ERR_INVALID, "I420 needs an even frame size, the context's is %dx%d (cv::cvtColor throws too)",
+                    c->w, c->h);
+    const size_t fb = (size_t)c->w * c->h * 3 / 2;
+    if (!dst) return fail(c, POPPY_CUDA_ERR_INVALID, "dst is null");
+    if (first < 0 || count < 1 || first + count > c->max_frames)
+        return fail(c, POPPY_CUDA_ERR_INVALID, "bad download range [%d, %d) of a %d-slot ring", first, first + count, c->max_frames);
+    if (frame_stride < fb) return fail(c, POPPY_CUDA_ERR_INVALID, "frame_stride %zu is below the I420 frame size %zu", frame_stride, fb);
+    CU_TRY(c, cudaSetDevice(c->device));
+    if (!c->d_i420) {
+        const int n = std::min(kI420StageFrames, c->max_frames);
+        CU_TRY(c, cudaMalloc((void**)&c->d_i420, fb * n));
+        c->i420_frames = n;
+    }
+    if (int rc = copy_after_renders(c)) return rc;
+    // conversion and copy of each piece on the copy stream, in order: a piece's conversion overwrites the staging only after
+    // the previous piece's copy has read it
+    for (int done = 0; done < count; done += c->i420_frames) {
+        const int n = std::min(c->i420_frames, count - done);
+        launch_bgr_to_i420(c->copy_stream, c->d_frames, c->frame_bytes(), first + done, n, c->d_i420, c->w, c->h);
+        c->launches++; c->class_launches[KC_MISC]++;
+        CU_TRY(c, cudaGetLastError());
+        if (frame_stride == fb) {
+            CU_TRY(c, cudaMemcpyAsync(dst + (size_t)done * fb, c->d_i420, (size_t)n * fb, cudaMemcpyDeviceToHost, c->copy_stream));
+        } else {
+            for (int i = 0; i < n; ++i)
+                CU_TRY(c, cudaMemcpyAsync(dst + (size_t)(done + i) * frame_stride, c->d_i420 + (size_t)i * fb, fb,
+                                          cudaMemcpyDeviceToHost, c->copy_stream));
+        }
+    }
+    return copies_enqueued(c, first, count);
+}
+
+int poppy_cuda_download_async(poppy_cuda_ctx* c, int first, int count, uint8_t* dst, size_t step, size_t frame_stride,
+                              uint64_t* ticket) {
+    if (!c || !ticket) return POPPY_CUDA_ERR_INVALID;
+    if (int rc = poppy_cuda_download(c, first, count, dst, step, frame_stride)) return rc;
+    return issue_ticket(c, ticket);
+}
+
+int poppy_cuda_download_i420_async(poppy_cuda_ctx* c, int first, int count, uint8_t* dst, size_t frame_stride, uint64_t* ticket) {
+    if (!c || !ticket) return POPPY_CUDA_ERR_INVALID;
+    if (int rc = poppy_cuda_download_i420(c, first, count, dst, frame_stride)) return rc;
+    return issue_ticket(c, ticket);
 }
 
 int poppy_cuda_download_wait(poppy_cuda_ctx* c, uint64_t ticket) {

@@ -191,6 +191,19 @@ class MorphRenderer:
         self.sync()
         return out
 
+    def download_i420(self, first, count, out: np.ndarray | None = None) -> np.ndarray:
+        """Frames [first, first + count) as I420, converted on the GPU: (count, H * 3 // 2, W) uint8, per frame what
+        cv2.cvtColor(frame, cv2.COLOR_BGR2YUV_I420) returns for the BGR frame (Y rows, then the U and V planes). Needs an even
+        frame size."""
+        shape = (count, self.height * 3 // 2, self.width)
+        if out is None:
+            out = np.empty(shape, np.uint8)
+        if out.dtype != np.uint8 or out.shape != shape or not out.flags.c_contiguous:
+            raise ValueError("out must be a C-contiguous (count, H * 3 // 2, W) uint8 array")
+        self._check(self._lib.poppy_cuda_download_i420(self._ctx, first, count, _ptr(out), out.strides[0]))
+        self.sync()
+        return out
+
     def download_async(self, first, count, host_ptr, step, frame_stride):
         """Raw-pointer download into caller-owned (pinned) memory; poppy_cuda_sync() before reading."""
         self._check(self._lib.poppy_cuda_download(self._ctx, first, count, C.c_void_p(host_ptr), step, frame_stride))
