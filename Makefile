@@ -11,8 +11,8 @@ NVCCFLAGS := -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -f
 # host stages: no implicit FMA contraction (the Delaunay predicates mirror a non-FMA build of cv::Subdiv2D)
 CXXFLAGS  := -O2 -std=c++17 -fPIC -ffp-contract=off -Wall -pthread -Iinclude
 
-CU_SRC   := poppy_cuda.cu device/kernels_geometry.cu device/kernels_warp.cu device/kernels_pyramid.cu device/kernels_unsharp.cu device/kernels_yuv.cu margin.cu denoise.cu
-CPP_SRC  := host/delaunay.cpp host/morph_images.cpp host/host_abi.cpp host/writer.cpp
+CU_SRC   := poppy_cuda.cu device/kernels_geometry.cu device/kernels_warp.cu device/kernels_pyramid.cu device/kernels_unsharp.cu device/kernels_yuv.cu device/kernels_ffv1.cu margin.cu denoise.cu
+CPP_SRC  := host/delaunay.cpp host/morph_images.cpp host/host_abi.cpp host/writer.cpp host/ffv1_config.cpp host/mkv.cpp
 OBJS     := $(addprefix $(OBJDIR)/,$(CU_SRC:.cu=.cu.o) $(CPP_SRC:.cpp=.cpp.o))
 HEADERS  := $(wildcard $(CSRC)/*.cuh $(CSRC)/device/*.cuh $(CSRC)/host/*.hpp include/*.h)
 

@@ -191,6 +191,15 @@ int poppy_cuda_download_wait(poppy_cuda_ctx* ctx, uint64_t ticket);
  * of the same pool as poppy_cuda_download_async, for poppy_cuda_download_wait. */
 int poppy_cuda_download_i420(poppy_cuda_ctx* ctx, int first, int count, uint8_t* dst, size_t frame_stride);
 int poppy_cuda_download_i420_async(poppy_cuda_ctx* ctx, int first, int count, uint8_t* dst, size_t frame_stride, uint64_t* ticket);
+/* Frames [first, first+count) as lossless FFV1 packets, encoded on the device: FFV1 version 3 with the range coder, RGB
+ * (JPEG2000-RCT), 8 bits, no alpha, every frame a keyframe, a slice grid that depends on the frame size only
+ * (poppy_host_ffv1_config gives the matching configuration record). The packets land back to back at dst; sizes[i] receives
+ * the size of packet i. Only the packet bytes and the sizes cross PCIe. The bytes are a function of the frame alone. Ordering
+ * is that of poppy_cuda_download: encoding and copies run on the copy stream after every render queued so far, and a later
+ * render of these slots waits for them; the call returns when dst and sizes are filled. Device staging is allocated on the
+ * first call. POPPY_CUDA_ERR_INVALID for a null dst or sizes or a bad range, and when the packets need more than `cap`
+ * bytes: sizes[] is still filled then, so their sum is the capacity to pass. */
+int poppy_cuda_download_ffv1(poppy_cuda_ctx* ctx, int first, int count, uint8_t* dst, size_t cap, uint32_t* sizes);
 /* Page-locked host memory for download targets (asynchronous copies need it). */
 int poppy_cuda_alloc_pinned(size_t bytes, void** out);
 void poppy_cuda_free_pinned(void* p);

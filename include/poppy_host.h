@@ -82,6 +82,22 @@ void poppy_host_writer_destroy_cuda(poppy_host_writer* w);  /* flushes, joins th
  * size. Destroy it with poppy_host_writer_destroy_cuda. */
 int poppy_host_writer_create_i420(poppy_host_writer** out, poppy_cuda_ctx* ctx, int ring_frames, poppy_write_fn write,
                                   poppy_write_fn convert /* may be NULL */, int workers, void* user);
+/* The same ring delivering FFV1 packets (poppy_cuda_download_ffv1, encoded on the GPU): `packet` receives the frame index
+ * and the packet's bytes, in frame order. Destroy it with poppy_host_writer_destroy_cuda. */
+typedef void (*poppy_packet_fn)(void* user, int frame_index, const uint8_t* data, size_t size);
+int poppy_host_writer_create_ffv1(poppy_host_writer** out, poppy_cuda_ctx* ctx, int ring_frames, poppy_packet_fn packet, void* user);
+
+/* ---- FFV1 in Matroska (the reference's default output, cv::VideoWriter with fourcc FFV1) ------------------------------
+ * poppy_host_ffv1_config: the configuration record (codec extradata) of the packets poppy_cuda_download_ffv1 writes at
+ * width x height; *size receives its length, and POPPY_CUDA_ERR_INVALID is returned if dst is null or cap is smaller.
+ * poppy_host_mkv_*: one video track (CodecID V_FFV1, CodecPrivate = that record) at fps_num / fps_den frames per second;
+ * write() appends one packet as a keyframe SimpleBlock, close() writes the sizes and the duration and frees the writer.
+ * Every call returns 0 or POPPY_CUDA_ERR_INVALID (bad argument, or the file could not be written). */
+int poppy_host_ffv1_config(int width, int height, uint8_t* dst, size_t cap, size_t* size);
+typedef struct poppy_host_mkv poppy_host_mkv;
+int poppy_host_mkv_open(poppy_host_mkv** out, const char* path, int width, int height, int fps_num, int fps_den);
+int poppy_host_mkv_write(poppy_host_mkv* m, const uint8_t* packet, size_t size);
+int poppy_host_mkv_close(poppy_host_mkv* m);
 
 /* The same machinery over a caller-supplied transport (tests run it without a GPU; another source of frames can reuse it). */
 typedef struct poppy_host_writer_io {

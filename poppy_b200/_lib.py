@@ -53,6 +53,11 @@ def load():
         "poppy_shim_release": (None, []),
         "poppy_host_writer_create": (i32, [C.POINTER(vp), vp, i32, vp, vp, i32, vp]),
         "poppy_host_writer_create_i420": (i32, [C.POINTER(vp), vp, i32, vp, vp, i32, vp]),
+        "poppy_host_writer_create_ffv1": (i32, [C.POINTER(vp), vp, i32, vp, vp]),
+        "poppy_host_ffv1_config": (i32, [i32, i32, vp, C.c_size_t, C.POINTER(C.c_size_t)]),
+        "poppy_host_mkv_open": (i32, [C.POINTER(vp), C.c_char_p, i32, i32, i32, i32]),
+        "poppy_host_mkv_write": (i32, [vp, vp, C.c_size_t]),
+        "poppy_host_mkv_close": (i32, [vp]),
         "poppy_host_writer_create_io": (i32, [C.POINTER(vp), vp, i32, i32, i32, i32]),
         "poppy_host_writer_submit": (i32, [vp, i32, i32, i32]),
         "poppy_host_writer_flush": (i32, [vp]),
@@ -82,6 +87,7 @@ def load():
         "poppy_cuda_download_wait": (i32, [vp, C.c_uint64]),
         "poppy_cuda_download_i420": (i32, [vp, i32, i32, vp, C.c_size_t]),
         "poppy_cuda_download_i420_async": (i32, [vp, i32, i32, vp, C.c_size_t, u64p]),
+        "poppy_cuda_download_ffv1": (i32, [vp, i32, i32, vp, C.c_size_t, C.POINTER(C.c_uint32)]),
         "poppy_cuda_alloc_pinned": (i32, [C.c_size_t, C.POINTER(vp)]),
         "poppy_cuda_free_pinned": (None, [vp]),
         "poppy_cuda_blur_margin": (i32, [i32, vp, C.c_size_t, i32, i32, i32, i32, vp, C.c_size_t]),
@@ -119,6 +125,7 @@ CUDA_ABI_SYMBOLS = [
     "poppy_cuda_version", "poppy_cuda_get_info", "poppy_cuda_set_tile_list_capacity", "poppy_cuda_set_unsharp_mode",
     "poppy_cuda_unsharp_stats", "poppy_cuda_set_image", "poppy_cuda_set_source1_from_slot",
     "poppy_cuda_download_async", "poppy_cuda_download_wait", "poppy_cuda_download_i420", "poppy_cuda_download_i420_async",
+    "poppy_cuda_download_ffv1",
     "poppy_cuda_alloc_pinned", "poppy_cuda_free_pinned",
     "poppy_cuda_blur_margin", "poppy_cuda_blur_margin_last_error", "poppy_cuda_gabor_filter",
     "poppy_cuda_denoise", "poppy_cuda_set_segments", "poppy_cuda_set_segment", "poppy_cuda_render_segments", "poppy_cuda_get_segment_points",
@@ -126,7 +133,8 @@ CUDA_ABI_SYMBOLS = [
 HOST_ABI_SYMBOLS = [
     "poppy_host_morph_points", "poppy_host_triangulate", "poppy_host_triangulate_next", "poppy_host_chain_ratio", "poppy_host_plan_create",
     "poppy_host_plan_triangles", "poppy_host_plan_points", "poppy_host_plan_destroy", "poppy_morph_images",
-    "poppy_host_last_error", "poppy_host_writer_create", "poppy_host_writer_create_i420",
+    "poppy_host_last_error", "poppy_host_writer_create", "poppy_host_writer_create_i420", "poppy_host_writer_create_ffv1",
+    "poppy_host_ffv1_config", "poppy_host_mkv_open", "poppy_host_mkv_write", "poppy_host_mkv_close",
     "poppy_host_writer_create_io", "poppy_host_writer_submit",
     "poppy_host_writer_flush", "poppy_host_writer_destroy", "poppy_host_writer_destroy_cuda",
     "poppy_shim_morph_images", "poppy_shim_morph_sequence", "poppy_shim_morph_segments", "poppy_shim_morph_segments_devices",

@@ -18,21 +18,25 @@ does before its frame loop (gabor_filter(corrected2 * 1/255), src/poppy.hpp:119-
 morph_sequence, render_phases and morph_segments take pixel_format="bgr" (H x W x 3 frames) or "i420": each frame is then
 converted on the GPU to what cv2.cvtColor(frame, cv2.COLOR_BGR2YUV_I420) returns, an (H * 3 // 2) x W plane stack (Y, then U
 and V at half resolution) that an encoder fed yuv420p takes as it is, and half the bytes cross PCIe. I420 needs an even
-frame size.
+frame size. "ffv1" returns lossless FFV1 packets (bytes) encoded on the GPU, the reference's default output format; a
+MatroskaWriter(path, w, h) as the writer gives the .mkv that cv::VideoWriter with fourcc FFV1 writes.
 
 Host stages (clip / uniq / Delaunay / index lookup) run in the C++ part of libpoppy_cuda.so, everything else in its
 CUDA kernels. Nothing in this module computes pixels; without the native library or a GPU every call raises.
 """
 from __future__ import annotations
 
+import ctypes as C
+import os
 from dataclasses import dataclass
+from fractions import Fraction
 
 import operator
 import threading
 
 import numpy as np
 
-from . import host, shard
+from . import _lib, host, shard
 from .renderer import MorphRenderer, device_count
 
 
@@ -215,24 +219,61 @@ def _optional(gabor2):
     return None if gabor2 is None else np.ascontiguousarray(gabor2)
 
 
-def _i420(pixel_format, w, h, fn):
-    """True for pixel_format "i420", False for "bgr"; ValueError for any other format, or for I420 at an odd frame size
-    (cv::cvtColor throws there too). Called before anything is planned or rendered."""
-    if pixel_format not in ("bgr", "i420"):
-        raise ValueError(f"{fn}: pixel_format must be 'bgr' or 'i420', not {pixel_format!r}")
+def _pixel_format(pixel_format, w, h, fn):
+    """pixel_format checked before anything is planned or rendered: "bgr", "i420" or "ffv1"; ValueError for any other
+    format, or for I420 at an odd frame size (cv::cvtColor throws there too)."""
+    if pixel_format not in ("bgr", "i420", "ffv1"):
+        raise ValueError(f"{fn}: pixel_format must be 'bgr', 'i420' or 'ffv1', not {pixel_format!r}")
     if pixel_format == "i420" and (w % 2 or h % 2):
         raise ValueError(f"{fn}: I420 needs an even frame size, got {w}x{h}")
-    return pixel_format == "i420"
+    return pixel_format
+
+
+def _download(r, fmt, count):
+    """Ring slots [0, count) of renderer r in pixel format fmt."""
+    return {"bgr": r.download, "i420": r.download_i420, "ffv1": r.download_ffv1}[fmt](0, count)
+
+
+class MatroskaWriter:
+    """FFV1 packets (pixel_format="ffv1") into a Matroska file, the reference's default output (cv::VideoWriter with fourcc
+    FFV1): write(packet) appends one frame, close() finishes the file. cv2.VideoCapture plays it back."""
+
+    def __init__(self, path, width, height, fps=30):
+        self._lib = _lib.load()
+        fps = Fraction(fps).limit_denominator(1001000)
+        self._m = C.c_void_p()
+        if self._lib.poppy_host_mkv_open(C.byref(self._m), os.fsencode(path), int(width), int(height), fps.numerator,
+                                         fps.denominator) != 0:
+            raise OSError(f"cannot write a {width}x{height} Matroska file at {path!r}")
+
+    def write(self, packet):
+        if not self._m:
+            raise ValueError("MatroskaWriter is closed")
+        if self._lib.poppy_host_mkv_write(self._m, bytes(packet), len(packet)) != 0:
+            raise OSError("MatroskaWriter: write failed")
+
+    def close(self):
+        if self._m:
+            m, self._m = self._m, C.c_void_p()
+            if self._lib.poppy_host_mkv_close(m) != 0:
+                raise OSError("MatroskaWriter: close failed")
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
 
 
 def morph_sequence(corrected1, corrected2, gabor2, src_points1, src_points2, writer=None, number_of_frames=None,
                    threads=0, pixel_format="bgr"):
     """Chain mode: frame j = morph_images(previous frame, previous morphed points, shape = color = 1/(N-j)).
-    Returns the frames (N x H x W x 3, or N x 3H/2 x W with pixel_format="i420") and calls writer.write(frame) per frame
+    Returns the frames (N x H x W x 3, N x 3H/2 x W with pixel_format="i420", or a list of N FFV1 packets with
+    pixel_format="ffv1") and calls writer.write(frame) per frame
     if a writer is given. gabor2=None: derived on the GPU from corrected2."""
     n_frames = int(number_of_frames if number_of_frames is not None else Settings.instance().number_of_frames)
     h, w = corrected1.shape[:2]
-    i420 = _i420(pixel_format, w, h, "morph_sequence")
+    fmt = _pixel_format(pixel_format, w, h, "morph_sequence")
     ratio = np.array([host.chain_ratio(j, n_frames) for j in range(n_frames)], np.float64)
     plan = host.SequencePlan(src_points1, src_points2, w, h, ratio.astype(np.float32), chain=True, threads=threads)
     try:
@@ -240,7 +281,7 @@ def morph_sequence(corrected1, corrected2, gabor2, src_points1, src_points2, wri
         r.set_pair(np.ascontiguousarray(corrected1), np.ascontiguousarray(corrected2), _optional(gabor2))
         r.set_points(src_points1, src_points2)
         r.render(ratio.astype(np.float32), ratio, plan.tri_idx, plan.tri_offsets, chain=True)
-        frames = r.download_i420(0, n_frames) if i420 else r.download(0, n_frames)
+        frames = _download(r, fmt, n_frames)
     finally:
         plan.close()
     if writer is not None:
@@ -252,9 +293,10 @@ def morph_sequence(corrected1, corrected2, gabor2, src_points1, src_points2, wri
 def render_phases(corrected1, corrected2, gabor2, src_points1, src_points2, phases, mask_ratios=None, threads=0,
                   pixel_format="bgr"):
     """Direct mode: independent phases s_k of one pair, shape = s_k and mask = mask_ratios[k] (default s_k).
-    Returns N x H x W x 3 frames, or N x 3H/2 x W with pixel_format="i420". gabor2=None: derived on the GPU from corrected2."""
+    Returns N x H x W x 3 frames, N x 3H/2 x W with pixel_format="i420", or a list of N FFV1 packets with
+    pixel_format="ffv1". gabor2=None: derived on the GPU from corrected2."""
     h, w = corrected1.shape[:2]
-    i420 = _i420(pixel_format, w, h, "render_phases")
+    fmt = _pixel_format(pixel_format, w, h, "render_phases")
     phases = np.ascontiguousarray(phases, np.float32)
     masks = np.ascontiguousarray(mask_ratios if mask_ratios is not None else phases.astype(np.float64), np.float64)
     plan = host.SequencePlan(src_points1, src_points2, w, h, phases, chain=False, threads=threads)
@@ -263,7 +305,7 @@ def render_phases(corrected1, corrected2, gabor2, src_points1, src_points2, phas
         r.set_pair(np.ascontiguousarray(corrected1), np.ascontiguousarray(corrected2), _optional(gabor2))
         r.set_points(src_points1, src_points2)
         r.render(phases, masks, plan.tri_idx, plan.tri_offsets, chain=False)
-        return r.download_i420(0, len(phases)) if i420 else r.download(0, len(phases))
+        return _download(r, fmt, len(phases))
     finally:
         plan.close()
 
@@ -301,10 +343,9 @@ def _check_devices(devices):
     return devices
 
 
-def _render_segment_range(r, segments, plans, lo, hi, per_batch, shape, ratio, frames, i420, stop=None):
-    """Segments [lo, hi) on renderer r, per_batch at a time, downloaded (as BGR or I420) into frames[lo:hi]."""
-    n_frames = frames.shape[1]
-    download = r.download_i420 if i420 else r.download
+def _render_segment_range(r, segments, plans, lo, hi, per_batch, shape, ratio, frames, fmt, stop=None):
+    """Segments [lo, hi) on renderer r, per_batch at a time, downloaded (as BGR, I420 or FFV1 packets) into frames[lo:hi]."""
+    n_frames = len(shape)
     for b0 in range(lo, hi, per_batch):
         if stop is not None and stop.is_set():
             return
@@ -316,13 +357,20 @@ def _render_segment_range(r, segments, plans, lo, hi, per_batch, shape, ratio, f
                           np.reshape(p2, (-1, 2)))
         tri, offs = interleave_segment_plans([plans[s] for s in batch], n_frames)
         r.render_segments(0, shape, ratio, tri, offs)
-        download(0, len(batch) * n_frames, out=frames[b0:b0 + len(batch)].reshape((-1,) + frames.shape[2:]))
+        if fmt == "ffv1":
+            packets = r.download_ffv1(0, len(batch) * n_frames)
+            for i in range(len(batch)):
+                frames[b0 + i] = packets[i * n_frames:(i + 1) * n_frames]
+        else:
+            download = r.download_i420 if fmt == "i420" else r.download
+            download(0, len(batch) * n_frames, out=frames[b0:b0 + len(batch)].reshape((-1,) + frames.shape[2:]))
 
 
 def morph_segments(segments, number_of_frames=None, writer=None, threads=0, devices=None, pixel_format="bgr"):
     """The segments of a multi-image sequence: segments[i] = (corrected1, corrected2, gabor2 or None, pts1, pts2) of one
     consecutive pair, all of one frame size. Each is the chain morph_sequence renders, and they are rendered together.
-    Returns the frames as a (K, N, H, W, 3) array, or (K, N, 3H/2, W) with pixel_format="i420", and calls writer.write(frame)
+    Returns the frames as a (K, N, H, W, 3) array, (K, N, 3H/2, W) with pixel_format="i420", or K lists of N packets (bytes)
+    with pixel_format="ffv1", and calls writer.write(frame)
     in the reference's order: the N frames of segment 0, then those of segment 1, and so on (one video, as run() writes it).
 
     devices=None renders on Settings.cuda_device. devices=[d0, d1, ...] shards the K segments over the first
@@ -333,7 +381,7 @@ def morph_segments(segments, number_of_frames=None, writer=None, threads=0, devi
     n_frames = int(number_of_frames if number_of_frames is not None else Settings.instance().number_of_frames)
     K = len(segments)
     h, w = segments[0][0].shape[:2] if K else (0, 0)
-    i420 = _i420(pixel_format, w, h, "morph_segments")
+    fmt = _pixel_format(pixel_format, w, h, "morph_segments")
     if devices is not None:
         devices = _check_devices(devices)
     if K == 0:
@@ -347,7 +395,10 @@ def morph_segments(segments, number_of_frames=None, writer=None, threads=0, devi
     shape = ratio.astype(np.float32)
     plans = [host.SequencePlan(np.reshape(p1, (-1, 2)), np.reshape(p2, (-1, 2)), w, h, shape, chain=True, threads=threads)
              for _, _, _, p1, p2 in segments]
-    frames = np.empty((K, n_frames, h * 3 // 2, w) if i420 else (K, n_frames, h, w, 3), np.uint8)
+    if fmt == "ffv1":
+        frames = [None] * K
+    else:
+        frames = np.empty((K, n_frames, h * 3 // 2, w) if fmt == "i420" else (K, n_frames, h, w, 3), np.uint8)
     n_max, tri_max = max(p.n for p in plans), max(p.max_triangles for p in plans)
 
     def per_batch(count):
@@ -356,7 +407,7 @@ def morph_segments(segments, number_of_frames=None, writer=None, threads=0, devi
     try:
         if devices is None:
             r = _renderer(w, h, n_max, tri_max, per_batch(K) * n_frames)
-            _render_segment_range(r, segments, plans, 0, K, per_batch(K), shape, ratio, frames, i420)
+            _render_segment_range(r, segments, plans, 0, K, per_batch(K), shape, ratio, frames, fmt)
         else:
             G = min(len(devices), K)
             stop, errors = threading.Event(), []
@@ -367,7 +418,7 @@ def morph_segments(segments, number_of_frames=None, writer=None, threads=0, devi
                     d, b = devices[g], per_batch(hi - lo)
                     r = _renderer(w, h, n_max, tri_max, b * n_frames) if d == Settings.instance().cuda_device \
                         else _device_renderer(d, w, h, n_max, tri_max, b * n_frames)
-                    _render_segment_range(r, segments, plans, lo, hi, b, shape, ratio, frames, i420, stop)
+                    _render_segment_range(r, segments, plans, lo, hi, b, shape, ratio, frames, fmt, stop)
                 except BaseException as e:      # the other devices stop before their next batch; re-raised below
                     errors.append(e)
                     stop.set()

@@ -19,6 +19,7 @@ CUDA_SOURCES = [
     "device/kernels_pyramid.cu",
     "device/kernels_unsharp.cu",
     "device/kernels_yuv.cu",
+    "device/kernels_ffv1.cu",
     "margin.cu",
     "denoise.cu",
 ]
@@ -27,6 +28,8 @@ HOST_SOURCES = [
     "host/morph_images.cpp",
     "host/host_abi.cpp",
     "host/writer.cpp",
+    "host/ffv1_config.cpp",
+    "host/mkv.cpp",
 ]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-fmad=false",

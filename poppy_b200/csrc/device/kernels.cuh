@@ -143,4 +143,17 @@ void launch_checksum(cudaStream_t st, const uint8_t* data, size_t bytes, unsigne
 void launch_bgr_to_i420(cudaStream_t st, const uint8_t* ring, size_t frame_bytes, int first_slot, int frames, uint8_t* out, int w,
                         int h);
 
+// ---- kernels_ffv1.cu ---------------------------------------------------------------------------------------------
+// FFV1 packets of ring slots [first_slot, first_slot + frames) (ffv1_format.hpp). sym: w * h * 3 uint32 per frame. code: `count`
+// slices (slice t = slice t % (nh * nv) of frame t / (nh * nv)), or those `list` names, each into `cap` bytes at out; see the
+// kernel. pack: offsets (frames * slices + 1) and frame_sizes (frames), then the packets, contiguous, at `packets`.
+void launch_ffv1_symbols(cudaStream_t st, const uint8_t* ring, size_t frame_bytes, int first_slot, int frames, uint32_t* sym, int w,
+                         int h, int nh, int nv);
+cudaError_t launch_ffv1_code(cudaStream_t st, const uint32_t* sym, const uint8_t* tables, int w, int h, int nh, int nv, int count,
+                             const int* list, uint8_t* out, size_t cap, uint32_t* sizes, int* slot_of, int* overflow_count,
+                             int* overflow_list);
+void launch_ffv1_pack(cudaStream_t st, const uint32_t* sizes, int slices, int frames, uint64_t* offsets, uint32_t* frame_sizes,
+                      const uint8_t* slots, size_t cap, const uint8_t* scratch, size_t scratch_cap, const int* slot_of,
+                      uint8_t* packets);
+
 }  // namespace poppy

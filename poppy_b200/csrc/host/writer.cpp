@@ -8,6 +8,7 @@
 #include <condition_variable>
 #include <cstring>
 #include <deque>
+#include <map>
 #include <mutex>
 #include <string>
 #include <thread>
@@ -27,7 +28,7 @@ struct poppy_host_writer {
     std::deque<Item> pending;                   // submitted, in frame order
     size_t next_convert = 0;                    // first entry of `pending` no worker has taken yet
     uint64_t submitted = 0, written = 0;
-    bool stop = false;
+    bool stop = false, owned_ffv1 = false;     // owned_ffv1: io.owned_transport is an FFV1 transport
     int error = 0;
     std::thread deliverer;
     std::vector<std::thread> pool;
@@ -213,11 +214,68 @@ int poppy_host_writer_create_i420(poppy_host_writer** out, poppy_cuda_ctx* ctx, 
     return cuda_writer_create(out, ctx, ring_frames, write, convert, workers, user, true);
 }
 
+namespace {
+
+// FFV1: the ring buffers hold W*H*3 bytes + a margin, which every natural frame's packet fits. The encode is synchronous (the
+// packet size is known only after it), so the transport has no wait step. A packet that does not fit its buffer (noise)
+// goes to a heap buffer of its exact size, handed to `packet` in place of the ring buffer.
+struct Ffv1Transport {
+    poppy_cuda_ctx* ctx;
+    poppy_packet_fn packet;
+    void* user;
+    size_t cap;
+    std::mutex mu;
+    std::map<const uint8_t*, std::vector<uint8_t>> large;   // ring buffer -> the packet that did not fit it
+    std::map<const uint8_t*, size_t> size;                   // ring buffer -> its packet's size
+};
+int ft_download(void* u, int slot, uint8_t* dst, size_t, uint64_t* ticket) {
+    auto* t = (Ffv1Transport*)u;
+    uint32_t n = 0;
+    *ticket = 0;
+    int rc = poppy_cuda_download_ffv1(t->ctx, slot, 1, dst, t->cap, &n);
+    if (rc == POPPY_CUDA_ERR_INVALID && n > t->cap) {
+        std::vector<uint8_t> big(n);
+        rc = poppy_cuda_download_ffv1(t->ctx, slot, 1, big.data(), big.size(), &n);
+        if (rc == 0) { std::lock_guard<std::mutex> lk(t->mu); t->large[dst] = std::move(big); }
+    }
+    if (rc == 0) { std::lock_guard<std::mutex> lk(t->mu); t->size[dst] = n; }
+    return rc;
+}
+void ft_write(void* u, int idx, uint8_t* buf, int, int, size_t) {
+    auto* t = (Ffv1Transport*)u;
+    std::vector<uint8_t> big;
+    size_t n;
+    {
+        std::lock_guard<std::mutex> lk(t->mu);
+        n = t->size[buf];
+        auto it = t->large.find(buf);
+        if (it != t->large.end()) { big = std::move(it->second); t->large.erase(it); }
+    }
+    t->packet(t->user, idx, big.empty() ? buf : big.data(), n);
+}
+}  // namespace
+
+int poppy_host_writer_create_ffv1(poppy_host_writer** out, poppy_cuda_ctx* ctx, int ring_frames, poppy_packet_fn packet, void* user) {
+    if (!out || !ctx || !packet) return POPPY_CUDA_ERR_INVALID;
+    int w = 0, h = 0;
+    if (int rc = poppy_cuda_get_info(ctx, &w, &h, nullptr, nullptr, nullptr, nullptr)) return rc;
+    auto* t = new Ffv1Transport{ctx, packet, user, (size_t)w * h * 3 + 65536, {}, {}, {}};
+    poppy_host_writer_io io{};
+    io.user = t; io.download = ft_download; io.wait = nullptr; io.alloc = ct_alloc; io.release = ct_release; io.write = ft_write;
+    const int rc = writer_create(out, &io, w, h, 0, t->cap, ring_frames, 0);
+    if (rc != 0) { delete t; return rc; }
+    (*out)->io.owned_transport = t;
+    (*out)->owned_ffv1 = true;
+    return 0;
+}
+
 void poppy_host_writer_destroy_cuda(poppy_host_writer* w) {
     if (!w) return;
-    auto* t = (CudaTransport*)w->io.owned_transport;
+    void* t = w->io.owned_transport;
+    const bool ffv1 = w->owned_ffv1;
     poppy_host_writer_destroy(w);
-    delete t;
+    if (ffv1) delete (Ffv1Transport*)t;
+    else delete (CudaTransport*)t;
 }
 
 }  // extern "C"

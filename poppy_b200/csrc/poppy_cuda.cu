@@ -9,6 +9,9 @@
 //                       warped pair 2 x uint32 BGRX [H][pitch0]; Gaussian levels 1..L (7 planes); collapsed levels 0..L
 //                       (3 planes); level-0 blend mask float [H][pitch0]
 //   I420 staging      : (optional, poppy_cuda_download_i420) up to kI420StageFrames x W*H*3/2 bytes, allocated on first use
+//   FFV1 staging      : (optional, poppy_cuda_download_ffv1) a piece of up to kFfv1StagePixels pixels: 12 B of symbols and
+//                       3 B + slice allowance of slice slots per pixel, the packets, per-slice tables; overflow scratch
+//                       on demand. Allocated on first use.
 //   segments (optional, poppy_cuda_set_segments): per segment the pair's resident data - corrected1, corrected2 and chain
 //                       arrays, a mask basis (one allocation, padded_pixels() floats each), raw and clipped point sets;
 //                       per lane a SegFrame table and a BGRX staging plane per frame of a chunk
@@ -25,6 +28,7 @@
 
 #include "../../include/poppy_cuda.h"
 #include "device/kernels.cuh"
+#include "ffv1_format.hpp"
 
 using namespace poppy;
 
@@ -57,6 +61,9 @@ constexpr int kRenderLanes = 4;
 // I420 downloads convert at most this many frames per piece into device staging (a 4K frame is 12.4 MB in I420)
 constexpr int kI420StageFrames = 8;
 
+// FFV1 downloads encode at most this many pixels per piece (8 4K frames, 1,003 MB of device staging)
+constexpr size_t kFfv1StagePixels = (size_t)8 * 3840 * 2160;
+
 }  // namespace
 
 struct poppy_cuda_ctx {
@@ -81,6 +88,16 @@ struct poppy_cuda_ctx {
     int copy_lo = 0, copy_hi = 0;        // ring slots [lo, hi) with a download enqueued since the last sync
     uint8_t* d_i420 = nullptr;           // I420 staging of poppy_cuda_download_i420 (copy stream only)
     int i420_frames = 0;                 // frames d_i420 holds
+    struct Ffv1Stage {                   // poppy_cuda_download_ffv1 (copy stream only)
+        int frames = 0, nh = 0, nv = 0;
+        size_t cap = 0, scratch_cap = 0, scratch_slices = 0, packets_cap = 0;
+        uint32_t* d_sym = nullptr;
+        uint8_t *d_slots = nullptr, *d_packets = nullptr, *d_tables = nullptr, *d_scratch = nullptr;
+        uint32_t *d_sizes = nullptr, *d_frame_sizes = nullptr;
+        uint64_t* d_offsets = nullptr;
+        int *d_slot_of = nullptr, *d_overflow = nullptr;   // d_overflow: count, then the list
+        int* h_overflow = nullptr;                         // pinned
+    } ffv1;
     std::string err;
     uint64_t launches = 0;
 
@@ -761,6 +778,10 @@ void poppy_cuda_destroy(poppy_cuda_ctx* c) {
     }
     cudaFree(c->d_pts1_raw); cudaFree(c->d_pts2_raw); cudaFree(c->d_pts1); cudaFree(c->d_pts2); cudaFree(c->d_morphed);
     cudaFree(c->d_tail_levels);
+    cudaFree(c->ffv1.d_sym); cudaFree(c->ffv1.d_slots); cudaFree(c->ffv1.d_packets); cudaFree(c->ffv1.d_tables);
+    cudaFree(c->ffv1.d_scratch); cudaFree(c->ffv1.d_sizes); cudaFree(c->ffv1.d_frame_sizes); cudaFree(c->ffv1.d_offsets);
+    cudaFree(c->ffv1.d_slot_of); cudaFree(c->ffv1.d_overflow);
+    if (c->ffv1.h_overflow) cudaFreeHost(c->ffv1.h_overflow);
     cudaFree(c->d_frames); cudaFree(c->d_i420); cudaFree(c->d_sum); cudaFree(c->d_calm_total); cudaFree(c->d_probe_total); cudaFree(c->d_plan_tri);
     if (c->ev_begin) cudaEventDestroy(c->ev_begin);
     if (c->ev_end) cudaEventDestroy(c->ev_end);
@@ -1291,6 +1312,100 @@ int poppy_cuda_download_i420_async(poppy_cuda_ctx* c, int first, int count, uint
     if (!c || !ticket) return POPPY_CUDA_ERR_INVALID;
     if (int rc = poppy_cuda_download_i420(c, first, count, dst, frame_stride)) return rc;
     return issue_ticket(c, ticket);
+}
+
+namespace {
+
+int ffv1_stage(poppy_cuda_ctx* c) {
+    auto& f = c->ffv1;
+    if (f.d_sym) return 0;
+    poppy::ffv1::slice_grid(c->w, c->h, &f.nh, &f.nv);
+    // at most 4096 frames a piece: the symbol kernel's grid z
+    f.frames = (int)std::max<size_t>(1, std::min<size_t>({(size_t)c->max_frames, kFfv1StagePixels / c->pixels(), (size_t)4096}));
+    const int slices = f.nh * f.nv * f.frames;
+    // the largest slice: columns and rows are split as evenly as integer division allows
+    const size_t slice_px = (size_t)((c->w + f.nh - 1) / f.nh) * ((c->h + f.nv - 1) / f.nv);
+    f.cap = (slice_px * 3 + poppy::ffv1::kSliceAllowance + 15) / 16 * 16;                // raw sample bytes + allowance
+    f.scratch_cap = (slice_px * poppy::ffv1::kWorstBytesPer3Samples + 2 * poppy::ffv1::kSliceAllowance + 15) / 16 * 16;
+    uint8_t tables[512];
+    poppy::ffv1::build_states(tables, tables + 256);
+    CU_TRY(c, dmalloc(&f.d_sym, c->pixels() * 3 * f.frames));
+    CU_TRY(c, dmalloc(&f.d_slots, f.cap * slices));
+    f.packets_cap = f.cap * slices + (size_t)3 * slices;     // grows when slices are coded again into scratch
+    CU_TRY(c, dmalloc(&f.d_packets, f.packets_cap));
+    CU_TRY(c, dmalloc(&f.d_tables, 512));
+    CU_TRY(c, dmalloc(&f.d_sizes, slices));
+    CU_TRY(c, dmalloc(&f.d_frame_sizes, f.frames));
+    CU_TRY(c, dmalloc(&f.d_offsets, slices + 1));
+    CU_TRY(c, dmalloc(&f.d_slot_of, slices));
+    CU_TRY(c, dmalloc(&f.d_overflow, slices + 1));
+    CU_TRY(c, cudaMallocHost((void**)&f.h_overflow, sizeof(int)));
+    CU_TRY(c, cudaMemcpy(f.d_tables, tables, 512, cudaMemcpyHostToDevice));
+    return 0;
+}
+
+}  // namespace
+
+int poppy_cuda_download_ffv1(poppy_cuda_ctx* c, int first, int count, uint8_t* dst, size_t cap, uint32_t* sizes) {
+    if (!c) return POPPY_CUDA_ERR_INVALID;
+    if (!dst || !sizes) return fail(c, POPPY_CUDA_ERR_INVALID, "dst or sizes is null");
+    if (first < 0 || count < 1 || first + count > c->max_frames)
+        return fail(c, POPPY_CUDA_ERR_INVALID, "bad download range [%d, %d) of a %d-slot ring", first, first + count, c->max_frames);
+    CU_TRY(c, cudaSetDevice(c->device));
+    if (int rc = ffv1_stage(c)) return rc;
+    auto& f = c->ffv1;
+    const int per_frame = f.nh * f.nv;
+    if (int rc = copy_after_renders(c)) return rc;
+    size_t total = 0;
+    for (int done = 0; done < count; done += f.frames) {
+        const int n = std::min(f.frames, count - done), slices = n * per_frame;
+        launch_ffv1_symbols(c->copy_stream, c->d_frames, c->frame_bytes(), first + done, n, f.d_sym, c->w, c->h, f.nh, f.nv);
+        CU_TRY(c, cudaMemsetAsync(f.d_overflow, 0, sizeof(int), c->copy_stream));
+        CU_TRY(c, launch_ffv1_code(c->copy_stream, f.d_sym, f.d_tables, c->w, c->h, f.nh, f.nv, slices, nullptr, f.d_slots, f.cap,
+                                   f.d_sizes, f.d_slot_of, f.d_overflow, f.d_overflow + 1));
+        CU_TRY(c, cudaMemcpyAsync(f.h_overflow, f.d_overflow, sizeof(int), cudaMemcpyDeviceToHost, c->copy_stream));
+        CU_TRY(c, cudaStreamSynchronize(c->copy_stream));
+        const int over = *f.h_overflow;
+        c->launches += 2; c->class_launches[KC_MISC] += 2;
+        if (over > 0) {
+            // slices whose samples did not fit their raw size are coded again, into worst-case scratch
+            if ((size_t)over > f.scratch_slices) {
+                CU_TRY(c, cudaFree(f.d_scratch));
+                f.d_scratch = nullptr; f.scratch_slices = 0;
+                CU_TRY(c, dmalloc(&f.d_scratch, f.scratch_cap * over));
+                f.scratch_slices = over;
+            }
+            // the packets then hold up to `over` slices of scratch size
+            const size_t need = (size_t)(slices - over) * f.cap + (size_t)over * f.scratch_cap + (size_t)3 * slices;
+            if (need > f.packets_cap) {
+                CU_TRY(c, cudaFree(f.d_packets));
+                f.d_packets = nullptr; f.packets_cap = 0;
+                CU_TRY(c, dmalloc(&f.d_packets, need));
+                f.packets_cap = need;
+            }
+            CU_TRY(c, launch_ffv1_code(c->copy_stream, f.d_sym, f.d_tables, c->w, c->h, f.nh, f.nv, over, f.d_overflow + 1,
+                                       f.d_scratch, f.scratch_cap, f.d_sizes, f.d_slot_of, f.d_overflow, f.d_overflow + 1));
+            c->launches++; c->class_launches[KC_MISC]++;
+        }
+        launch_ffv1_pack(c->copy_stream, f.d_sizes, per_frame, n, f.d_offsets, f.d_frame_sizes, f.d_slots, f.cap, f.d_scratch,
+                         f.scratch_cap, f.d_slot_of, f.d_packets);
+        c->launches += 2; c->class_launches[KC_MISC] += 2;
+        CU_TRY(c, cudaGetLastError());
+        // only the packets cross PCIe: their sizes first, then exactly their bytes
+        CU_TRY(c, cudaMemcpyAsync(sizes + done, f.d_frame_sizes, sizeof(uint32_t) * n, cudaMemcpyDeviceToHost, c->copy_stream));
+        CU_TRY(c, cudaStreamSynchronize(c->copy_stream));
+        size_t bytes = 0;
+        for (int i = 0; i < n; ++i) bytes += sizes[done + i];
+        if (total + bytes <= cap)
+            CU_TRY(c, cudaMemcpyAsync(dst + total, f.d_packets, bytes, cudaMemcpyDeviceToHost, c->copy_stream));
+        total += bytes;
+    }
+    if (int rc = copies_enqueued(c, first, count)) return rc;
+    CU_TRY(c, cudaStreamSynchronize(c->copy_stream));
+    if (total > cap)
+        return fail(c, POPPY_CUDA_ERR_INVALID, "the %d packets take %zu bytes, dst holds %zu (sizes[] has each packet's size)", count,
+                    total, cap);
+    return 0;
 }
 
 int poppy_cuda_download_wait(poppy_cuda_ctx* c, uint64_t ticket) {

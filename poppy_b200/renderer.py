@@ -204,6 +204,24 @@ class MorphRenderer:
         self.sync()
         return out
 
+    def download_ffv1(self, first, count) -> list[bytes]:
+        """Frames [first, first + count) as lossless FFV1 packets encoded on the GPU, one bytes object per frame; a
+        MatroskaWriter of this frame size (api.py) stores them as the .mkv cv::VideoWriter with fourcc FFV1 writes."""
+        sizes = np.zeros(count, np.uint32)
+        cap = count * (self.width * self.height * 3 + 65536)
+        while True:
+            out = np.empty(cap, np.uint8)
+            rc = self._lib.poppy_cuda_download_ffv1(self._ctx, first, count, _ptr(out), cap,
+                                                    sizes.ctypes.data_as(C.POINTER(C.c_uint32)))
+            need = int(sizes.sum(dtype=np.uint64))
+            if rc == 0 or not (rc == -2 and need > cap):
+                break
+            cap = need                            # packets larger than their raw frames (noise): encode again at their size
+        self._check(rc)
+        ends = np.cumsum(sizes, dtype=np.int64)
+        data = out[:need].tobytes()
+        return [data[e - n:e] for e, n in zip(ends.tolist(), sizes.tolist())]
+
     def download_async(self, first, count, host_ptr, step, frame_stride):
         """Raw-pointer download into caller-owned (pinned) memory; poppy_cuda_sync() before reading."""
         self._check(self._lib.poppy_cuda_download(self._ctx, first, count, C.c_void_p(host_ptr), step, frame_stride))
