@@ -39,7 +39,7 @@ def _content(kind, w, h, seed=0):
     if kind == "noise":
         return rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
     if kind == "morph":      # the renderer's own inputs: smooth photographic-like content
-        return any_size_inputs(w, h, seed=seed)[0]
+        return any_size_inputs(w, h, seed=seed, smooth=True)[0]
     raise ValueError(kind)
 
 
