@@ -7,7 +7,7 @@ import pytest
 
 from oracle import port, ref
 from poppy_b200 import synth
-from tests.util import bits_differ
+from tests.util import bits_differ, random_triangles, remap_map_families
 
 needs_ref = pytest.mark.skipif(not ref.available(), reason="oracle/_ref/libpoppy_ref.so not built")
 
@@ -46,28 +46,8 @@ def test_stage_decomposition_equals_morph_images():
 
 @needs_ref
 def test_fill_convex_poly_random_and_degenerate():
-    rng = np.random.default_rng(3)
     w, h = 97, 71
-    tris = []
-    for i in range(4000):
-        k = i % 10
-        if k < 6:
-            t = np.stack([rng.integers(0, w, 3), rng.integers(0, h, 3)], 1)
-        elif k < 8:
-            c = np.array([rng.integers(6, w - 6), rng.integers(6, h - 6)])
-            t = c + rng.integers(-6, 7, (3, 2))
-        elif k == 8:   # collinear / repeated vertices
-            a = np.array([rng.integers(0, w), rng.integers(0, h)])
-            d = rng.integers(-3, 4, 2)
-            t = np.stack([a, a + d, a + 2 * d if i % 20 < 10 else a])
-            t[:, 0] = np.clip(t[:, 0], 0, w - 1)
-            t[:, 1] = np.clip(t[:, 1], 0, h - 1)
-        else:          # axis aligned
-            x0, x1 = sorted(rng.integers(0, w, 2))
-            y0, y1 = sorted(rng.integers(0, h, 2))
-            t = np.array([[x0, y0], [x1, y0], [x0, y1]])
-        tris.append(t.reshape(6))
-    tris = np.array(tris, np.int32)
+    tris = random_triangles(w, h, 4000)
     # one triangle at a time (coverage of each) and all together (later index wins)
     for i in range(0, 4000, 7):
         assert (ref.fill_triangles(w, h, tris[i:i + 1]) == port.fill_triangles(w, h, tris[i:i + 1])).all(), tris[i]
@@ -108,19 +88,7 @@ def test_remap_borders_ties_and_saturation():
     rng = np.random.default_rng(8)
     h, w = 57, 83
     src = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
-    yy, xx = np.mgrid[0:h, 0:w].astype(np.float32)
-    maps = {
-        "identity": (xx, yy),
-        "smooth": (xx + 3 * np.sin(yy / 7).astype(np.float32), yy + 2 * np.cos(xx / 5).astype(np.float32)),
-        "fractions": ((xx % 8) + (np.arange(w * h).reshape(h, w) % 32 / 32).astype(np.float32),
-                      (yy % 8) + (np.arange(w * h).reshape(h, w) // 32 % 32 / 32).astype(np.float32)),
-        "out_of_bounds": (xx * 1.5 - 20, yy * 1.5 - 15),
-        "ties": (xx + np.float32(1 / 64), yy + np.float32(3 / 64)),
-        "huge": (xx * 800 - 20000, yy * 900 - 20000),
-        "edge": (xx + np.float32(0.5) - 1, yy + np.float32(0.75) - 1),
-    }
-    for name, (mx, my) in maps.items():
-        mx, my = np.ascontiguousarray(mx, np.float32), np.ascontiguousarray(my, np.float32)
+    for name, (mx, my) in remap_map_families(w, h).items():
         assert (ref.remap_u8c3(src, mx, my) == port.remap_u8c3(src, mx, my)).all(), name
 
 

@@ -43,6 +43,49 @@ def any_size_inputs(w, h, seed=0, smooth=False):
     return bgr1, bgr2, gab, pts1, pts2
 
 
+def remap_map_families(w, h):
+    """{name: (mapx, mapy)} float32 maps of a w x h destination that reach remap's borders, ties and saturation: identity,
+    smooth, every 1/32 fraction, out of bounds, 1/64 ties, coordinates past the 16-bit clamp, half-pixel edges."""
+    yy, xx = np.mgrid[0:h, 0:w].astype(np.float32)
+    maps = {
+        "identity": (xx, yy),
+        "smooth": (xx + 3 * np.sin(yy / 7).astype(np.float32), yy + 2 * np.cos(xx / 5).astype(np.float32)),
+        "fractions": ((xx % 8) + (np.arange(w * h).reshape(h, w) % 32 / 32).astype(np.float32),
+                      (yy % 8) + (np.arange(w * h).reshape(h, w) // 32 % 32 / 32).astype(np.float32)),
+        "out_of_bounds": (xx * 1.5 - 20, yy * 1.5 - 15),
+        "ties": (xx + np.float32(1 / 64), yy + np.float32(3 / 64)),
+        "huge": (xx * 800 - 20000, yy * 900 - 20000),
+        "edge": (xx + np.float32(0.5) - 1, yy + np.float32(0.75) - 1),
+    }
+    return {k: (np.ascontiguousarray(mx, np.float32), np.ascontiguousarray(my, np.float32)) for k, (mx, my) in maps.items()}
+
+
+def random_triangles(w, h, n, seed=3):
+    """n x 6 int32 triangles (x0, y0, x1, y1, x2, y2) with every vertex inside a w x h image: in every 10, six anywhere,
+    two small ones, one collinear or with repeated vertices, one axis aligned."""
+    rng = np.random.default_rng(seed)
+    tris = []
+    for i in range(n):
+        k = i % 10
+        if k < 6:
+            t = np.stack([rng.integers(0, w, 3), rng.integers(0, h, 3)], 1)
+        elif k < 8:
+            c = np.array([rng.integers(6, w - 6), rng.integers(6, h - 6)])
+            t = c + rng.integers(-6, 7, (3, 2))
+        elif k == 8:   # collinear / repeated vertices
+            a = np.array([rng.integers(0, w), rng.integers(0, h)])
+            d = rng.integers(-3, 4, 2)
+            t = np.stack([a, a + d, a + 2 * d if i % 20 < 10 else a])
+            t[:, 0] = np.clip(t[:, 0], 0, w - 1)
+            t[:, 1] = np.clip(t[:, 1], 0, h - 1)
+        else:          # axis aligned
+            x0, x1 = sorted(rng.integers(0, w, 2))
+            y0, y1 = sorted(rng.integers(0, h, 2))
+            t = np.array([[x0, y0], [x1, y0], [x0, y1]])
+        tris.append(t.reshape(6))
+    return np.array(tris, np.int32)
+
+
 def bits_differ(a: np.ndarray, b: np.ndarray) -> int:
     """Number of elements whose bit patterns differ (floats compared as uint32, so -0/+0 and NaNs count)."""
     assert a.shape == b.shape, (a.shape, b.shape)
